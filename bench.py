@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- cell-layer updates/s of the msqg timestep (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one full predictor-corrector timestep (2 x (PV inversion + RHS +
 stage update)) of the 4096^2 x nl=4 synthetic double-gyre workload of
@@ -9,7 +9,16 @@ SURVEY.md 8(d).  `value` is measured with the state resident in HBM; `e2e` is
 the same step driven through the C ABI with HOST buffers (q uploaded from and
 downloaded to pinned host memory every step).  `--impl reference` times the
 CPU oracle (the reference itself cannot be built here: Basilisk/qcc absent) on
-all host cores on a bounded sample of the same workload.
+all host cores on the same workload.
+
+`--dump-outputs DIR` writes, after the K timed steps, what the timed path returned
+in its last step as DIR/<name>.npy (float64): `dt` and `t` (the last time step and
+the model time after it) and `psi` and `q` (the stream function and potential
+vorticity, flattened [layer][y][x]; fields of more than DUMP_SAMPLE values are cut
+to a fixed seeded sample, see dump_indices).  Inputs are synthetic and seeded, so
+two builds run with the same arguments can be compared file for file.  (The
+`--impl reference` sweep is an OpenMP loop whose result depends on thread timing;
+its outputs repeat from run to run with OMP_NUM_THREADS=1 only.)
 """
 import argparse
 import json
@@ -20,6 +29,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from as it found it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -58,6 +68,26 @@ def workload_name(N, nl):
     return "msqg double-gyre %d^2 x nl=%d, %s, tolerance 1e-3%s%s" % (
         N, nl, "vertical-mode inversion (MODE_PV_INVERT 1)" if MODAL else "layer-coupled multigrid inversion (MODE_PV_INVERT 0)",
         ", doubly periodic (sbc = -1)" if PERIODIC else "", ", Ro(y) (varRo = 1)" if VARRO else "")
+
+
+DUMP_SAMPLE = 1 << 21  # values kept per field by --dump-outputs (16 MB in float64; psi + q stay well under 64 MB)
+
+
+def dump_indices(n):
+    """Flat indices of a field of n values that --dump-outputs keeps: all of them up to DUMP_SAMPLE, else a sorted
+    sample drawn without replacement from a fixed seed, so runs with the same arguments keep the same cells."""
+    if n <= DUMP_SAMPLE:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+
+
+def dump_outputs(d, dt, t, psi, q):
+    """--dump-outputs: the last timed step's dt and model time t, and psi and q (sampled by dump_indices)"""
+    os.makedirs(d, exist_ok=True)
+    psi, q = np.ravel(psi), np.ravel(q)
+    idx = dump_indices(psi.size)
+    for name, a in (("dt", np.ravel(dt)), ("t", np.ravel(t)), ("psi", psi[idx]), ("q", q[idx])):
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def algorithmic_bytes(nl):
@@ -162,9 +192,9 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm), "source": "nvidia-smi"}
 
 
-def cpu_oracle_run(N, nl, steps, warmup, smoother="lex"):
+def cpu_oracle_run(N, nl, steps, warmup, smoother="lex", dump=None):
     """The CPU oracle built with OpenMP (same algorithm and loop order as the reference,
-    foreach() as an omp-for like `qcc -fopenmp`), on all host cores."""
+    foreach() as an omp-for like `qcc -fopenmp`), on all host cores.  dump: --dump-outputs directory or None."""
     from oracle import oracle as O
     cores = os.cpu_count() or 1
     os.environ.setdefault("OMP_NUM_THREADS", str(cores))
@@ -176,9 +206,11 @@ def cpu_oracle_run(N, nl, steps, warmup, smoother="lex"):
         m.step()
     t0 = time.perf_counter()
     for _ in range(steps):
-        m.step()
+        step_dt = m.step()
     dt = time.perf_counter() - t0
     cyc = m.L.orc_total_cycles(m.h)
+    if dump:
+        dump_outputs(dump, step_dt, m.t, m.get(O.PSI), m.get(O.Q))
     m.close()
     return N * N * nl * steps / dt, dt / steps * 1e3, int(os.environ["OMP_NUM_THREADS"]), cyc
 
@@ -193,11 +225,11 @@ def run_reference(args):
     if os.environ.get("OMP_NUM_THREADS", "1") == "1" and "TORCHELASTIC_RUN_ID" in os.environ:
         os.environ["OMP_NUM_THREADS"] = str(cores)
     # the SAME configuration as our arm: the full args.N^2 x nl grid (4096^2 x 4: a few seconds per step on 16+ cores),
-    # the reference's own sweep (lexicographic, foreach() as an omp-for).  Steps are bounded so that the run ends
-    # within a few minutes whatever K the driver passes; the metric is a rate, so fewer steps do not change it.
-    rsteps, rwarm = max(1, min(args.steps, 5)), max(0, min(args.warmup, 1))
-    val, ms, threads, _ = cpu_oracle_run(args.N, args.nl, rsteps, rwarm, "lex")
-    sample = ("the full %d^2 x nl=%d workload, %d timed steps after %d warm-up (bounded: the CPU takes seconds per step)"
+    # the reference's own sweep (lexicographic, foreach() as an omp-for), --steps timed steps after at most one warm-up
+    # step (the CPU takes seconds per step).
+    rsteps, rwarm = args.steps, max(0, min(args.warmup, 1))
+    val, ms, threads, _ = cpu_oracle_run(args.N, args.nl, rsteps, rwarm, "lex", dump=args.dump_outputs)
+    sample = ("the full %d^2 x nl=%d workload, %d timed steps after %d warm-up (warm-up bounded: the CPU takes seconds per step)"
               % (args.N, args.nl, rsteps, rwarm))
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
@@ -235,13 +267,16 @@ def run_ensemble(args):
     if world > 1:
         dist.barrier()
     t0 = time.perf_counter()
-    ens.step(args.steps)
+    step_dts = ens.step(args.steps)
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
     if world > 1:
         t = torch.tensor([dt], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         dt = float(t.item())
+    if args.dump_outputs:   # one value of dt and t per member, psi and q stacked [member][layer][y][x]
+        dump_outputs(args.dump_outputs, [d[-1] for d in step_dts],
+                     [ens.L.msqg_ensemble_time(ens.h, k) for k in range(len(ens))], ens.get(G.PSI), ens.get(G.Q))
     cycles = sum(m.total_cycles for m in ens.members)
     launches = sum(m.launches for m in ens.members)
     ens.close()
@@ -334,7 +369,7 @@ def run_ours(args):
         with torch.cuda.stream(stream):
             e0.record(stream)
             for _ in range(args.steps):
-                step()
+                step_dt = step()
             e1.record(stream)
         e1.synchronize()
         ms_total = e0.elapsed_time(e1)
@@ -346,6 +381,8 @@ def run_ours(args):
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     cycles, launches = m.total_cycles - c0, m.launches - l0
+    if args.dump_outputs:   # before the untimed passes below advance the state further
+        dump_outputs(args.dump_outputs, step_dt, m.t, m.get(G.PSI), m.get(G.Q))
     ms_total = allmax(ms_total)
     ms_step = ms_total / args.steps
     value = N * N * nl * args.steps / (ms_total * 1e-3)
@@ -570,7 +607,14 @@ def main():
     ap.add_argument("--agg-n", type=int, default=0, dest="agg_n",
                     help="multi-GPU: levels with fewer than agg_n cells per side are not distributed (rb: replicated on every "
                          "GPU, default 512; lex: agglomerated on rank 0, default N)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, dest="dump_outputs",
+                    help="after the timed steps, write what the last one returned as DIR/{dt,t,psi,q}.npy (float64; "
+                         "psi and q as a fixed seeded sample when larger than %d values)" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "ours" and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs supports the single-process run only")
     if args.agg_n <= 0:
         args.agg_n = args.N if args.smoother == "lex" else min(512, args.N)
     global MODAL, PERIODIC, VARRO
