@@ -272,8 +272,10 @@ int msqg_group_create_nccl(const msqg_params *p, int device, int px, int py, int
                            const void *uid128, msqg_group **out);
 /* Periodic boundaries (p->sbc == -1; red-black groups only): every side of every tile is an internal side and the
  * neighbour across a side of the domain is the tile on the opposite side (the tile itself where px or py is 1, in which
- * case msqg_group_create_local_sm accepts px = py = 1); levels up to 32^2 are swept by the single-CTA coarse kernel with
- * wrap-around neighbours, agg_n is chosen by the library.
+ * case msqg_group_create_local_sm accepts px = py = 1).  agg_n is chosen by the library from nl: every replicated level
+ * is swept by the single-CTA coarse kernel with wrap-around neighbours, which holds levels up to 32^2 for nl <= 9 and
+ * up to 16^2 for nl >= 10, so tiles start at 64^2 (nl <= 9) or 32^2 (nl >= 10) cells.  A red-black tile needs >= 16
+ * cells per side there: at nl >= 10 a grid of 4 or more tiles across (4 x 2, 2 x 4, ...) is refused (MSQG_ERR_ARG).
  * The same with the smoother named (msqg_set_smoother): 1 = red-black.  A red-black group gives the bits of the
  * single-GPU red-black solve whatever px, py and agg_n are (a half-sweep is decomposition independent); levels with
  * fewer than agg_n cells per side are replicated on every GPU (all-gather of the restricted residual, redundant coarse

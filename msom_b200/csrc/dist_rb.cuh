@@ -38,7 +38,7 @@ struct HaloPlan {
  *   - two receive buffers alternate (parity of the counter): a tile can be at most one exchange ahead of a neighbour,
  *     because its unpack of exchange e waits for the neighbour's pack of e, which follows the neighbour's unpack of e-1;
  *   - flags only grow, spins are bounded (an error word is raised instead of hanging the GPU). */
-#define XCHG_MAXITEMS 12 /* da of one level + res of every distributed level (a periodic 8192^2 grid has 8 of them) */
+#define XCHG_MAXITEMS 12 /* da of one level + res of every distributed level (a periodic 8192^2 grid has 8 of them, 9 for nl >= 10) */
 #define XCHG_SPIN_NS 4000000000ll
 #define XCHG_EPB 1024 /* elements per block: 256 threads x 4 independent loads */
 struct XItemDev { double *arr; Geom g; int nf, w, ring; long long off[9]; };

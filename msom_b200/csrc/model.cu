@@ -392,6 +392,21 @@ static void fill_geom_consts(Geom &g, double Delta) {
   g.D2x = 2 * g.Delta; g.rD2x = 1. / g.D2x;
 }
 
+/* shared memory of the single-CTA coarse kernel k_coarse_rb, which keeps da and res of levels 1 .. Lc */
+#define RB_COARSE_SMEM (200 * 1024)
+/* the largest Lc (<= RB_COARSE_MAXLEV) whose levels 1 .. Lc fit into k_coarse_rb for nf planes: 5 (32^2) for nf <= 9,
+ * 4 (16^2) for nf = 10 .. 12; 0 if not even levels 1 .. 2 fit */
+static int coarse_max_level(int nf) {
+  int Lc = RB_COARSE_MAXLEV;
+  while (Lc >= 2) {
+    size_t cells = 0;
+    for (int l = 1; l <= Lc; l++) cells += (size_t)1 << (2 * l);
+    if (2 * (size_t)nf * cells * sizeof(double) <= RB_COARSE_SMEM) break;
+    Lc--;
+  }
+  return Lc >= 2 ? Lc : 0;
+}
+
 static int create_model(const msqg_params *p, int device, int px, int py, int ix, int iy, int agg_n, cudaStream_t shared,
                         msqg_model **out, int rb_dist = 0) {
   *out = nullptr;
@@ -433,8 +448,11 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
   m->periodic = per; m->group = nullptr;
   const bool tiled = px * py > 1 || per;
   m->rb_dist = tiled ? rb_dist : 0;
-  if (per) { /* levels <= 32^2 are swept by k_coarse_rb (wrap-around neighbours), everything above lives on tiles */
-    agg_n = p->N < 64 ? p->N : 64;
+  if (per) {
+    /* the replicated levels must all be swept by k_coarse_rb, the only kernel of those levels with wrap-around
+       neighbours: levels up to 32^2 for nl <= 9, up to 16^2 for nl >= 10; everything above lives on tiles */
+    const int top = 2 << coarse_max_level(p->nl);
+    agg_n = p->N < top ? p->N : top;
   }
   if (px * py > 1 && p->sbc > 0) { msqg_destroy(m); FAIL(MSQG_ERR_ARG, "partial slip (sbc > 0) is not supported on decomposed grids"); }
   if (tiled) {
@@ -442,6 +460,13 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
     while ((1 << la) < agg_n) la++;
     const char *why = nullptr;
     if (la > depth) why = "the agglomeration threshold exceeds N";
+    else if (per && (((1 << la) / px) < MSQG_FRAME || ((1 << la) / py) < MSQG_FRAME)) {
+      /* agg_n is not the caller's choice here: it is what the wrap-around coarse kernel holds for this nl */
+      delete m;
+      FAIL(MSQG_ERR_ARG, "a periodic %d^2 x nl=%d grid is replicated on every tile below its %d^2 level (what the wrap-around "
+           "coarse kernel holds for this nl), so %d x %d tiles leave fewer than the %d cells per side a red-black tile needs there",
+           p->N, p->nl, 1 << la, px, py, MSQG_FRAME);
+    }
     else if (((1 << la) / px) < 8 || ((1 << la) / py) < 8) why = "tiles must keep >= 8 cells per side on every distributed level (raise agg_n)";
     else if (rb_dist && (((1 << la) / px) < MSQG_FRAME || ((1 << la) / py) < MSQG_FRAME))
       why = "red-black tiles must keep >= 16 cells per side on every distributed level (raise agg_n)";
@@ -1323,14 +1348,8 @@ static int coarse_top_level(msqg_model *m, int nf_problem, int maxlevel) {
   { const char *e = getenv("MSQG_RB_COARSE_TABLES"); /* A/B: tables through the level-by-level streaming kernel */
     if (e && atoi(e) == 0 && (nf_problem > 1 ? !m->s_uniform : !m->modes_uniform)) return 0; }
   if (!m->periodic) { const char *e = getenv("MSQG_RB_COARSE"); if (e && atoi(e) == 0) return 0; } /* A/B: level-by-level launches */
-  int Lc = RB_COARSE_MAXLEV;
+  int Lc = coarse_max_level(nf_problem);
   if (Lc > maxlevel) Lc = maxlevel;
-  while (Lc >= 2) {
-    size_t cells = 0;
-    for (int l = 1; l <= Lc; l++) cells += (size_t)1 << (2 * l);
-    if (2 * (size_t)nf_problem * cells * sizeof(double) <= 200 * 1024) break;
-    Lc--;
-  }
   return Lc >= 2 ? Lc : 0;
 }
 template <int NL, bool RCOEF = false>
@@ -1354,7 +1373,7 @@ static int launch_coarse_rb(msqg_model *m, int Lc, int nrelax, const CoarseCoef<
   if (!st.set[dev].load(std::memory_order_acquire)) {
     std::lock_guard<std::mutex> lk(g_kernel_init_mu);
     if (!st.set[dev].load(std::memory_order_relaxed)) {
-      CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, RB_COARSE_SMEM));
       st.set[dev].store(true, std::memory_order_release);
     }
   }
@@ -1542,6 +1561,9 @@ static int mg_levels(msqg_model *m, int nf, int mode, int nrelax, int from, int 
   dim3 b(32, 8);
   const int D = m->depth;
   const int Lc = coarse_top_level(m, nf, top < D ? top : D - 1);
+  /* k_prolong4 and the level relax kernels meet dirichlet ghosts on an undecomposed level: with periodic boundaries every
+     level of this loop must be inside the wrap-around coarse kernel (create_model sizes agg_n for that) */
+  if (m->periodic && Lc < top) FAIL(MSQG_ERR_ARG, "periodic level %d is not covered by the wrap-around coarse kernel (levels 1 .. %d)", top, Lc);
   for (int l = from - 1; l >= (Lc ? Lc : 1); l--) {
     ProfScope ps(m, PROF_RESTRICT, l);
     k_restrict<<<grid2(m->g[l].nx, m->g[l].ny, b, nf), b, 0, m->stream>>>(m->res.lev[l + 1], m->res.lev[l], m->g[l + 1], m->g[l], -1., 0);

@@ -62,7 +62,9 @@ def test_decomposition_differs_from_serial_only_at_solver_tolerance(gpu):
 
 
 @pytest.mark.parametrize("N,nl,px,py,agg_n,p2p", [(128, 2, 2, 1, 64, 1), (128, 3, 2, 2, 64, 1), (256, 2, 4, 2, 128, 1), (256, 4, 1, 2, 64, 1),
-                                                   (512, 4, 4, 2, 256, 1), (256, 3, 2, 2, 64, 0), (256, 2, 4, 2, 128, 0)])
+                                                   (512, 4, 4, 2, 256, 1), (256, 3, 2, 2, 64, 0), (256, 2, 4, 2, 128, 0),
+                                                   # 2 and 1 fused sweeps per tile pass (nl 5-8, 9-12), both transports
+                                                   (256, 7, 2, 2, 64, 1), (256, 12, 2, 1, 64, 1), (256, 9, 1, 2, 64, 0)])
 def test_red_black_group_equals_single_gpu_and_oracle(gpu, N, nl, px, py, agg_n, p2p, monkeypatch):
     """Throughput mode on tiles: a red-black half-sweep does not depend on the decomposition, so the group (deep halos,
     one exchange per level, replicated coarse levels) must give the bits of the undecomposed solve and of the oracle

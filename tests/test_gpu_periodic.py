@@ -1,8 +1,9 @@
 """Doubly periodic boundaries, sbc = -1 (msqg/qg.h:80, :842-846: periodic(right); periodic(top), bc_type = -2).
 
 On the GPU the periodic domain runs on the tile machinery of the multi-GPU path: every side of every tile is an internal
-side whose halo comes from the tile across the seam -- the tile itself for px = 1 or py = 1 -- levels up to 32^2 are
-swept by the single-CTA coarse kernel with wrap-around neighbours.  Red-black ordering only (a half-sweep does not
+side whose halo comes from the tile across the seam -- the tile itself for px = 1 or py = 1 -- and the levels below
+the tiles (up to 32^2 for nl <= 9, up to 16^2 for nl >= 10) are swept by the single-CTA coarse kernel with wrap-around
+neighbours.  Red-black ordering only (a half-sweep does not
 depend on where the seam is).  Bit-exact against the oracle, whose boundary() copies the opposite side into the ghost
 ring on every level ([BASILISK] periodic box boundaries)."""
 import numpy as np
@@ -13,8 +14,17 @@ from common import base_kw, periodic_psi
 pytestmark = pytest.mark.gpu
 
 
+def _diff(a, b):
+    d = np.abs(a - b)
+    return "max |difference| %.3e at %d of %d cells" % (d.max(), int((d > 0).sum()), d.size)
+
+
 @pytest.mark.parametrize("N,nl,px,py,over", [(64, 2, 1, 1, {}), (128, 3, 1, 1, dict(Re=200.)), (128, 4, 2, 1, {}), (128, 3, 2, 2, {}),
-                                              (256, 2, 4, 2, dict(Eks=0.001)), (32, 3, 1, 1, {}), (64, 5, 1, 2, {})])
+                                              (256, 2, 4, 2, dict(Eks=0.001)), (32, 3, 1, 1, {}), (64, 5, 1, 2, {}),
+                                              # layer counts whose coarse kernel holds fewer levels (nl >= 10), and 2 or 1
+                                              # fused sweeps per pass of the tile relaxation (nl 5-8, 9-12)
+                                              (64, 10, 1, 1, {}), (128, 12, 2, 1, {}), (64, 11, 2, 2, {}), (128, 6, 1, 1, {}),
+                                              (128, 7, 2, 2, {}), (64, 8, 1, 2, {}), (128, 9, 2, 1, {})])
 def test_periodic_domain_matches_oracle(gpu, N, nl, px, py, over):
     from oracle import oracle as O
     from msom_b200 import capi as G
@@ -25,19 +35,19 @@ def test_periodic_domain_matches_oracle(gpu, N, nl, px, py, over):
     g = Group(G.make_params(**kw), px, py, 0, gpu, smoother="rb")
     mo.set(O.PSI, psi); g.set_global(G.PSI, psi)
     mo.set_const(); g.set_const()
-    assert np.array_equal(g.get_global(G.Q), mo.get(O.Q))
+    assert np.array_equal(g.get_global(G.Q), mo.get(O.Q)), "q: " + _diff(g.get_global(G.Q), mo.get(O.Q))
     z = np.zeros_like(psi)
     mo.set(O.PSI, z); g.set_global(G.PSI, z)
     mo.invertq(); g.invertq()
     so, sg = mo.mgstats(), g.mgstats()
+    assert np.array_equal(g.get_global(G.PSI), mo.get(O.PSI)), "psi after invertq: " + _diff(g.get_global(G.PSI), mo.get(O.PSI))
     assert (sg.i, sg.nrelax, sg.resb, sg.resa) == (so.i, so.nrelax, so.resb, so.resa)
-    assert np.array_equal(g.get_global(G.PSI), mo.get(O.PSI))
     mo.set(O.PSI, psi); g.set_global(G.PSI, psi)
     for _ in range(4):
         assert g.step() == mo.step()
     assert g.total_cycles == mo.L.orc_total_cycles(mo.h)
-    assert np.array_equal(g.get_global(G.Q), mo.get(O.Q))
-    assert np.array_equal(g.get_global(G.PSI), mo.get(O.PSI))
+    assert np.array_equal(g.get_global(G.Q), mo.get(O.Q)), "q: " + _diff(g.get_global(G.Q), mo.get(O.Q))
+    assert np.array_equal(g.get_global(G.PSI), mo.get(O.PSI)), "psi: " + _diff(g.get_global(G.PSI), mo.get(O.PSI))
     # periodic and closed-basin runs of the same initial state differ from the first step on
     kw2 = base_kw(N, nl, **over)
     mc = O.Model(O.make_params(**kw2)); mc.set_smoother("rb")
@@ -87,6 +97,13 @@ def test_periodic_rejects_what_is_not_built(gpu):
         G.Model(G.make_params(**base_kw(64, 2, sbc=-1., upg=[0.1, 0.], vpg=[0., 0.])), gpu)
     with pytest.raises(G.MsqgError):
         G.Model(G.make_params(**base_kw(64, 2, sbc=-1., mode_pv_invert=1)), gpu)
+    # the wrap-around coarse kernel holds levels up to 32^2 for nl <= 9 but only up to 16^2 for nl >= 10: from nl = 10 on
+    # the tiles start at the 32^2 level, which 4 tiles across cannot split into the 16 cells a red-black tile needs
+    Group(G.make_params(**base_kw(128, 9, sbc=-1.)), 4, 2, 0, gpu, smoother="rb").close()
+    with pytest.raises(G.MsqgError, match="periodic"):
+        Group(G.make_params(**base_kw(128, 10, sbc=-1.)), 4, 2, 0, gpu, smoother="rb")
+    with pytest.raises(G.MsqgError, match="periodic"):
+        Group(G.make_params(**base_kw(128, 12, sbc=-1.)), 2, 4, 0, gpu, smoother="rb")
 
 
 def test_periodic_full_size_translation_equivariance(gpu):

@@ -34,7 +34,10 @@ def _level_s(N, nl, level, kw):
 
 @pytest.mark.parametrize("nl,level,nsweeps", [(2, 3, 1), (2, 5, 4), (3, 6, 4), (4, 7, 4), (4, 6, 3), (4, 5, 2), (4, 8, 1),
                                                (3, 7, 7), (2, 6, 13), (10, 5, 4), (4, 1, 4), (4, 2, 5), (2, 8, 4),
-                                               (4, 9, 4), (6, 7, 3), (12, 6, 2), (4, 10, 6)])
+                                               (4, 9, 4), (6, 7, 3), (12, 6, 2), (4, 10, 6),
+                                               # every layer count of the streaming kernel: 2 fused sweeps per pass for nl
+                                               # 5-8 (odd nl: uneven plane split), 1 for nl 9-12; several strips from level 7
+                                               (5, 7, 5), (7, 8, 3), (8, 7, 4), (9, 8, 3), (11, 7, 2), (11, 9, 1)])
 @pytest.mark.parametrize("reuse,tile,wxmin", [(1, 0, 1024), (0, 0, 1024), (1, 512, 1024)])
 def test_relax_rb_matches_oracle(gpu, nl, level, nsweeps, reuse, tile, wxmin, monkeypatch):
     """one level, nsweeps red-black sweeps: strips, row chunks, window halos and multi-pass splits all exercised, with the
@@ -80,7 +83,10 @@ def test_relax_rb_scalar_matches_oracle(gpu, level, nsweeps, lam, tile, monkeypa
     assert np.array_equal(a_gpu, a_ref), np.abs(a_gpu - a_ref).max()
 
 
-@pytest.mark.parametrize("N,nl", [(64, 2), (256, 2), (128, 3), (128, 4), (64, 10)])
+NL_HIGH = range(5, 13)   # layer counts above the one-window relax kernel: 2 (nl <= 8) or 1 fused sweeps per pass
+
+
+@pytest.mark.parametrize("N,nl", [(64, 2), (256, 2), (128, 3), (128, 4), (64, 10)] + [(256, nl) for nl in NL_HIGH])
 def test_invertq_rb(gpu, N, nl):
     from oracle import oracle as O
     from msom_b200 import capi as G
@@ -95,7 +101,8 @@ def test_invertq_rb(gpu, N, nl):
     assert np.array_equal(mg.get(G.PSI), mo.get(O.PSI))
 
 
-@pytest.mark.parametrize("N,nl,nsteps", [(256, 2, 1), (256, 2, 100), (128, 3, 20), (128, 4, 20), (512, 4, 3)])
+@pytest.mark.parametrize("N,nl,nsteps", [(256, 2, 1), (256, 2, 100), (128, 3, 20), (128, 4, 20), (512, 4, 3)]
+                         + [(256, nl, 3) for nl in NL_HIGH])
 def test_steps_rb(gpu, N, nl, nsteps):
     """BASELINE config 1 (256^2 x 2) in throughput mode: 1 and 100 steps, bit-exact against the oracle with the same
     ordering, equal multigrid cycle counts"""
@@ -160,7 +167,8 @@ def test_modal_rb(gpu):
     assert np.array_equal(mg.get(G.Q), mo.get(O.Q))
 
 
-@pytest.mark.parametrize("N,nl,over", [(256, 4, {}), (128, 3, {"mode_pv_invert": 1}), (64, 10, {}), (16, 2, {})])
+@pytest.mark.parametrize("N,nl,over", [(256, 4, {}), (128, 3, {"mode_pv_invert": 1}), (64, 10, {}), (16, 2, {}),
+                                       (128, 9, {}), (128, 12, {})])   # coarse kernel up to 32^2 at nl = 9, up to 16^2 at nl = 12
 def test_fused_coarse_levels_equal_level_by_level(gpu, N, nl, over, monkeypatch):
     """k_coarse_rb (levels up to 32^2 in one launch, restrictions and prolongations included) against the
     level-by-level kernels (MSQG_RB_COARSE=0) and against the oracle: same bits, same cycle counts"""

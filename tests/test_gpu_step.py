@@ -10,7 +10,10 @@ from common import make_pair, rel_l2
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("N,nl", [(64, 2), (256, 2), (128, 3), (128, 4), (64, 10)])
+NL_HIGH = range(5, 13)   # every layer count of the reference-order relax kernel above the common ones
+
+
+@pytest.mark.parametrize("N,nl", [(64, 2), (256, 2), (128, 3), (128, 4), (64, 10)] + [(256, nl) for nl in NL_HIGH])
 def test_set_const_and_invertq(gpu, N, nl):
     from oracle import oracle as O
     from msom_b200 import capi as G
@@ -41,7 +44,7 @@ def test_update_qg(gpu, N, nl):
     assert np.array_equal(mg.get(G.DQ), mo.get(O.DQ))
 
 
-@pytest.mark.parametrize("N,nl,nsteps", [(256, 2, 1), (256, 2, 100), (128, 3, 20), (128, 4, 20)])
+@pytest.mark.parametrize("N,nl,nsteps", [(256, 2, 1), (256, 2, 100), (128, 3, 20), (128, 4, 20)] + [(256, nl, 3) for nl in NL_HIGH])
 def test_steps(gpu, N, nl, nsteps):
     """BASELINE config 1 (256^2 x 2): 1 and 100 steps."""
     from oracle import oracle as O

@@ -76,7 +76,7 @@ def numpy_solve(a, b, s_fine, dh, L0, tol=1e-3, bc=-1):
     return a, stats, hist
 
 
-@pytest.mark.parametrize("N,nl,varRo", [(64, 2, 0), (64, 3, 0), (32, 4, 1)])
+@pytest.mark.parametrize("N,nl,varRo", [(64, 2, 0), (64, 3, 0), (32, 4, 1), (64, 7, 0), (64, 12, 0), (32, 6, 1)])
 def test_inversion_against_numpy_multigrid(N, nl, varRo):
     kw = base_kw(N, nl, varRo=varRo)
     m = O.Model(O.make_params(**kw)); m.set_smoother("rb")
@@ -96,7 +96,7 @@ def test_inversion_against_numpy_multigrid(N, nl, varRo):
     assert so.i >= 1
 
 
-@pytest.mark.parametrize("N,nl", [(32, 2), (64, 3)])
+@pytest.mark.parametrize("N,nl", [(32, 2), (64, 3), (64, 7), (64, 10), (64, 12)])
 def test_periodic_inversion_against_numpy_multigrid(N, nl):
     """sbc = -1: the same solve with wrap-around ghost rings on every level (np.pad(..., mode="wrap") in the numpy
     version, boundary_level() in the oracle) -- relaxation across the seam, prolongation from the wrapped coarse ring,
