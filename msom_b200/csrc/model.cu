@@ -1177,10 +1177,12 @@ static int launch_relax_w_t(msqg_model *m, double *da, const double *res, int le
 
 template <int NL>
 static int launch_relax_rb(msqg_model *m, double *da, const double *res, int lev, int nrelax, const RelaxCoef<NL> &C,
-                           const int *orange, int halo);
+                           const int *orange, int halo, double *corr_a);
 template <int NL>
-static int launch_relax(msqg_model *m, double *da, const double *res, int lev, int nrelax, const RelaxCoef<NL> &C) {
-  if (m->smoother == 1) return launch_relax_rb<NL>(m, da, res, lev, nrelax, C, nullptr, 0);
+static int launch_relax(msqg_model *m, double *da, const double *res, int lev, int nrelax, const RelaxCoef<NL> &C,
+                        double *corr_a = nullptr) {
+  if (m->smoother == 1) return launch_relax_rb<NL>(m, da, res, lev, nrelax, C, nullptr, 0, corr_a);
+  if (corr_a) FAIL(MSQG_ERR_ARG, "the correction is folded into red-black passes only");
   int done = 0;
   while (done < nrelax) {
     int ns = nrelax - done;
@@ -1207,9 +1209,18 @@ static int launch_relax(msqg_model *m, double *da, const double *res, int lev, i
 /* (handles of several host threads -- ensemble members -- may reach a kernel's first launch together: the one-time
    setup is double-checked under g_kernel_init_mu, the flag is published with release / read with acquire) */
 struct KernelDevState { std::atomic<bool> set[64]; int occ[64][RB_NSMAX + 1]; }; /* only ever `static`: zero-initialised */
+/* levels / tiles of at most lim^2 cells go through k_relax_rb_tile instead of the streaming k_relax_rb (nl <= 4) */
+static bool rb_tiled(int nf, bool rcoef, long long cells) {
+  if (nf > 4) return false;
+  int lim = 512;
+  { const char *e = getenv("MSQG_RB_TILE"); if (e) lim = atoi(e); }
+  if (rcoef) { const char *e = getenv("MSQG_RB_COARSE_TABLES"); if (e && atoi(e) == 0) lim = 0; }
+  return cells <= (long long)lim * lim;
+}
 template <int NL, bool RCOEF, int WXT>
 static int launch_relax_rb_pass_w(msqg_model *m, double *da, const double *res, int lev, int ns, const RelaxCoef<NL> &C,
-                                const int *orange /* optional {ox_lo, ox_hi, oy_lo, oy_hi} */, int halo) {
+                                const int *orange /* optional {ox_lo, ox_hi, oy_lo, oy_hi} */, int halo,
+                                double *corr_a = nullptr /* k_relax_rb<..., FOLD = true>: a += da instead of da2 = da */) {
   using Cfg = RbCfg<NL, WXT>;
   const Geom &g = m->g[lev];
   const int nh = 2 * ns;
@@ -1235,12 +1246,16 @@ static int launch_relax_rb_pass_w(msqg_model *m, double *da, const double *res, 
   A.reuse = m->rb_reuse;
   if (RCOEF && (g.bc || !A.coef)) FAIL(MSQG_ERR_ARG, "horizontally varying stretching (varRo, frpg) is supported on undecomposed levels only");
   const int nxo_ = A.ox_hi - A.ox_lo, nyo_ = A.oy_hi - A.oy_lo;
+  const bool fold = corr_a != nullptr;
+  if (fold) {
+    if (orange || halo || g.bc || WXT != RB_WX || rb_tiled(NL, RCOEF, (long long)nxo_ * nyo_))
+      FAIL(MSQG_ERR_ARG, "the correction is folded into streaming passes over a whole undecomposed level only");
+    if (!rb_can_fold(NL)) FAIL(MSQG_ERR_ARG, "nl = %d has no folded relax pass", NL);
+    A.a = corr_a;
+  }
   if constexpr (NL <= 4) {
     /* small levels / tiles: one shared-memory window per CTA instead of the streaming pipeline (k_relax_rb_tile) */
-    int lim = 512;
-    { const char *e = getenv("MSQG_RB_TILE"); if (e) lim = atoi(e); }
-    if (RCOEF) { const char *e = getenv("MSQG_RB_COARSE_TABLES"); if (e && atoi(e) == 0) lim = 0; }
-    if ((long long)nxo_ * nyo_ <= (long long)lim * lim) {
+    if (rb_tiled(NL, RCOEF, (long long)nxo_ * nyo_)) {
       constexpr int WS = RB_TO + 4 * RB_NSMAX;
       const size_t tsmem = (size_t)2 * NL * WS * WS * sizeof(double);
       auto tk = k_relax_rb_tile<NL, RCOEF>;
@@ -1264,8 +1279,10 @@ static int launch_relax_rb_pass_w(msqg_model *m, double *da, const double *res, 
   }
   const size_t smem = (size_t)A.R * Cfg::row_bytes;
   const int threads = Cfg::NSMAX * WXT; /* fixed block: stages beyond nh only stream */
-  auto kern = k_relax_rb<NL, RCOEF, WXT>;
-  static KernelDevState st;
+  auto kern = k_relax_rb<NL, RCOEF, WXT, false>;
+  if constexpr (rb_can_fold(NL) && WXT == RB_WX) { if (fold) kern = k_relax_rb<NL, RCOEF, WXT, true>; }
+  static KernelDevState sts[2];
+  KernelDevState &st = sts[fold ? 1 : 0];
   const int dev = m->device & 63;
   if (!st.set[dev].load(std::memory_order_acquire)) {
     std::lock_guard<std::mutex> lk(g_kernel_init_mu);
@@ -1291,8 +1308,10 @@ static int launch_relax_rb_pass_w(msqg_model *m, double *da, const double *res, 
   kern<<<dim3(nstrips, nchunks), threads, smem, m->stream>>>(A, Cc);
   m->launches++;
   CK(cudaGetLastError());
-  std::swap(m->da.lev[lev], m->da2.lev[lev]);
-  if (m->swap_log) m->swap_log->push_back({m->tile_index, lev});
+  if (!fold) { /* a correcting pass writes no da: da and da2 stay as they were */
+    std::swap(m->da.lev[lev], m->da2.lev[lev]);
+    if (m->swap_log) m->swap_log->push_back({m->tile_index, lev});
+  }
   return MSQG_OK;
 }
 /* window width.  A 64-column window halves the ring so that two CTAs share an SM, but the kernel is bound by
@@ -1301,7 +1320,8 @@ static int launch_relax_rb_pass_w(msqg_model *m, double *da, const double *res, 
  * instance is therefore only built with -DMSQG_EXPERIMENTS (MSQG_RB_WX=64, MSQG_RB_WX_MIN=<smallest level side>). */
 template <int NL, bool RCOEF>
 static int launch_relax_rb_pass(msqg_model *m, double *da, const double *res, int lev, int ns, const RelaxCoef<NL> &C,
-                                const int *orange, int halo) {
+                                const int *orange, int halo, double *corr_a = nullptr) {
+  if (corr_a) return launch_relax_rb_pass_w<NL, RCOEF, RB_WX>(m, da, res, lev, ns, C, orange, halo, corr_a);
 #ifdef MSQG_EXPERIMENTS
   int wx = 128;
   { const char *e = getenv("MSQG_RB_WX"); if (e) wx = atoi(e); }
@@ -1315,10 +1335,11 @@ static int launch_relax_rb_pass(msqg_model *m, double *da, const double *res, in
 #endif
   return launch_relax_rb_pass_w<NL, RCOEF, RB_WX>(m, da, res, lev, ns, C, orange, halo);
 }
-/* nrelax sweeps as ceil(nrelax / NSMAX) passes of (almost) equal length; the result does not depend on the split */
+/* nrelax sweeps as ceil(nrelax / NSMAX) passes of (almost) equal length; the result does not depend on the split.
+ * corr_a (optional): the last pass adds da to this unknown instead of storing da (k_relax_rb<..., FOLD = true>). */
 template <int NL>
 static int launch_relax_rb(msqg_model *m, double *da, const double *res, int lev, int nrelax, const RelaxCoef<NL> &C,
-                           const int *orange = nullptr, int halo = 0) {
+                           const int *orange = nullptr, int halo = 0, double *corr_a = nullptr) {
   constexpr int NSMAX = RbCfg<NL>::NSMAX;
   int left = nrelax;
   if (da != m->da.lev[lev]) FAIL(MSQG_ERR_ARG, "the rb relax pass works on the model's da list");
@@ -1326,12 +1347,13 @@ static int launch_relax_rb(msqg_model *m, double *da, const double *res, int lev
   while (left > 0) {
     const int passes = (left + NSMAX - 1) / NSMAX;
     const int ns = (left + passes - 1) / passes;
+    double *ca = left == ns ? corr_a : nullptr;
     int rc;
     if (relax_uses_table<NL>(m)) {
-      if constexpr (NL <= 6) rc = launch_relax_rb_pass<NL, true>(m, m->da.lev[lev], res, lev, ns, C, orange, halo);
+      if constexpr (NL <= 6) rc = launch_relax_rb_pass<NL, true>(m, m->da.lev[lev], res, lev, ns, C, orange, halo, ca);
       else FAIL(MSQG_ERR_ARG, "varRo > 0 with the layer-coupled solver is built for nl <= 6 (nl = %d)", NL);
     } else
-      rc = launch_relax_rb_pass<NL, false>(m, m->da.lev[lev], res, lev, ns, C, orange, halo);
+      rc = launch_relax_rb_pass<NL, false>(m, m->da.lev[lev], res, lev, ns, C, orange, halo, ca);
     if (rc) return rc;
     left -= ns;
   }
@@ -1557,9 +1579,16 @@ static int mg_corr_residual(msqg_model *m, const MgProblem &P, const double *da,
 /* restriction of res from level `from` down to level 1, then the up-leg of the cycle on levels 1 .. top (da = 0 on
  * level 1, bilinear prolongation, nrelax sweeps).  With the red-black smoother the levels up to 32^2 run as ONE launch
  * (k_coarse_rb), which also does their restrictions. */
-static int mg_levels(msqg_model *m, int nf, int mode, int nrelax, int from, int top) {
+/* MSQG_RB_FOLD=0: a separate k_correct launch instead of the correction folded into the last relax pass (A/B) */
+static bool rb_fold_enabled() { const char *e = getenv("MSQG_RB_FOLD"); return !(e && atoi(e) == 0); }
+/* corrected != NULL (mg_cycle): when level D of an undecomposed grid goes through the streaming red-black kernel, its
+ * last pass adds da to corr_a (no k_correct); *corrected tells the caller whether that happened.  Same bits. */
+static int mg_levels(msqg_model *m, int nf, int mode, int nrelax, int from, int top, double *corr_a = nullptr,
+                     bool *corrected = nullptr) {
   dim3 b(32, 8);
   const int D = m->depth;
+  const bool fold = corrected && m->smoother == 1 && !m->periodic && rb_fold_enabled();
+  if (corrected) *corrected = false;
   const int Lc = coarse_top_level(m, nf, top < D ? top : D - 1);
   /* k_prolong4 and the level relax kernels meet dirichlet ghosts on an undecomposed level: with periodic boundaries every
      level of this loop must be inside the wrap-around coarse kernel (create_model sizes agg_n for that) */
@@ -1597,6 +1626,8 @@ static int mg_levels(msqg_model *m, int nf, int mode, int nrelax, int from, int 
   const int minlevel = top < 1 ? top : 1;
   for (int l = Lc ? Lc + 1 : minlevel; l <= top; l++) {
     const Geom &g = m->g[l];
+    const bool rcoef = mode < 0 ? !m->s_uniform : !m->modes_uniform; /* relax_uses_table of the launches below */
+    double *ca = (fold && l == D && rb_can_fold(nf) && g.bc == 0 && !rb_tiled(nf, rcoef, (long long)g.nx * g.ny)) ? corr_a : nullptr;
     if (l == minlevel) { /* da = 0 on the coarsest level */
       CK(cudaMemsetAsync(m->da.lev[l], 0, (size_t)nf * g.plane * sizeof(double), m->stream));
     } else {
@@ -1607,14 +1638,15 @@ static int mg_levels(msqg_model *m, int nf, int mode, int nrelax, int from, int 
     }
     ProfScope ps(m, l == D ? PROF_RELAX_FINE : PROF_RELAX_COARSE, nrelax);
     if (mode < 0) {
-      NL_SWITCH(m->nl, { auto C = relax_coef_layers<NL>(m, l); rc = launch_relax<NL>(m, m->da.lev[l], m->res.lev[l], l, nrelax, C); });
+      NL_SWITCH(m->nl, { auto C = relax_coef_layers<NL>(m, l); rc = launch_relax<NL>(m, m->da.lev[l], m->res.lev[l], l, nrelax, C, ca); });
     } else {
       auto C = relax_coef_scalar(m, l, m->lam_lev[(size_t)l * m->nl + mode]);
       m->coef_mode = m->modes_uniform ? -1 : mode;
-      rc = launch_relax<1>(m, m->da.lev[l], m->res.lev[l], l, nrelax, C);
+      rc = launch_relax<1>(m, m->da.lev[l], m->res.lev[l], l, nrelax, C, ca);
       m->coef_mode = -1;
     }
     if (rc) return rc;
+    if (ca) *corrected = true;
   }
   return MSQG_OK;
 }
@@ -1623,9 +1655,10 @@ static int mg_cycle(msqg_model *m, const MgProblem &P, int nrelax, int fused = 0
   const int D = m->depth;
   dim3 b(32, 8);
   /* restriction(res): levels D-1..1 (level 0 is never read with minlevel = 1), then levels 1 .. D */
-  int rc = mg_levels(m, P.nf, P.mode, nrelax, fused ? D - 1 : D, D);
+  bool corrected = false;
+  int rc = mg_levels(m, P.nf, P.mode, nrelax, fused ? D - 1 : D, D, fused ? nullptr : P.a, fused ? nullptr : &corrected);
   if (rc) return rc;
-  if (fused == 2) return MSQG_OK;
+  if (fused == 2 || corrected) return MSQG_OK; /* corrected: the last relax pass on level D did a += da */
   const Geom &g = m->g[D];
   { ProfScope ps(m, PROF_CORRECT, 0);
   k_correct<<<grid2(g.nx, g.ny, b, P.nf), b, 0, m->stream>>>(P.a, m->da.lev[D], g); }

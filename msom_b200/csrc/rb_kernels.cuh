@@ -54,11 +54,20 @@ struct RbArgs {
   const double *coef; /* RCOEF: per-row [ny][6][NL] or per-cell [ny][nx][6][NL] Thomas coefficients (k_rowcoef) */
   int coef_cell;
   int reuse;          /* 1: south / in-pair neighbours from registers (default); 0: always from shared memory */
+  double *a;          /* k_relax_rb<..., FOLD = true>, last pass on the finest level of an undecomposed grid: the store is
+                         a += da with the dirichlet ghost ring of a (k_correct) instead of da_out = da; da_out is not
+                         written */
 };
 
 __device__ __forceinline__ void cp_async8(unsigned smem_addr, const void *gsrc) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(smem_addr), "l"(gsrc));
 }
+
+/* sweeps per pass: bounded by the ring (4 ns + 1 + RB_PF rows <= 227 KB) and by registers (threads = 128 ns) */
+__host__ __device__ constexpr int rb_nsmax(int nl) { return nl <= 4 ? RB_NSMAX : (nl <= 8 ? 2 : 1); }
+/* layer counts with a FOLD instance of k_relax_rb: the single-stage instances (nl > 8) are at the register limit
+   already (the prefetched values of a would spill), their finest levels keep the separate k_correct launch */
+__host__ __device__ constexpr bool rb_can_fold(int nl) { return rb_nsmax(nl) > 1; }
 
 template <int NL, int WXT = RB_WX>
 struct RbCfg {
@@ -66,14 +75,13 @@ struct RbCfg {
   static constexpr int ARR2 = NL2 * WXT;            /* double2 per array per ring row */
   static constexpr int ROW2 = 2 * ARR2;             /* double2 per ring row: da, then res */
   static constexpr size_t row_bytes = (size_t)ROW2 * 16;
-  /* sweeps per pass: bounded by the ring (4 ns + 1 + RB_PF rows <= 227 KB) and by registers (threads = 128 ns) */
-  static constexpr int NSMAX = NL <= 4 ? RB_NSMAX : (NL <= 8 ? 2 : 1);
+  static constexpr int NSMAX = rb_nsmax(NL);
   static_assert((size_t)(4 * NSMAX + 1 + RB_PF) * row_bytes <= 227 * 1024, "ring does not fit");
 };
 
 /* WXT: window columns, 128 or 64.  The narrow window halves the ring, so two CTAs share an SM (twice the warps to hide
  * the latency of the Thomas recurrence) at the price of more halo redundancy (64/48 instead of 128/112 at ns = 4). */
-template <int NL, bool RCOEF, int WXT = RB_WX>
+template <int NL, bool RCOEF, int WXT = RB_WX, bool FOLD = false>
 __global__ void __launch_bounds__(RbCfg<NL, WXT>::NSMAX * WXT, WXT == 64 ? 2 : 1)
 k_relax_rb(RbArgs A, RelaxCoef<NL> C) {
   using Cfg = RbCfg<NL, WXT>;
@@ -81,6 +89,7 @@ k_relax_rb(RbArgs A, RelaxCoef<NL> C) {
   constexpr int NL2 = Cfg::NL2, ARR2 = Cfg::ARR2, ROW2 = Cfg::ROW2;
   constexpr int EPT = (2 * NL + NSMAX - 1) / NSMAX; /* planes (da: 0..NL-1, res: NL..2NL-1) streamed per thread */
   constexpr int EPO = (NL + NSMAX - 1) / NSMAX;     /* planes stored per thread */
+  static_assert(!FOLD || rb_can_fold(NL), "no FOLD instance for this layer count");
   extern __shared__ double2 ring[];
   /* the block always has NSMAX * 128 threads: stages k >= nh only help with the streaming */
   const int tid = threadIdx.x;
@@ -116,6 +125,7 @@ k_relax_rb(RbArgs A, RelaxCoef<NL> C) {
     src[i] = (arr ? A.res : A.da) + (pok[i] ? (long long)l * plane + (long long)(jw0 + 1) * pitch + MSQG_OX + gxl : 0);
     dofs[i] = (unsigned)((arr * 2 * ARR2 + (l >> 1) * 2 * WX + (l & 1) + colofs) * 8);
   }
+  const bool corr = FOLD && A.a != nullptr; /* correction out: the store goes to a (+= da), not to da_out */
   double *dst[EPO];
   unsigned sofs[EPO];
   bool sok[EPO];
@@ -123,7 +133,7 @@ k_relax_rb(RbArgs A, RelaxCoef<NL> C) {
   for (int i = 0; i < EPO; i++) {
     const int q = q0 + i * NSMAX;
     sok[i] = ovalid && q < NL;
-    dst[i] = A.da_out + (sok[i] ? (long long)q * plane + (long long)(jw0 + 1) * pitch + MSQG_OX + gxl : 0);
+    dst[i] = (corr ? A.a : A.da_out) + (sok[i] ? (long long)q * plane + (long long)(jw0 + 1) * pitch + MSQG_OX + gxl : 0);
     sofs[i] = (unsigned)((q >> 1) * 2 * WX + (q & 1) + colofs);
   }
   int ld_row = 0;      /* next window row to fetch */
@@ -173,8 +183,13 @@ k_relax_rb(RbArgs A, RelaxCoef<NL> C) {
   double F0[NL], F1[NL], F2[NL];
 #pragma unroll
   for (int l = 0; l < NL; l++) { F0[l] = 0.; F1[l] = 0.; F2[l] = 0.; }
+  /* correction out: a of the row stored at step t is loaded at step t - 3 (HBM latency under full bandwidth is more
+     than one step) into the buffer of step t mod 3, rotated by the same three-step unroll as the FIFO above */
+  double A0[EPO], A1[EPO], A2[EPO];
+#pragma unroll
+  for (int i = 0; i < EPO; i++) { A0[i] = 0.; A1[i] = 0.; A2[i] = 0.; }
 
-  auto step = [&](double (&Fn)[NL], double (&Fi)[NL], double (&Fs)[NL]) {
+  auto step = [&](double (&Fn)[NL], double (&Fi)[NL], double (&Fs)[NL], double (&Av)[EPO]) {
     load_row();
     if (stage_on && (unsigned)r < (unsigned)nrw) {
       const unsigned rowc = ring_s + slB;
@@ -270,8 +285,31 @@ k_relax_rb(RbArgs A, RelaxCoef<NL> C) {
         if (sok[i]) {
           double v;
           asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(ring_s + soB + sofs[i] * 8u));
-          *dst[i] = v;
+          if (FOLD && corr) {
+            /* k_correct: a += da (a first), then the dirichlet ghost ring of a: -w on the sides, +w at the corners */
+            const double w = Av[i] + v;
+            double *pa = dst[i];
+            *pa = w;
+            const int gy = jw0 + ro;
+            const bool gl = gxl == 0, gr = gxl == nx - 1, gb = gy == 0, gt = gy == ny - 1;
+            if (gl) pa[-1] = -w;
+            if (gr) pa[1] = -w;
+            if (gb) pa[-pitch] = -w;
+            if (gt) pa[pitch] = -w;
+            if (gl && gb) pa[-pitch - 1] = w;
+            if (gl && gt) pa[pitch - 1] = w;
+            if (gr && gb) pa[-pitch + 1] = w;
+            if (gr && gt) pa[pitch + 1] = w;
+          } else {
+            *dst[i] = v;
+          }
         }
+    }
+    if (FOLD && corr && ro + 3 >= ro_lo && ro + 3 < ro_hi) { /* a of the row stored three steps later (ro starts <= -4) */
+      const int ahead = ro >= 0 ? 3 : ro + 3;                  /* dst points at row max(ro, 0) */
+#pragma unroll
+      for (int i = 0; i < EPO; i++)
+        if (sok[i]) Av[i] = dst[i][(long long)ahead * pitch];
     }
     if (ro >= 0) {
 #pragma unroll
@@ -285,9 +323,9 @@ k_relax_rb(RbArgs A, RelaxCoef<NL> C) {
 
 #pragma unroll 1
   for (int t = 0; t < T; t += 3) {
-    step(F0, F2, F1);
-    if (t + 1 < T) step(F1, F0, F2);
-    if (t + 2 < T) step(F2, F1, F0);
+    step(F0, F2, F1, A0);
+    if (t + 1 < T) step(F1, F0, F2, A1);
+    if (t + 2 < T) step(F2, F1, F0, A2);
   }
   cp_async_wait<0>();
 }
