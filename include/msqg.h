@@ -279,7 +279,10 @@ int msqg_group_create_nccl(const msqg_params *p, int device, int px, int py, int
  * The same with the smoother named (msqg_set_smoother): 1 = red-black.  A red-black group gives the bits of the
  * single-GPU red-black solve whatever px, py and agg_n are (a half-sweep is decomposition independent); levels with
  * fewer than agg_n cells per side are replicated on every GPU (all-gather of the restricted residual, redundant coarse
- * solve) and the sweeps of a distributed level need ONE halo exchange (deep halos, communication-avoiding). */
+ * solve) and the sweeps of a distributed level need ONE halo exchange (deep halos, communication-avoiding).
+ * Groups run the layer-coupled inversion; a closed-basin red-black group also runs the vertical-mode inversion
+ * (p->mode_pv_invert) when the modes are uniform: varRo <= 0 and the same Fr on every tile (msqg_group_set_const checks
+ * it).  Refused with MSQG_ERR_ARG: stochastic forcing, modal inversion on a lexicographic or periodic group. */
 int msqg_group_create_local_sm(const msqg_params *p, int device, int px, int py, int agg_n, int smoother, msqg_group **out);
 int msqg_group_create_nccl_sm(const msqg_params *p, int device, int px, int py, int agg_n, int smoother, int rank, int nranks,
                               const void *uid128, msqg_group **out);
@@ -296,6 +299,8 @@ int msqg_group_set_const(msqg_group *g);
 int msqg_group_invertq(msqg_group *g, int q_id);
 int msqg_group_step(msqg_group *g, double t, double tnext, double *dt_out, double *tnext_out);
 int msqg_group_last_mgstats(msqg_group *g, msqg_mgstats *out);
+/* as msqg_last_mgstats: mode < 0 the last solve, else the solve of that vertical mode (mode_pv_invert) */
+int msqg_group_last_mode_mgstats(msqg_group *g, int mode, msqg_mgstats *out);
 long msqg_group_total_cycles(msqg_group *g);
 long msqg_group_exchanges(msqg_group *g);
 long msqg_group_launches(msqg_group *g);

@@ -136,7 +136,7 @@ struct msqg_group {
   ncclComm_t comm;
   double *d_red, *h_red; /* reduction scratch (device / pinned host), 64 doubles */
   double ts_previous;
-  msqg_mgstats mgpsi;
+  msqg_mgstats mgpsi, mgmode[MSQG_MAXL]; /* last solve; per vertical mode (mode_pv_invert) */
   long total_cycles;
   double umax_pg[MSQG_MAXL];
   long exchanges;
@@ -330,13 +330,21 @@ static int group_create(const msqg_params *p, int device, int px, int py, int ag
   const int per = p->sbc == -1;
   if (px * py < 2 && !per) FAIL(MSQG_ERR_ARG, "a group needs px*py >= 2 tiles");
   if (per && smoother != 1) FAIL(MSQG_ERR_ARG, "periodic boundaries (sbc = -1) need the red-black smoother");
-  if (p->mode_pv_invert || p->stochastic) FAIL(MSQG_ERR_ARG, "decomposed grids support the layer-coupled, deterministic path only");
+  if (p->stochastic) FAIL(MSQG_ERR_ARG, "stochastic forcing is not built on decomposed grids");
+  if (p->mode_pv_invert) {
+    /* the vertical-mode inversion runs the red-black cycle once per mode; the lexicographic tile sweep has no modal solve */
+    if (smoother != 1) FAIL(MSQG_ERR_ARG, "the vertical-mode inversion (mode_pv_invert) on tiles needs the red-black smoother");
+    if (per) FAIL(MSQG_ERR_ARG, "the vertical-mode inversion (mode_pv_invert) is not built for periodic boundaries");
+    if (p->varRo > 0)
+      FAIL(MSQG_ERR_ARG, "the vertical-mode inversion (mode_pv_invert) on tiles needs uniform vertical modes: varRo > 0 makes them vary with y");
+  }
   if (kind == 1 && nranks != px * py) FAIL(MSQG_ERR_ARG, "nranks must equal px*py");
   msqg_group *G = new msqg_group();
   G->p = *p; G->px = px; G->py = py; G->agg_n = agg_n; G->device = device; G->kind = kind;
   G->rank = rank; G->nranks = nranks; G->nccl = nullptr; G->comm = nullptr; G->rb = smoother == 1;
   G->ts_previous = 0.; G->total_cycles = 0; G->exchanges = 0;
   memset(&G->mgpsi, 0, sizeof(G->mgpsi));
+  memset(G->mgmode, 0, sizeof(G->mgmode));
   memset(G->umax_pg, 0, sizeof(G->umax_pg));
   CK(cudaSetDevice(device));
   CK(cudaStreamCreateWithFlags(&G->stream, cudaStreamNonBlocking));
@@ -412,26 +420,46 @@ extern "C" long msqg_group_total_cycles(msqg_group *G) { return G->total_cycles;
 extern "C" long msqg_group_exchanges(msqg_group *G) { return G->exchanges; }
 extern "C" long msqg_group_launches(msqg_group *G) { long s = 0; for (msqg_model *m : G->tiles) s += m->launches; return s; }
 extern "C" int msqg_group_last_mgstats(msqg_group *G, msqg_mgstats *out) { *out = G->mgpsi; return MSQG_OK; }
+extern "C" int msqg_group_last_mode_mgstats(msqg_group *G, int mode, msqg_mgstats *out) {
+  if (mode >= G->p.nl) FAIL(MSQG_ERR_ARG, "bad mode");
+  *out = mode < 0 ? G->mgpsi : G->mgmode[mode];
+  return MSQG_OK;
+}
 extern "C" int msqg_group_set_stream_sync(msqg_group *G) { CK(cudaStreamSynchronize(G->stream)); return MSQG_OK; }
 
 /* ------------------------------------------------------------------ multigrid on tiles */
-static int g_residual_enqueue(msqg_group *G, int q_id) {
+/* the problem of every tile: the layer-coupled solve psi <- q_id (mode < 0), or vertical mode `mode`, pm <- qm */
+static std::vector<MgProblem> g_problem(msqg_group *G, int mode, int q_id) {
+  std::vector<MgProblem> P;
   for (msqg_model *m : G->tiles) {
     const int D = m->depth;
+    const size_t pl = m->g[D].plane;
+    if (mode < 0) P.push_back(MgProblem{m->nl, -1, m->psi.lev[D], list_by_id(m, q_id)->lev[D]});
+    else P.push_back(MgProblem{1, mode, m->pm.lev[D] + (size_t)mode * pl, m->qm.lev[D] + (size_t)mode * pl});
+  }
+  return P;
+}
+static int g_residual_enqueue(msqg_group *G, const std::vector<MgProblem> &P) {
+  for (int t = 0; t < (int)G->tiles.size(); t++) {
+    msqg_model *m = G->tiles[t];
+    const int D = m->depth;
     const Geom &g = m->g[D];
-    List *ql = list_by_id(m, q_id);
     CK(zero_words(G->stream, m->d_scal, 1));
     dim3 b(64, 4);
-    LayerMetrics M = metrics_of(m);
     ProfScope ps(m, PROF_RESIDUAL, 0);
-    NL_SWITCH(m->nl, k_residual<NL><<<grid2(g.nx, g.ny, b), b, 0, G->stream>>>(m->psi.lev[D], ql->lev[D], m->res.lev[D], m->str.lev[D], g, M, m->d_scal));
+    if (P[t].mode < 0) {
+      LayerMetrics M = metrics_of(m);
+      NL_SWITCH(m->nl, k_residual<NL><<<grid2(g.nx, g.ny, b), b, 0, G->stream>>>(P[t].a, P[t].b, m->res.lev[D], m->str.lev[D], g, M, m->d_scal));
+    } else
+      k_residual_scalar<<<grid2(g.nx, g.ny, b), b, 0, G->stream>>>(P[t].a, P[t].b, m->res.lev[D], m->ibu.lev[D] + (size_t)P[t].mode * g.plane, g,
+                                                                   m->d_scal);
     m->launches++;
   }
   CK(cudaGetLastError());
   return reduce_max_enqueue(G, 0, 1);
 }
-static int g_residual(msqg_group *G, int q_id, double *maxres) {
-  int rc = g_residual_enqueue(G, q_id);
+static int g_residual(msqg_group *G, const std::vector<MgProblem> &P, double *maxres) {
+  int rc = g_residual_enqueue(G, P);
   if (rc) return rc;
   return reduce_max_finish(G, 1, maxres);
 }
@@ -553,40 +581,35 @@ static int g_check_err(msqg_group *G) {
 
 #include "dist_rb.cuh"
 
-/* mg_solve + poisson_layer + invertq on the decomposed grid */
-static int g_invertq(msqg_group *G, int q_id) {
-  for (msqg_model *m : G->tiles) {
-    if (!m->const_set) FAIL(MSQG_ERR_ARG, "set_const must be called before invertq");
-    if (!m->s_uniform) FAIL(MSQG_ERR_ARG, "horizontally varying stretching is not supported by the relax kernel yet");
-  }
+/* mg_solve on the decomposed grid: problem P[t] on tile t (NITERMIN 1, NITERMAX 100, nrelax starts at 4) */
+static int g_solve(msqg_group *G, const std::vector<MgProblem> &P, msqg_mgstats *st) {
   int rc;
-  if ((rc = exchange_list(G, MSQG_PSI, G->tiles[0]->depth))) return rc;
   msqg_mgstats s;
   memset(&s, 0, sizeof(s));
   s.nrelax = 4;
   double resb;
-  if ((rc = g_residual(G, q_id, &resb))) return rc;
+  if ((rc = g_residual(G, P, &resb))) return rc;
   s.resb = s.resa = resb;
   for (s.i = 0; s.i < 100 && (s.i < 1 || s.resa > 1e-3); s.i++) {
     if (G->rb) {
-      /* one cycle + residual + its all-reduce: a single graph launch (keyed by nrelax, the right-hand side and the
-         current da buffers of every tile) */
+      /* one cycle + residual + its all-reduce: a single graph launch (keyed by nrelax, the mode, the unknown and the
+         right-hand side of tile 0 and the current da buffers of every tile) */
       msqg_model *m0 = G->tiles[0];
       unsigned long long mask = 0;
       for (msqg_model *m : G->tiles) mask = mask * 1315423911ull + da_parity_mask(m);
       bool graphed = m0->use_graphs != 0;
       for (msqg_model *m : G->tiles) graphed = graphed && !m->prof_on;
-      GraphKey key(s.nrelax, -1, (const void *)m0->psi.lev[m0->depth], (const void *)list_by_id(m0, q_id)->lev[m0->depth], mask);
+      GraphKey key(s.nrelax, P[0].mode, (const void *)P[0].a, (const void *)P[0].b, mask);
       rc = run_graphed(G->stream, G->graphs, key, G->tiles, &G->exchanges, graphed, [&]() -> int {
-        int r2 = g_cycle_rb(G, s.nrelax);
+        int r2 = g_cycle_rb(G, P, s.nrelax);
         if (r2) return r2;
-        return g_residual_enqueue(G, q_id);
+        return g_residual_enqueue(G, P);
       });
       if (rc) return rc;
       if ((rc = reduce_max_finish(G, 1, &s.resa))) return rc;
     } else {
       if ((rc = g_cycle(G, s.nrelax))) return rc;
-      if ((rc = g_residual(G, q_id, &s.resa))) return rc;
+      if ((rc = g_residual(G, P, &s.resa))) return rc;
     }
     if (s.resa > 1e-3) {
       if (resb / s.resa < 1.2 && s.nrelax < 100) s.nrelax++;
@@ -597,7 +620,52 @@ static int g_invertq(msqg_group *G, int q_id) {
   if ((rc = g_check_err(G))) return rc;
   if ((rc = group_check_p2p(G))) return rc;
   G->total_cycles += s.i;
-  G->mgpsi = s;
+  *st = s;
+  return MSQG_OK;
+}
+
+/* poisson_layer + invertq on the decomposed grid (invertq_list's order) */
+static int g_invertq(msqg_group *G, int q_id) {
+  for (msqg_model *m : G->tiles) {
+    if (!m->const_set) FAIL(MSQG_ERR_ARG, "set_const must be called before invertq");
+    if (!m->s_uniform) FAIL(MSQG_ERR_ARG, "horizontally varying stretching is not supported by the relax kernel yet");
+  }
+  const int D = G->tiles[0]->depth;
+  int rc;
+  if (!G->p.mode_pv_invert) {
+    if ((rc = exchange_list(G, MSQG_PSI, D))) return rc; /* the warm start's ring */
+    return g_solve(G, g_problem(G, -1, q_id), &G->mgpsi);
+  }
+  /* vertical modes (uniform on tiles: group_create and set_const refuse the others, so the matrices are constants) */
+  if ((rc = exchange_list(G, MSQG_PM, D))) return rc; /* the warm start's ring, every mode */
+  dim3 b(64, 4), bg(32, 8);
+  for (msqg_model *m : G->tiles) {
+    const Geom &g = m->g[D];
+    NL_SWITCH(m->nl, {
+      ModeMat<NL> M;
+      for (int k = 0; k < NL * NL; k++) M.a[k] = m->h_cl2m[k];
+      k_project<NL><<<grid2(g.nx, g.ny, b), b, 0, G->stream>>>(list_by_id(m, q_id)->lev[D], m->qm.lev[D], g, M, nullptr, 0);
+    });
+    m->launches++;
+  }
+  CK(cudaGetLastError());
+  for (int l = 0; l < G->p.nl; l++) {
+    if ((rc = g_solve(G, g_problem(G, l, q_id), &G->mgmode[l]))) return rc;
+    G->mgpsi = G->mgmode[l];
+  }
+  /* psi on the interior and on the ring of the internal sides: each mode's k_correct_ring left the owner's bits of pm
+     there, so the neighbour's psi needs no exchange; then the ghosts of the physical sides */
+  for (msqg_model *m : G->tiles) {
+    const Geom &g = m->g[D];
+    NL_SWITCH(m->nl, {
+      ModeMat<NL> M;
+      for (int k = 0; k < NL * NL; k++) M.a[k] = m->h_cm2l[k];
+      k_project<NL, true><<<grid2(g.nx + 2, g.ny + 2, b), b, 0, G->stream>>>(m->pm.lev[D], m->psi.lev[D], g, M, nullptr, 0);
+    });
+    k_ghosts<<<grid2(g.nx + 2, g.ny + 2, bg, m->nl), bg, 0, G->stream>>>(m->psi.lev[D], m->nl, g, -1.);
+    m->launches += 2;
+  }
+  CK(cudaGetLastError());
   return MSQG_OK;
 }
 extern "C" int msqg_group_invertq(msqg_group *G, int q_id) {
@@ -612,6 +680,35 @@ extern "C" int msqg_group_set_field(msqg_group *G, int t, int id, const double *
 extern "C" int msqg_group_get_field(msqg_group *G, int t, int id, double *host_tile) {
   return msqg_get_field(G->tiles[t], id, host_tile);
 }
+/* Uniform vertical modes are computed by every tile from its own Fr (set_const_local): a Fr field that is constant on
+ * each tile but differs between tiles would give the tiles different matrices and a wrong result without any error.
+ * So every tile and rank must have used the same Fr bits.  reduce_max takes maxima of non-negative words, so each value
+ * goes in as its two 32-bit halves h and their complements 2^32 - 1 - h: max(h) + max(2^32 - 1 - h) = 2^32 - 1 exactly
+ * when h is the same everywhere. */
+static int g_check_modes_agree(msqg_group *G) {
+  const int nl = G->p.nl, n = 4 * (nl - 1), nt = (int)G->tiles.size();
+  const double ones = 4294967295.;
+  std::vector<double> w((size_t)nt * n), out(n);
+  for (int t = 0; t < nt; t++) {
+    msqg_model *m = G->tiles[t];
+    const size_t tc = (size_t)m->tnx * m->tny;
+    double *wt = &w[(size_t)t * n];
+    for (int l = 0; l < nl - 1; l++) {
+      unsigned long long u;
+      memcpy(&u, &m->h_fr[(size_t)l * tc], sizeof(u));
+      const double hi = (double)(u >> 32), lo = (double)(u & 0xffffffffull);
+      wt[4 * l] = hi; wt[4 * l + 1] = ones - hi; wt[4 * l + 2] = lo; wt[4 * l + 3] = ones - lo;
+    }
+    CK(cudaMemcpyAsync(m->d_scal + 1, wt, n * sizeof(double), cudaMemcpyHostToDevice, G->stream));
+  }
+  int rc = reduce_max(G, 1, n, out.data());
+  if (rc) return rc;
+  for (int k = 0; k < n; k += 2)
+    if (out[k] + out[k + 1] != ones)
+      FAIL(MSQG_ERR_ARG, "Fr of interface %d differs between tiles: the vertical-mode inversion on tiles needs the same Fr "
+                         "everywhere (uniform vertical modes)", k / 4);
+  return MSQG_OK;
+}
 extern "C" int msqg_group_set_const(msqg_group *G) {
   CK(cudaSetDevice(G->device));
   G->graphs.clear();
@@ -619,6 +716,7 @@ extern "C" int msqg_group_set_const(msqg_group *G) {
   const int D = G->tiles[0]->depth;
   for (msqg_model *m : G->tiles)
     if ((rc = set_const_local(m))) return rc;
+  if (G->p.mode_pv_invert && (rc = g_check_modes_agree(G))) return rc;
   for (int id : {MSQG_PSI, MSQG_PSIPG, MSQG_TOPO})
     if ((rc = exchange_list(G, id, D))) return rc;
   for (msqg_model *m : G->tiles)

@@ -352,9 +352,11 @@ __global__ void k_correct_ring(double *__restrict__ a, const double *__restrict_
   a[c] = a[c] + da[c];
 }
 
-static int g_cycle_rb(msqg_group *G, int nrelax) {
+/* one cycle of the problem P[t] of every tile t: the layer-coupled solve (nl, -1, psi, q) or the scalar Helmholtz
+ * solve of one vertical mode (1, mode, plane `mode` of pm, of qm) */
+static int g_cycle_rb(msqg_group *G, const std::vector<MgProblem> &P, int nrelax) {
   msqg_model *m0 = G->tiles[0];
-  const int D = m0->depth, La = m0->agg_level, nl = G->p.nl;
+  const int D = m0->depth, La = m0->agg_level, nf = P[0].nf, mode = P[0].mode;
   const int nt = (int)G->tiles.size(), nranks = G->px * G->py;
   dim3 b(32, 8);
   int rc;
@@ -362,17 +364,17 @@ static int g_cycle_rb(msqg_group *G, int nrelax) {
   for (msqg_model *m : G->tiles) {
     for (int l = D - 1; l >= La; l--) {
       ProfScope ps(m, PROF_RESTRICT, l);
-      k_restrict<<<grid2(m->g[l].nx, m->g[l].ny, b, nl), b, 0, G->stream>>>(m->res.lev[l + 1], m->res.lev[l], m->g[l + 1], m->g[l], -1., 0);
+      k_restrict<<<grid2(m->g[l].nx, m->g[l].ny, b, nf), b, 0, G->stream>>>(m->res.lev[l + 1], m->res.lev[l], m->g[l + 1], m->g[l], -1., 0);
       m->launches++;
     }
-    k_restrict<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nl), b, 0, G->stream>>>(m->res.lev[La], m->res_patch, m->g[La], m->gpatch, -1., 0);
-    k_unpack<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nl), b, 0, G->stream>>>(m->patch_stage, m->res_patch, nl, m->gpatch);
+    k_restrict<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nf), b, 0, G->stream>>>(m->res.lev[La], m->res_patch, m->g[La], m->gpatch, -1., 0);
+    k_unpack<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nf), b, 0, G->stream>>>(m->patch_stage, m->res_patch, nf, m->gpatch);
     m->launches += 2;
   }
   CK(cudaGetLastError());
   /* every tile receives every tile's block of level La-1 (all-gather) and assembles the full level */
   const int hx = m0->gpatch.nx, hy = m0->gpatch.ny;
-  const size_t blk = (size_t)nl * hx * hy;
+  const size_t blk = (size_t)nf * hx * hy;
   if (G->kind == 0) {
     for (msqg_model *m : G->tiles)
       for (int r = 0; r < nt; r++)
@@ -384,13 +386,13 @@ static int g_cycle_rb(msqg_group *G, int nrelax) {
   const int chunk0 = nrelax < 7 ? nrelax : 7;
   /* replicated coarse levels: every tile solves levels 1 .. La-1 (same arithmetic, same bits everywhere) */
   for (msqg_model *m : G->tiles) {
-    k_place_all<<<grid2(hx, hy, b, nranks * nl), b, 0, G->stream>>>(m->res.lev[La - 1], m->g[La - 1], m->gather_buf, hx, hy, G->px, nranks, nl);
+    k_place_all<<<grid2(hx, hy, b, nranks * nf), b, 0, G->stream>>>(m->res.lev[La - 1], m->g[La - 1], m->gather_buf, hx, hy, G->px, nranks, nf);
     m->launches++;
-    if ((rc = mg_levels(m, nl, -1, nrelax, La - 1, La - 1))) return rc;
+    if ((rc = mg_levels(m, nf, mode, nrelax, La - 1, La - 1))) return rc;
     /* this tile's block of level La-1 plus a one-cell ring (homogeneous dirichlet ghosts evaluated on the fly) */
-    k_extract_patch<<<grid2(hx + 2, hy + 2, b, nl), b, 0, G->stream>>>(m->da.lev[La - 1], m->g[La - 1], m->patch_stage, hx, hy, m->ix * hx, m->iy * hy,
+    k_extract_patch<<<grid2(hx + 2, hy + 2, b, nf), b, 0, G->stream>>>(m->da.lev[La - 1], m->g[La - 1], m->patch_stage, hx, hy, m->ix * hx, m->iy * hy,
                                                                         m->periodic);
-    k_load_patch<<<grid2(hx + 2, hy + 2, b, nl), b, 0, G->stream>>>(m->da_patch, m->gpatch, m->patch_stage);
+    k_load_patch<<<grid2(hx + 2, hy + 2, b, nf), b, 0, G->stream>>>(m->da_patch, m->gpatch, m->patch_stage);
     m->launches += 2;
   }
   CK(cudaGetLastError());
@@ -398,8 +400,8 @@ static int g_cycle_rb(msqg_group *G, int nrelax) {
   for (int l = La; l <= D; l++) {
     for (msqg_model *m : G->tiles) {
       ProfScope ps(m, PROF_PROLONG, l);
-      if (l == La) launch_prolong(G->stream, nl, m->da_patch, m->da.lev[l], m->gpatch, m->g[l]);
-      else launch_prolong(G->stream, nl, m->da.lev[l - 1], m->da.lev[l], m->g[l - 1], m->g[l]);
+      if (l == La) launch_prolong(G->stream, nf, m->da_patch, m->da.lev[l], m->gpatch, m->g[l]);
+      else launch_prolong(G->stream, nf, m->da.lev[l - 1], m->da.lev[l], m->g[l - 1], m->g[l]);
       m->launches++;
     }
     CK(cudaGetLastError());
@@ -414,14 +416,14 @@ static int g_cycle_rb(msqg_group *G, int nrelax) {
       if (w < 2 * c) FAIL(MSQG_ERR_ARG, "tiles of level %d are too small for %d fused sweeps (raise agg_n)", l, c);
       std::vector<XItem> items(1);
       for (msqg_model *m : G->tiles) { items[0].arr.push_back(m->da.lev[l]); items[0].geo.push_back(m->g[l]); }
-      items[0].nf = nl; items[0].w = w; items[0].ring = 0;
+      items[0].nf = nf; items[0].w = w; items[0].ring = 0;
       if (l == La && left == nrelax) {
         /* the halo of res on ALL distributed levels (the sweeps recompute up to 2 nrelax border cells of the neighbours)
            rides in the same exchange: one neighbour synchronisation less per cycle */
         for (int l2 = La; l2 <= D; l2++) {
           XItem X;
           for (msqg_model *m : G->tiles) { X.arr.push_back(m->res.lev[l2]); X.geo.push_back(m->g[l2]); }
-          X.nf = nl; X.w = 2 * chunk0; X.ring = 0;
+          X.nf = nf; X.w = 2 * chunk0; X.ring = 0;
           if (X.w > m0->g[l2].nx) X.w = m0->g[l2].nx;
           if (X.w > m0->g[l2].ny) X.w = m0->g[l2].ny;
           items.push_back(X);
@@ -430,27 +432,32 @@ static int g_cycle_rb(msqg_group *G, int nrelax) {
       if ((rc = exchange_multi(G, items))) return rc;
       for (msqg_model *m : G->tiles) {
         ProfScope ps(m, l == D ? PROF_RELAX_FINE : PROF_RELAX_COARSE, c);
-        NL_SWITCH(m->nl, { auto C = relax_coef_layers<NL>(m, l); rc = relax_rb_tile<NL>(m, l, c, w, C); });
+        if (mode < 0) {
+          NL_SWITCH(m->nl, { auto C = relax_coef_layers<NL>(m, l); rc = relax_rb_tile<NL>(m, l, c, w, C); });
+        } else
+          rc = relax_rb_tile<1>(m, l, c, w, relax_coef_scalar(m, l, m->lam_lev[(size_t)l * m->nl + mode]));
         if (rc) return rc;
       }
       left -= c;
     }
   }
   /* a += da ; boundary(a) */
-  for (msqg_model *m : G->tiles) {
+  for (int t = 0; t < nt; t++) {
+    msqg_model *m = G->tiles[t];
     const Geom &g = m->g[D];
     ProfScope ps(m, PROF_CORRECT, 0);
-    k_correct<<<grid2(g.nx, g.ny, b, nl), b, 0, G->stream>>>(m->psi.lev[D], m->da.lev[D], g, 1);
+    k_correct<<<grid2(g.nx, g.ny, b, nf), b, 0, G->stream>>>(P[t].a, m->da.lev[D], g, 1);
     m->launches++;
   }
   CK(cudaGetLastError());
   /* one halo cell of da survived the sweeps: the neighbours' correction of those cells is applied here with the same
      operands (a_halo + da_halo, the bits the owner computes), then the ghosts of the physical sides next to a halo
      column / row are rebuilt from it -- no exchange of psi */
-  for (msqg_model *m : G->tiles) {
+  for (int t = 0; t < nt; t++) {
+    msqg_model *m = G->tiles[t];
     const Geom &g = m->g[D];
-    k_correct_ring<<<dim3((2 * (g.nx + g.ny + 2) + 255) / 256, nl), 256, 0, G->stream>>>(m->psi.lev[D], m->da.lev[D], g);
-    k_ghosts<<<grid2(g.nx + 2, g.ny + 2, b, nl), b, 0, G->stream>>>(m->psi.lev[D], nl, g, -1.);
+    k_correct_ring<<<dim3((2 * (g.nx + g.ny + 2) + 255) / 256, nf), 256, 0, G->stream>>>(P[t].a, m->da.lev[D], g);
+    k_ghosts<<<grid2(g.nx + 2, g.ny + 2, b, nf), b, 0, G->stream>>>(P[t].a, nf, g, -1.);
     m->launches += 2;
   }
   CK(cudaGetLastError());

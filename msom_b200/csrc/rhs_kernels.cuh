@@ -616,13 +616,23 @@ struct ModeMat {
   double a[NL * NL];
 };
 
-template <int NL>
+/* RING (tiles): the threads cover the interior plus the one-cell ring, and project the ring cells of the INTERNAL sides
+ * too (cells of a neighbouring tile whose input holds the owner's bits, so the output does as well); the ghosts of the
+ * physical sides are left to k_ghosts, and `ghosts` is ignored */
+template <int NL, bool RING = false>
 __global__ void __launch_bounds__(256)
 k_project(const double *__restrict__ in, double *__restrict__ out, Geom g, ModeMat<NL> M,
           const double *__restrict__ matf /* optional per-cell matrix planes */, int ghosts) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x;
-  const int y = blockIdx.y * blockDim.y + threadIdx.y;
-  if (x >= g.nx || y >= g.ny) return;
+  const int x = blockIdx.x * blockDim.x + threadIdx.x - (RING ? 1 : 0);
+  const int y = blockIdx.y * blockDim.y + threadIdx.y - (RING ? 1 : 0);
+  if (RING) {
+    if (x > g.nx || y > g.ny) return;
+    const bool okx = x < 0 ? (g.bc & 1) : (x >= g.nx ? (g.bc & 2) : true);
+    const bool oky = y < 0 ? (g.bc & 4) : (y >= g.ny ? (g.bc & 8) : true);
+    if (!okx || !oky) return;
+    ghosts = 0;
+  } else if (x >= g.nx || y >= g.ny)
+    return;
   const size_t c = GIDX(g.pitch, y, x);
   const size_t pl = g.plane;
   double v[NL];

@@ -48,6 +48,7 @@ def _bind():
     L.msqg_group_invertq.argtypes = [vp, C.c_int]
     L.msqg_group_step.argtypes = [vp, C.c_double, C.c_double, pd, pd]
     L.msqg_group_last_mgstats.argtypes = [vp, C.POINTER(G.MgStats)]
+    L.msqg_group_last_mode_mgstats.argtypes = [vp, C.c_int, C.POINTER(G.MgStats)]
     for f in ("msqg_group_total_cycles", "msqg_group_exchanges", "msqg_group_launches"):
         getattr(L, f).argtypes = [vp]
         getattr(L, f).restype = C.c_long
@@ -134,9 +135,10 @@ class Group:
     def invertq(self, q_id=G.Q):
         G.check(self.L.msqg_group_invertq(self.h, q_id))
 
-    def mgstats(self):
+    def mgstats(self, mode=-1):
+        """statistics of the last solve (mode < 0), or of vertical mode `mode` of the last modal inversion"""
         s = G.MgStats()
-        G.check(self.L.msqg_group_last_mgstats(self.h, C.byref(s)))
+        G.check(self.L.msqg_group_last_mode_mgstats(self.h, mode, C.byref(s)))
         return s
 
     def step(self, tnext_event=-1.0):

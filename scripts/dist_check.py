@@ -1,5 +1,6 @@
-"""torchrun --nproc-per-node N scripts/dist_check.py : the NCCL back-end of the domain decomposition
-against the CPU oracle's emulation of the same decomposition, bit for bit, on every rank."""
+"""torchrun --nproc-per-node N scripts/dist_check.py [lex|rb|rbper|rbmodal] : the NCCL back-end of the domain
+decomposition against the CPU oracle's emulation of the same decomposition, bit for bit, on every rank.
+rbmodal: the vertical-mode inversion (mode_pv_invert = 1) on red-black tiles, every mode's statistics compared too."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -15,9 +16,12 @@ torch.cuda.set_device(local)
 dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 N, nl, agg_n = 256, 3, 64
 sm = sys.argv[1] if len(sys.argv) > 1 else "lex"
+modal = sm == "rbmodal"   # one scalar Helmholtz solve per vertical mode on the tiles
+if modal:
+    sm = "rb"
 if sm == "rb":
     agg_n = 128 if world > 2 else 64
-kw = base_kw(N, nl)
+kw = base_kw(N, nl, mode_pv_invert=1) if modal else base_kw(N, nl)
 periodic = sm == "rbper"   # doubly periodic domain (sbc = -1) on the process grid: neighbours wrap around
 if periodic:
     sm = "rb"
@@ -34,6 +38,10 @@ mo.set(O.PSI, psi); mo.set_const()
 ok = True
 for s in range(3):
     ok &= (g.step() == mo.step())
+if modal:
+    for k in range(nl):
+        sg, so = g.mgstats(k), mo.mgstats(k)
+        ok &= (sg.i, sg.nrelax, sg.resb, sg.resa) == (so.i, so.nrelax, so.resb, so.resa)
 _, _, x0, y0, nx, ny = g.boxes[0]
 for fg, fo in ((G.PSI, O.PSI), (G.Q, O.Q)):
     ok &= bool(np.array_equal(g.get_tile(0, fg), mo.get(fo)[:, y0:y0 + ny, x0:x0 + nx]))
@@ -41,7 +49,7 @@ ok &= (g.total_cycles == mo.L.orc_total_cycles(mo.h))
 t = torch.tensor([1 if ok else 0], device="cuda")
 dist.all_reduce(t, op=dist.ReduceOp.MIN)
 if rank == 0:
-    print("DIST_CHECK", "PASS" if int(t.item()) == 1 else "FAIL", sm + ("-periodic" if periodic else ""), g.transport, "world", world, "grid %dx%d" % (px, py), "exchanges", g.exchanges)
+    print("DIST_CHECK", "PASS" if int(t.item()) == 1 else "FAIL", sm + ("-periodic" if periodic else "") + ("-modal" if modal else ""), g.transport, "world", world, "grid %dx%d" % (px, py), "exchanges", g.exchanges)
 g.close()
 dist.destroy_process_group()
 sys.exit(0 if int(t.item()) == 1 else 1)
