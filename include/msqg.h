@@ -230,6 +230,11 @@ void msqg_derive_params(msqg_params *p);
 int msqg_test_relax(msqg_model *m, int level, double *a, const double *b, int nsweeps);
 int msqg_test_relax_scalar(msqg_model *m, int level, double lambda, double *a, const double *b, int nsweeps);
 int msqg_test_residual(msqg_model *m, const double *a, const double *b, double *res, double *maxres);
+/* the residual pass of the multigrid solve with the restriction pyramid it leaves: mode < 0 the layer-coupled problem
+ * (a, b [nl][n][n]), mode >= 0 the scalar Helmholtz problem of that vertical mode (mode_pv_invert, a, b [1][n][n]).
+ * out receives res on levels D, D-1, .., *bottom one after another, each [nf][2^l][2^l] (at most 4/3 of level D) */
+int msqg_test_residual_levels(msqg_model *m, int mode, const double *a, const double *b, double *out, double *maxres,
+                              int *bottom);
 int msqg_test_restrict(msqg_model *m, int level, const double *fine, double *coarse);
 int msqg_test_prolong(msqg_model *m, int level, const double *coarse, double *fine);
 /* div_by() (exact division by a pivot with known reciprocal) next to IEEE x/d */

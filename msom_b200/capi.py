@@ -132,6 +132,7 @@ def lib():
     L.msqg_test_relax.argtypes = [vp, C.c_int, dp, dp, C.c_int]
     L.msqg_test_relax_scalar.argtypes = [vp, C.c_int, C.c_double, dp, dp, C.c_int]
     L.msqg_test_residual.argtypes = [vp, dp, dp, dp, pd]
+    L.msqg_test_residual_levels.argtypes = [vp, C.c_int, dp, dp, dp, pd, C.POINTER(C.c_int)]
     L.msqg_test_restrict.argtypes = [vp, C.c_int, dp, dp]
     L.msqg_test_prolong.argtypes = [vp, C.c_int, dp, dp]
     L.msqg_test_div.argtypes = [C.c_int, dp, dp, dp, dp, C.c_int]

@@ -132,6 +132,26 @@ struct LayerMetrics {
   double idh0[MSQG_NLMAX], idh1[MSQG_NLMAX];
 };
 
+/* The per-cell expressions of the residual, shared by every residual kernel so that the association order is written
+ * once.  res_vertical: b and the stretching term of layer l out of NL (NL == 1: b alone); sm / sp = stretching of the
+ * interfaces above / below the layer (l - 1, l), am / ap = a of the layers l - 1, l + 1 (ignored where absent). */
+template <int NL>
+__device__ __forceinline__ double res_vertical(int l, double b, double sm, double sp, double am, double ac, double ap,
+                                               const LayerMetrics &M) {
+  if (NL == 1) return b;
+  if (l == 0) return b + sp * (ac - ap) * M.idh1[0];
+  if (l < NL - 1) return b + sm * (ac - am) * M.idh0[l] - sp * (ap - ac) * M.idh1[l];
+  return b + sm * (ac - am) * M.idh0[l];
+}
+/* r + the face-gradient Laplacian of a (x then y); x/Delta via div_by: same bits as the IEEE division, 6x fewer
+ * instructions */
+__device__ __forceinline__ double res_laplacian(double r, double ac, double aw, double ae, double as, double an, double D,
+                                                double rD) {
+  r += div_by(div_by(ac - aw, D, rD) - div_by(ae - ac, D, rD), D, rD);
+  r += div_by(div_by(ac - as, D, rD) - div_by(an - ac, D, rD), D, rD);
+  return r;
+}
+
 template <int NL>
 __global__ void __launch_bounds__(256)
 k_residual(const double *__restrict__ a, const double *__restrict__ b, double *__restrict__ res,
@@ -141,28 +161,182 @@ k_residual(const double *__restrict__ a, const double *__restrict__ b, double *_
   double m = 0.;
   if (x < g.nx && y < g.ny) {
     const size_t c = GIDX(g.pitch, y, x);
-    const double D = g.Delta, rD = g.rD; /* x/Delta via div_by: same bits as the IEEE division, 6x fewer instructions */
+    const double D = g.Delta, rD = g.rD;
     double ac[NL];
 #pragma unroll
     for (int l = 0; l < NL; l++) ac[l] = a[l * g.plane + c];
 #pragma unroll
     for (int l = 0; l < NL; l++) {
       const double *al = a + l * g.plane;
-      double r;
-      if (NL == 1)
-        r = b[c];
-      else if (l == 0)
-        r = b[c] + s[c] * (ac[0] - ac[1]) * M.idh1[0];
-      else if (l < NL - 1)
-        r = b[l * g.plane + c] + s[(l - 1) * g.plane + c] * (ac[l] - ac[l - 1]) * M.idh0[l] -
-            s[l * g.plane + c] * (ac[l + 1] - ac[l]) * M.idh1[l];
-      else
-        r = b[l * g.plane + c] + s[(l - 1) * g.plane + c] * (ac[l] - ac[l - 1]) * M.idh0[l];
-      r += div_by(div_by(ac[l] - al[c - 1], D, rD) - div_by(al[c + 1] - ac[l], D, rD), D, rD);
-      r += div_by(div_by(ac[l] - al[c - g.pitch], D, rD) - div_by(al[c + g.pitch] - ac[l], D, rD), D, rD);
+      const double sm = l > 0 ? s[(l - 1) * g.plane + c] : 0., sp = l < NL - 1 ? s[l * g.plane + c] : 0.;
+      double r = res_vertical<NL>(l, b[l * g.plane + c], sm, sp, l > 0 ? ac[l > 0 ? l - 1 : 0] : 0., ac[l],
+                                  l < NL - 1 ? ac[l < NL - 1 ? l + 1 : l] : 0., M);
+      r = res_laplacian(r, ac[l], al[c - 1], al[c + 1], al[c - g.pitch], al[c + g.pitch], D, rD);
       res[l * g.plane + c] = r;
       const double f = fabs(r);
       if (f > m) m = f;
+    }
+  }
+  block_max_to(maxres, m);
+}
+
+/* ------------------------------------------------------------------ residual + restriction pyramid
+ * The residual of k_residual (NL >= 2, SFIELD: stretching read from its field, else the per-layer constants S.s of a
+ * horizontally uniform field) or of k_residual_scalar (NL == 1: b - lambda a, lambda read from its plane), and from the
+ * same tile the restriction of res down the hierarchy (k_restrict's expression, each level from the one above it):
+ * levels D-1 .. D-5 of a 32x32 fine tile, as far as P.nlev says.  Undecomposed levels only (g.bc == 0, nx = ny = 2^D).
+ *   one thread = one 2x2 quad of fine cells = one cell of level D-1: the first restriction is in registers;
+ *   one warp = 16x2 quads: level D-2 by three shuffles, its 8 cells go to shared memory;
+ *   one CTA = 8 warps = 32x32 fine cells: levels D-3 (4x4), D-4 (2x2), D-5 (1x1) from shared memory at the end.
+ * Rows are read and written as 16-byte pairs (the interior of a row starts 128-byte aligned, a quad at an even x).  The
+ * layers are walked in order; a layer needs the centre values of its two neighbours only. */
+#define PYR_MAXLEV 5
+#define PYR_TILE 32
+struct PyrLevels {
+  double *p[PYR_MAXLEV]; /* res on levels D-1, D-2, ... */
+  int pitch[PYR_MAXLEV];
+  size_t plane[PYR_MAXLEV];
+  int n[PYR_MAXLEV];     /* cells per side */
+  int nlev;              /* levels written below D (0 .. PYR_MAXLEV) */
+};
+struct StretchConsts {
+  double s[MSQG_NLMAX];
+};
+
+__device__ __forceinline__ double restrict4(double c00, double c01, double c10, double c11) {
+  /* restriction_average, k_restrict's order: (0,0), (0,1) [y+1], (1,0) [x+1], (1,1); the leading 0. maps -0 to +0 */
+  double sum = 0.;
+  sum += c00;
+  sum += c01;
+  sum += c10;
+  sum += c11;
+  return sum / 4;
+}
+
+/* one shared-memory stage of the pyramid: W x W cells per layer of the CTA from the (2W) x (2W) of the stage above,
+ * kept in dst (unless null) for the next stage and stored on pyramid level k */
+template <int NL, int W>
+__device__ __forceinline__ void pyr_stage(const double *src, double *dst, const PyrLevels &P, int k, int tid) {
+  if (tid < NL * W * W) {
+    const int l = tid / (W * W), y = (tid / W) % W, x = tid % W;
+    const double *s = src + (l * 2 * W + 2 * y) * 2 * W + 2 * x;
+    const double v = restrict4(s[0], s[2 * W], s[1], s[2 * W + 1]);
+    if (dst) dst[(l * W + y) * W + x] = v;
+    const int gx = blockIdx.x * W + x, gy = blockIdx.y * W + y;
+    if (gx < P.n[k] && gy < P.n[k]) P.p[k][l * P.plane[k] + GIDX(P.pitch[k], gy, gx)] = v;
+  }
+}
+
+/* what a quad reads of one layer besides its centre: the rows below (up: y-1) and above (dn: y+2), the columns
+ * x-1 (w) and x+2 (e), b, and the stretching of the interface below the layer or lambda (s, when s != null) */
+struct PyrIn {
+  double2 up, dn, b0, b1, s0, s1;
+  double w0, w1, e0, e1;
+};
+__device__ __forceinline__ void pyr_load(PyrIn &L, const double *__restrict__ al, const double *__restrict__ bl,
+                                         const double *__restrict__ sl, size_t c0, size_t c1, int W) {
+  L.up = *(const double2 *)(al + c0 - W); L.dn = *(const double2 *)(al + c1 + W);
+  L.w0 = al[c0 - 1]; L.w1 = al[c1 - 1]; L.e0 = al[c0 + 2]; L.e1 = al[c1 + 2];
+  L.b0 = *(const double2 *)(bl + c0); L.b1 = *(const double2 *)(bl + c1);
+  if (sl) { L.s0 = *(const double2 *)(sl + c0); L.s1 = *(const double2 *)(sl + c1); }
+  else L.s0 = L.s1 = make_double2(0., 0.);
+}
+
+template <int NL, bool SFIELD>
+__global__ void __launch_bounds__(256, NL <= 8 ? 2 : 1)
+k_residual_pyr(const double *__restrict__ a, const double *__restrict__ b, double *__restrict__ res,
+               const double *__restrict__ s, StretchConsts S, Geom g, LayerMetrics M, PyrLevels P,
+               double *__restrict__ maxres) {
+  __shared__ double s2[NL * 64], s3[NL * 16], s4[NL * 4];
+  const int lane = threadIdx.x, tid = threadIdx.y * 32 + lane;
+  const int qx = blockIdx.x * (PYR_TILE / 2) + (lane & 15);
+  const int qy = blockIdx.y * (PYR_TILE / 2) + threadIdx.y * 2 + (lane >> 4);
+  const bool in = 2 * qx < g.nx && 2 * qy < g.ny;
+  const int W = g.pitch;
+  const size_t c0 = GIDX(W, 2 * qy, 2 * qx), c1 = c0 + W;
+  const double D = g.Delta, rD = g.rD;
+  /* centre rows of the quad, two layers ahead; the rest of a layer's inputs (neighbours, b, stretching or lambda) one
+     layer ahead, so that the loads of the next layer are in flight while this one is computed */
+  double2 ctr0[NL], ctr1[NL];
+  PyrIn ld[NL];
+  const bool sfield = NL == 1 || SFIELD;
+  if (in) {
+    ctr0[0] = *(const double2 *)(a + c0);
+    ctr1[0] = *(const double2 *)(a + c1);
+    if (NL > 1) {
+      ctr0[NL > 1 ? 1 : 0] = *(const double2 *)(a + g.plane + c0);
+      ctr1[NL > 1 ? 1 : 0] = *(const double2 *)(a + g.plane + c1);
+    }
+    pyr_load(ld[0], a, b, sfield ? s : nullptr, c0, c1, W);
+  }
+  double m = 0.;
+#pragma unroll
+  for (int l = 0; l < NL; l++) {
+    double r00 = 0., r10 = 0., r01 = 0., r11 = 0.; /* r<dx><dy> */
+    if (in) {
+      const int ln = l + 1 < NL ? l + 1 : l, ln2 = l + 2 < NL ? l + 2 : l;
+      if (l + 1 < NL)
+        pyr_load(ld[ln], a + ln * g.plane, b + ln * g.plane, sfield && ln < NL - 1 ? s + ln * g.plane : nullptr, c0, c1, W);
+      if (l + 2 < NL) {
+        ctr0[ln2] = *(const double2 *)(a + ln2 * g.plane + c0);
+        ctr1[ln2] = *(const double2 *)(a + ln2 * g.plane + c1);
+      }
+      const PyrIn &L = ld[l];
+      const double2 C0 = ctr0[l], C1 = ctr1[l];
+      const int lm = l > 0 ? l - 1 : 0;
+      const double2 M0 = ctr0[lm], M1 = ctr1[lm], P0 = ctr0[ln], P1 = ctr1[ln];
+      if (NL == 1) {
+        r00 = L.b0.x - L.s0.x * C0.x; r10 = L.b0.y - L.s0.y * C0.y; r01 = L.b1.x - L.s1.x * C1.x; r11 = L.b1.y - L.s1.y * C1.y;
+      } else {
+        double2 sm0, sm1, sp0, sp1;
+        if (SFIELD) { /* interface l-1 was loaded with the layer above */
+          sm0 = ld[lm].s0; sm1 = ld[lm].s1; sp0 = L.s0; sp1 = L.s1;
+        } else {
+          sm0 = sm1 = make_double2(S.s[lm], S.s[lm]);
+          sp0 = sp1 = make_double2(S.s[l], S.s[l]);
+        }
+        r00 = res_vertical<NL>(l, L.b0.x, sm0.x, sp0.x, M0.x, C0.x, P0.x, M);
+        r10 = res_vertical<NL>(l, L.b0.y, sm0.y, sp0.y, M0.y, C0.y, P0.y, M);
+        r01 = res_vertical<NL>(l, L.b1.x, sm1.x, sp1.x, M1.x, C1.x, P1.x, M);
+        r11 = res_vertical<NL>(l, L.b1.y, sm1.y, sp1.y, M1.y, C1.y, P1.y, M);
+      }
+      r00 = res_laplacian(r00, C0.x, L.w0, C0.y, L.up.x, C1.x, D, rD);
+      r10 = res_laplacian(r10, C0.y, C0.x, L.e0, L.up.y, C1.y, D, rD);
+      r01 = res_laplacian(r01, C1.x, L.w1, C1.y, C0.x, L.dn.x, D, rD);
+      r11 = res_laplacian(r11, C1.y, C1.x, L.e1, C0.y, L.dn.y, D, rD);
+      *(double2 *)(res + l * g.plane + c0) = make_double2(r00, r10);
+      *(double2 *)(res + l * g.plane + c1) = make_double2(r01, r11);
+      double f[4] = {fabs(r00), fabs(r10), fabs(r01), fabs(r11)};
+#pragma unroll
+      for (int i = 0; i < 4; i++) {
+        if (NL == 1 && !(f[i] > 0.)) f[i] = 0.; /* k_residual_scalar maps NaN to 0, k_residual skips it */
+        if (f[i] > m) m = f[i];
+      }
+    }
+    if (P.nlev >= 1) {
+      const double v1 = restrict4(r00, r01, r10, r11);
+      if (in) P.p[0][l * P.plane[0] + GIDX(P.pitch[0], qy, qx)] = v1;
+      if (P.nlev >= 2) {
+        const double u01 = __shfl_down_sync(FULLMASK, v1, 16), u10 = __shfl_down_sync(FULLMASK, v1, 1),
+                     u11 = __shfl_down_sync(FULLMASK, v1, 17);
+        if (lane < 16 && !(lane & 1)) {
+          const double v2 = restrict4(v1, u01, u10, u11);
+          if (in) P.p[1][l * P.plane[1] + GIDX(P.pitch[1], qy >> 1, qx >> 1)] = v2;
+          s2[(l * 8 + threadIdx.y) * 8 + (lane >> 1)] = v2;
+        }
+      }
+    }
+  }
+  if (P.nlev >= 3) {
+    __syncthreads();
+    pyr_stage<NL, 4>(s2, s3, P, 2, tid);
+    if (P.nlev >= 4) {
+      __syncthreads();
+      pyr_stage<NL, 2>(s3, s4, P, 3, tid);
+      if (P.nlev >= 5) {
+        __syncthreads();
+        pyr_stage<NL, 1>(s4, nullptr, P, 4, tid);
+      }
     }
   }
   block_max_to(maxres, m);
@@ -268,9 +442,7 @@ k_residual_scalar(const double *__restrict__ a, const double *__restrict__ b, do
     const size_t c = GIDX(g.pitch, y, x);
     const double D = g.Delta, rD = g.rD;
     const double ac = a[c];
-    double r = b[c] - lam[c] * ac;
-    r += div_by(div_by(ac - a[c - 1], D, rD) - div_by(a[c + 1] - ac, D, rD), D, rD);
-    r += div_by(div_by(ac - a[c - g.pitch], D, rD) - div_by(a[c + g.pitch] - ac, D, rD), D, rD);
+    const double r = res_laplacian(b[c] - lam[c] * ac, ac, a[c - 1], a[c + 1], a[c - g.pitch], a[c + g.pitch], D, rD);
     res[c] = r;
     m = fabs(r);
     if (!(m > 0.)) m = 0.;

@@ -1460,10 +1460,45 @@ struct MgProblem {
                                buffer of its out-of-place correction instead of copying it back */
 };
 
+/* Lowest level of res that mg_residual_enqueue leaves restricted: on one undecomposed, non-periodic grid the residual
+ * kernel also writes the restriction pyramid of its 32x32 tiles, levels D-1 .. D-5, never below level 1 (minlevel = 1:
+ * level 0 is not read).  Elsewhere it writes level D only. */
+static int residual_pyr_bottom(const msqg_model *m) {
+  const int D = m->depth;
+  if (m->g[D].bc != 0 || m->periodic || D < 2) return D;
+  return D - PYR_MAXLEV > 1 ? D - PYR_MAXLEV : 1;
+}
+
 static int mg_residual_enqueue(msqg_model *m, const MgProblem &P) {
   const int D = m->depth;
   const Geom &g = m->g[D];
   CK(zero_words(m->stream, m->d_scal, 1));
+  const int bottom = residual_pyr_bottom(m);
+  if (bottom < D) {
+    PyrLevels L;
+    L.nlev = D - bottom;
+    for (int k = 0; k < PYR_MAXLEV; k++) {
+      const int l = k < L.nlev ? D - 1 - k : D;
+      L.p[k] = m->res.lev[l]; L.pitch[k] = m->g[l].pitch; L.plane[k] = m->g[l].plane; L.n[k] = m->g[l].nx;
+    }
+    const dim3 b(32, 8), grid((g.nx + PYR_TILE - 1) / PYR_TILE, (g.ny + PYR_TILE - 1) / PYR_TILE);
+    const LayerMetrics M = metrics_of(m);
+    StretchConsts S;
+    for (int l = 0; l < MSQG_NLMAX; l++) S.s[l] = l < m->nl ? m->s_lev[(size_t)D * m->nl + l] : 0.;
+    { ProfScope ps(m, PROF_RESIDUAL, 0);
+    if (P.mode >= 0) {
+      k_residual_pyr<1, true><<<grid, b, 0, m->stream>>>(P.a, P.b, m->res.lev[D], m->ibu.lev[D] + (size_t)P.mode * g.plane, S, g, M, L, m->d_scal);
+    } else if (m->s_uniform) { /* s_lev holds the field's one value per layer, bit for bit */
+      NL_SWITCH(m->nl, k_residual_pyr<NL, false><<<grid, b, 0, m->stream>>>(P.a, P.b, m->res.lev[D], nullptr, S, g, M, L, m->d_scal));
+    } else {
+      NL_SWITCH(m->nl, k_residual_pyr<NL, true><<<grid, b, 0, m->stream>>>(P.a, P.b, m->res.lev[D], m->str.lev[D], S, g, M, L, m->d_scal));
+    }
+    }
+    m->launches++;
+    CK(cudaGetLastError());
+    CK(to_host(m->stream, m->h_scal, m->d_scal, 1));
+    return MSQG_OK;
+  }
   dim3 b(64, 4);
   { ProfScope ps(m, PROF_RESIDUAL, 0);
   if (P.mode < 0) {
@@ -1536,11 +1571,11 @@ static unsigned long long da_parity_mask(msqg_model *m) {
 /* experimental fusions of correction + residual + first restriction (k_corr_res), layer-coupled solves on an
  * undecomposed grid only */
 static int mg_fused(msqg_model *m, const MgProblem &P) {
-  /* 0: k_residual, k_restrict, k_correct (default).  Two fusions of the cycle's tail are kept behind MSQG_MG for A/B
-     measurements; both are bit-identical and both measured SLOWER on B200 at 4096^2 x 4 (ms per step, residual +
-     restrict + correct): split 6.27; MSQG_MG=rr (residual + first restriction in one kernel) 6.47; MSQG_MG=fused
-     (correction too, out of place) 8.03 -- the shared-memory hand-off and the neighbour gathers of a and da cost more
-     than the one or two plane reads they save, the split kernels already stream at 75-100 % of the HBM peak. */
+  /* 0: the default path (k_residual_pyr; correction folded into the relax pass).  Two fusions of the cycle's tail are
+     kept behind MSQG_MG for A/B measurements against the split kernels of an older default; both are bit-identical and
+     both measured SLOWER on B200 at 4096^2 x 4 (ms per step, residual + restrict + correct): split 6.27; MSQG_MG=rr
+     (residual + first restriction in one kernel) 6.47; MSQG_MG=fused (correction too, out of place) 8.03 -- the
+     shared-memory hand-off and the neighbour gathers of a and da cost more than the one or two plane reads they save. */
 #ifdef MSQG_EXPERIMENTS
   static int v = -1;
   if (v < 0) { const char *e = getenv("MSQG_MG"); v = (e && !strcmp(e, "rr")) ? 1 : (e && !strcmp(e, "fused")) ? 2 : 0; }
@@ -1654,9 +1689,11 @@ static int mg_levels(msqg_model *m, int nf, int mode, int nrelax, int from, int 
 static int mg_cycle(msqg_model *m, const MgProblem &P, int nrelax, int fused = 0) {
   const int D = m->depth;
   dim3 b(32, 8);
-  /* restriction(res): levels D-1..1 (level 0 is never read with minlevel = 1), then levels 1 .. D */
+  /* restriction(res): levels D-1..1 (level 0 is never read with minlevel = 1), then levels 1 .. D.  The residual
+     before the cycle has already restricted res down to residual_pyr_bottom (k_corr_res: to D-1) */
   bool corrected = false;
-  int rc = mg_levels(m, P.nf, P.mode, nrelax, fused ? D - 1 : D, D, fused ? nullptr : P.a, fused ? nullptr : &corrected);
+  const int from = fused ? D - 1 : residual_pyr_bottom(m);
+  int rc = mg_levels(m, P.nf, P.mode, nrelax, from, D, fused ? nullptr : P.a, fused ? nullptr : &corrected);
   if (rc) return rc;
   if (fused == 2 || corrected) return MSQG_OK; /* corrected: the last relax pass on level D did a += da */
   const Geom &g = m->g[D];
@@ -2684,6 +2721,24 @@ extern "C" int msqg_test_residual(msqg_model *m, const double *a, const double *
   MgProblem P{m->nl, -1, m->psi.lev[D], m->q.lev[D]};
   if ((rc = mg_residual(m, P, maxres))) return rc;
   return download_level(m, res, m->res.lev[D], m->nl, D);
+}
+extern "C" int msqg_test_residual_levels(msqg_model *m, int mode, const double *a, const double *b, double *out,
+                                         double *maxres, int *bottom) {
+  CK(cudaSetDevice(m->device));
+  if (!m->const_set) FAIL(MSQG_ERR_ARG, "needs set_const");
+  if (mode >= 0 && (!m->p.mode_pv_invert || mode >= m->nl)) FAIL(MSQG_ERR_ARG, "mode %d needs mode_pv_invert and mode < nl", mode);
+  const int D = m->depth, nf = mode < 0 ? m->nl : 1;
+  int rc;
+  if ((rc = upload_level(m, m->psi.lev[D], a, nf, D, -1.))) return rc;
+  if ((rc = upload_level(m, m->q.lev[D], b, nf, D, -1.))) return rc;
+  MgProblem P{nf, mode, m->psi.lev[D], m->q.lev[D]};
+  if ((rc = mg_residual(m, P, maxres))) return rc;
+  *bottom = residual_pyr_bottom(m);
+  for (int l = D; l >= *bottom; l--) {
+    if ((rc = download_level(m, out, m->res.lev[l], nf, l))) return rc;
+    out += (size_t)nf * m->g[l].nx * m->g[l].ny;
+  }
+  return MSQG_OK;
 }
 extern "C" int msqg_test_restrict(msqg_model *m, int level, const double *fine, double *coarse) {
   CK(cudaSetDevice(m->device));
