@@ -330,7 +330,6 @@ static int group_create(const msqg_params *p, int device, int px, int py, int ag
   const int per = p->sbc == -1;
   if (px * py < 2 && !per) FAIL(MSQG_ERR_ARG, "a group needs px*py >= 2 tiles");
   if (per && smoother != 1) FAIL(MSQG_ERR_ARG, "periodic boundaries (sbc = -1) need the red-black smoother");
-  if (p->stochastic) FAIL(MSQG_ERR_ARG, "stochastic forcing is not built on decomposed grids");
   if (p->mode_pv_invert) {
     /* the vertical-mode inversion runs the red-black cycle once per mode; the lexicographic tile sweep has no modal solve */
     if (smoother != 1) FAIL(MSQG_ERR_ARG, "the vertical-mode inversion (mode_pv_invert) on tiles needs the red-black smoother");
@@ -778,9 +777,42 @@ static double g_dt_chain(msqg_group *G, const double *umax, double dtmax) {
   G->ts_previous = m->ts_previous;
   return dtmax;
 }
+/* Stochastic forcing: every tile keeps its own corrector flag, noise mode, seed and draw counter (msqg_seed_noise and
+ * msqg_set_noise_mode act on one tile) and all of them advance identically, so the tiles draw, each for its window,
+ * the field of the undecomposed model.  Tiles seeded differently would give wrong bits without any error, so at the
+ * first stochastic step after a tile's seed or mode changed the group compares mode, seed and draw count across all
+ * tiles and ranks, with the complement trick of g_check_modes_agree.  Under NCCL every rank seeds its tile with the
+ * same arguments, so every rank takes this check at the same step. */
+static int g_check_noise_agree(msqg_group *G) {
+  bool pending = false;
+  for (msqg_model *m : G->tiles) pending |= !m->noise_agreed;
+  if (!pending) return MSQG_OK;
+  const int n = 8, nt = (int)G->tiles.size();
+  const double ones = 4294967295.;
+  std::vector<double> w((size_t)nt * n), out(n);
+  for (int t = 0; t < nt; t++) {
+    msqg_model *m = G->tiles[t];
+    const double h[4] = {(double)m->noise_mode, (double)m->noise_seed, (double)(m->noise_draw >> 32),
+                         (double)(m->noise_draw & 0xffffffffull)};
+    double *wt = &w[(size_t)t * n];
+    for (int k = 0; k < 4; k++) { wt[2 * k] = h[k]; wt[2 * k + 1] = ones - h[k]; }
+    CK(cudaMemcpyAsync(m->d_scal + 1, wt, n * sizeof(double), cudaMemcpyHostToDevice, G->stream));
+  }
+  int rc = reduce_max(G, 1, n, out.data());
+  if (rc) return rc;
+  static const char *what[4] = {"noise mode", "noise seed", "noise draw count", "noise draw count"};
+  for (int k = 0; k < n; k += 2)
+    if (out[k] + out[k + 1] != ones)
+      FAIL(MSQG_ERR_ARG, "the %s differs between tiles: seed every tile of a stochastic group alike (msqg_seed_noise, "
+                         "msqg_set_noise_mode on every tile and rank, with the same arguments)", what[k / 2]);
+  for (msqg_model *m : G->tiles) m->noise_agreed = 1;
+  return MSQG_OK;
+}
+
 extern "C" int msqg_group_step(msqg_group *G, double t, double tnext_event, double *dt_out, double *tnext_out) {
   CK(cudaSetDevice(G->device));
   int rc;
+  if (G->p.stochastic && (rc = g_check_noise_agree(G))) return rc;
   double umax[MSQG_MAXL];
   if ((rc = g_invertq(G, MSQG_Q))) return rc;
   if ((rc = g_rhs_prepare(G, umax))) return rc;
@@ -798,15 +830,19 @@ extern "C" int msqg_group_step(msqg_group *G, double t, double tnext_event, doub
     }
   } else
     tnext = t + dt;
-  for (msqg_model *m : G->tiles) {
+  for (msqg_model *m : G->tiles) { /* msqg_step: the noise of each stage is drawn before its right-hand side */
     const int D = m->depth;
-    if ((rc = rhs_launch(m, m->q, m->q.lev[D], m->qpred.lev[D], nullptr, dt / 2., 0.f))) return rc;
+    float dts = 0.f;
+    if (G->p.stochastic && (rc = stochastic_stage(m, sqrt(dt / 2.), &dts))) return rc;
+    if ((rc = rhs_launch(m, m->q, m->q.lev[D], m->qpred.lev[D], nullptr, dt / 2., dts))) return rc;
   }
   if ((rc = g_invertq(G, MSQG_QPRED))) return rc;
   if ((rc = g_rhs_prepare(G, umax))) return rc;
   for (msqg_model *m : G->tiles) {
     const int D = m->depth;
-    if ((rc = rhs_launch(m, m->qpred, m->q.lev[D], m->q.lev[D], nullptr, dt, 0.f))) return rc;
+    float dts = 0.f;
+    if (G->p.stochastic && (rc = stochastic_stage(m, sqrt(dt), &dts))) return rc;
+    if ((rc = rhs_launch(m, m->qpred, m->q.lev[D], m->q.lev[D], nullptr, dt, dts))) return rc;
   }
   CK(cudaStreamSynchronize(G->stream));
   (void)g_dt_chain(G, umax, dt);

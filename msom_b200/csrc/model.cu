@@ -173,7 +173,8 @@ struct msqg_model {
   std::vector<double> h_noise, h_sstoch;
   int noise_mode;               /* 0: host replay of the reference's libc rand() stream; 1: Philox on the device */
   unsigned int noise_seed;
-  unsigned long long noise_draw;
+  unsigned long long noise_draw; /* fields drawn since the last seed / mode change */
+  int noise_agreed;             /* a group checked that its tiles agree on mode, seed and draw count (dist_impl.cuh) */
   double umax_pg[MSQG_MAXL];
   msqg_mgstats mgpsi, mgmode[MSQG_MAXL];
   long total_cycles, launches;
@@ -417,8 +418,8 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
   if (per && !rb_dist)
     FAIL(MSQG_ERR_ARG, "periodic boundaries (sbc = -1) run on the tile machinery with the red-black smoother: "
                        "msqg_create does that by itself (a 1 x 1 group); tiles: msqg_group_create_local_sm(p, device, px, py, 0, 1, &group)");
-  if (per && (p->mode_pv_invert || p->stochastic || p->nptr > 0))
-    FAIL(MSQG_ERR_ARG, "periodic boundaries are built for the layer-coupled, deterministic path without tracers");
+  if (per && (p->mode_pv_invert || p->nptr > 0))
+    FAIL(MSQG_ERR_ARG, "periodic boundaries are built for the layer-coupled path without tracers");
   for (int l = 0; per && l < p->nl; l++)
     if (p->upg[l] != 0 || p->vpg[l] != 0)
       FAIL(MSQG_ERR_ARG, "periodic boundaries with a large-scale flow (non-periodic psi_pg, qg.h:1105-1114) are not built");
@@ -558,7 +559,7 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
   { const char *e = getenv("MSQG_RB_REUSE"); m->rb_reuse = (e && atoi(e) == 0) ? 0 : 1; }
   { const char *e = getenv("MSQG_GRAPH"); m->use_graphs = (e && atoi(e) == 0) ? 0 : 1; }
   m->swap_log = nullptr; m->tile_index = 0;
-  m->noise_mode = 0; m->noise_seed = 1; m->noise_draw = 0;
+  m->noise_mode = 0; m->noise_seed = 1; m->noise_draw = 0; m->noise_agreed = 0;
   memset(&m->mgpsi, 0, sizeof(m->mgpsi));
   memset(m->mgmode, 0, sizeof(m->mgmode));
   memset(m->umax_pg, 0, sizeof(m->umax_pg));
@@ -700,11 +701,11 @@ extern "C" double msqg_get_ts_previous(msqg_model *m) { return m->ts_previous; }
 extern "C" void msqg_set_ts_previous(msqg_model *m, double v) { m->ts_previous = v; }
 extern "C" int msqg_set_noise_mode(msqg_model *m, int mode) {
   if (mode != 0 && mode != 1) FAIL(MSQG_ERR_ARG, "noise mode is 0 (libc rand() replay) or 1 (Philox on the device)");
-  m->noise_mode = mode; m->noise_draw = 0;
+  m->noise_mode = mode; m->noise_draw = 0; m->noise_agreed = 0;
   return MSQG_OK;
 }
 extern "C" void msqg_seed_noise(msqg_model *m, unsigned seed) {
-  m->noise_seed = seed; m->noise_draw = 0;
+  m->noise_seed = seed; m->noise_draw = 0; m->noise_agreed = 0;
   memset(&m->rng, 0, sizeof(m->rng));
   initstate_r(seed, m->rng_state, sizeof(m->rng_state), &m->rng);
 }
@@ -2288,36 +2289,56 @@ extern "C" int msqg_update(msqg_model *m, int q_id, double dtmax, double *dtmax_
 }
 
 /* normal_noise / generate_noise, qg_stochastic.h:9,117-126: libc rand() in the
- * reference traversal order (x outer, y inner, layer innermost) on the host. */
+ * reference traversal order (x outer, y inner, layer innermost) on the host.
+ * A tile (decomposed or periodic group) replays the WHOLE N x N x nl stream of the undecomposed grid from its own
+ * random_r state and keeps the cells of its window [x0, x0 + tnx) x [y0, y0 + tny): the same bits as the
+ * undecomposed draw, at O(N^2 nl) host time per draw on every tile (every rank under NCCL).  That is the parity
+ * mode; the Philox mode draws only the tile's cells on the device. */
 static int generate_noise(msqg_model *m) {
-  const int n = m->N, nl = m->nl;
+  const int n = m->N, nl = m->nl, tx = m->tnx, ty = m->tny, x0 = m->x0, y0 = m->y0;
   const double pi = 3.14159265358979323846;
-  if (m->px * m->py > 1) FAIL(MSQG_ERR_ARG, "stochastic forcing is not supported on decomposed grids");
+  m->noise_draw++;
   if (m->noise_mode == 1) { /* one kernel, no host work: the production mode (and the only one that keeps a GPU busy) */
     const Geom &g = m->g[m->depth];
     dim3 b(64, 4);
-    k_noise_philox<<<grid2(g.nx, g.ny, b, nl), b, 0, m->stream>>>(m->nstoch.lev[m->depth], m->sstoch.lev[m->depth], g, m->p.amp_stoch,
-                                                                   m->noise_seed, m->noise_draw);
+    k_noise_philox<<<grid2(g.nx, g.ny, b, nl), b, 0, m->stream>>>(m->nstoch.lev[m->depth], m->sstoch.lev[m->depth], g, n, x0, y0,
+                                                                   m->p.amp_stoch, m->noise_seed, m->noise_draw - 1);
     m->launches++;
-    m->noise_draw++;
     CK(cudaGetLastError());
     return MSQG_OK;
   }
-  if (m->h_sstoch.empty()) m->h_sstoch.assign((size_t)nl * n * n, 0.);
-  m->h_noise.resize((size_t)nl * n * n);
+  if (m->h_sstoch.empty()) m->h_sstoch.assign((size_t)nl * tx * ty, 0.);
+  m->h_noise.resize((size_t)nl * tx * ty);
   for (int i = 0; i < n; i++)
-    for (int j = 0; j < n; j++)
+    for (int j = 0; j < n; j++) {
+      const bool mine = i >= x0 && i < x0 + tx && j >= y0 && j < y0 + ty;
       for (int l = 0; l < nl; l++) {
         /* normal_noise(): the two rand() calls in the order gcc evaluates the reference macro's operands */
         int32_t r1, r2;
         random_r(&m->rng, &r1);
         random_r(&m->rng, &r2);
+        if (!mine) continue;
         const double gsn = sqrt(-2. * log(((double)(r1) + 1.) / ((double)(RAND_MAX) + 2.))) *
                            cos(2 * pi * r2 / (double)RAND_MAX);
-        const size_t c = ((size_t)l * n + j) * n + i;
+        const size_t c = ((size_t)l * ty + j - y0) * tx + i - x0;
         m->h_noise[c] = m->p.amp_stoch * m->h_sstoch[c] * gsn;
       }
+    }
   return pack_to(m, m->nstoch, m->h_noise.data());
+}
+
+/* the noise part of one stochastic stage, qg_stochastic.h:128-138: the corrector flag toggles, and every other stage
+ * draws a field and scales the noise by 1/sqrt(2); sqrt_dt is sqrt(dt / 2.) in the predictor and sqrt(dt) in the
+ * corrector of a step, sqrt(dt) in advance_qg.  *dts is a float like the reference's. */
+static int stochastic_stage(msqg_model *m, double sqrt_dt, float *dts) {
+  m->corrector_step = (m->corrector_step + 1) % 2;
+  *dts = sqrt_dt;
+  if (m->corrector_step) {
+    int rc = generate_noise(m);
+    if (rc) return rc;
+    *dts = *dts / sqrt(2);
+  }
+  return MSQG_OK;
 }
 
 /* advance_qg(output, input, updates = DQ, dt), qg.h:594-606 / qg_stochastic.h:128-149 */
@@ -2329,13 +2350,8 @@ extern "C" int msqg_advance(msqg_model *m, int out_id, int in_id, double dt) {
   float dts = 0.f;
   const double *noise = nullptr;
   if (m->p.stochastic) {
-    m->corrector_step = (m->corrector_step + 1) % 2;
-    dts = sqrt(dt);
-    if (m->corrector_step) {
-      int rc = generate_noise(m);
-      if (rc) return rc;
-      dts = dts / sqrt(2);
-    }
+    int rc = stochastic_stage(m, sqrt(dt), &dts);
+    if (rc) return rc;
     noise = m->nstoch.lev[m->depth];
   }
   dim3 b(64, 4);
@@ -2383,28 +2399,14 @@ extern "C" int msqg_step(msqg_model *m, double t, double tnext_event, double *dt
   } else
     tnext = t + dt;
   float dts = 0.f;
-  if (m->p.stochastic) {
-    m->corrector_step = (m->corrector_step + 1) % 2;
-    dts = sqrt(dt / 2.);
-    if (m->corrector_step) {
-      if ((rc = generate_noise(m))) return rc;
-      dts = dts / sqrt(2);
-    }
-  }
+  if (m->p.stochastic && (rc = stochastic_stage(m, sqrt(dt / 2.), &dts))) return rc;
   double *dqp = m->keep_dq ? m->dq.lev[D] : nullptr;
   if ((rc = rhs_launch(m, m->q, m->q.lev[D], m->qpred.lev[D], dqp, dt / 2., dts))) return rc;
   if (m->p.nptr > 0 && (rc = ptr_launch(m, m->ptr, m->ptr.lev[D], m->ptr_pred.lev[D], nullptr, dt / 2.))) return rc;
   /* stage 2 */
   if ((rc = invertq_list(m, m->qpred))) return rc;
   if ((rc = rhs_prepare(m))) return rc;
-  if (m->p.stochastic) {
-    m->corrector_step = (m->corrector_step + 1) % 2;
-    dts = sqrt(dt);
-    if (m->corrector_step) {
-      if ((rc = generate_noise(m))) return rc;
-      dts = dts / sqrt(2);
-    }
-  }
+  if (m->p.stochastic && (rc = stochastic_stage(m, sqrt(dt), &dts))) return rc;
   if ((rc = rhs_launch(m, m->qpred, m->q.lev[D], m->q.lev[D], dqp, dt, dts))) return rc;
   if (m->p.nptr > 0 && (rc = ptr_launch(m, m->ptr_pred, m->ptr.lev[D], m->ptr.lev[D], nullptr, dt))) return rc;
   CK(cudaStreamSynchronize(m->stream));

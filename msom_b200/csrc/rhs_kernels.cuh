@@ -677,7 +677,10 @@ k_ke_partial(const double *__restrict__ p, Geom g, double *__restrict__ part) {
  * The reference draws n = amp * sigma * N(0,1) with Box-Muller on sequential libc rand() (qg_stochastic.h:9,117-126);
  * that stream is replayed on the host in the parity mode.  Here the same transform runs on a counter-based generator
  * (Philox4x32-10, counter = (cell-layer index, draw number), key = (seed, tag)), so a field of noise is one kernel and
- * does not depend on traversal order or on how many members share a GPU.  oracle/msqg_oracle.c mirrors it. */
+ * does not depend on traversal order or on how many members share a GPU.  oracle/msqg_oracle.c mirrors it.
+ * The counter is the GLOBAL cell-layer index (l*N + y0 + y)*N + x0 + x, with (x0, y0) the origin of the tile in the
+ * n x n grid: a decomposed or periodic group draws, cell by cell, the bits of the undecomposed field (where x0 = y0 = 0
+ * and n = g.nx = g.ny, the index of the whole grid). */
 __device__ __forceinline__ void philox4x32_10(unsigned int (&c)[4], unsigned int k0, unsigned int k1) {
 #pragma unroll
   for (int r = 0; r < 10; r++) {
@@ -689,13 +692,13 @@ __device__ __forceinline__ void philox4x32_10(unsigned int (&c)[4], unsigned int
   }
 }
 __global__ void __launch_bounds__(256)
-k_noise_philox(double *__restrict__ noise, const double *__restrict__ sigma, Geom g, double amp, unsigned int seed,
-               unsigned long long draw) {
+k_noise_philox(double *__restrict__ noise, const double *__restrict__ sigma, Geom g, int n, int x0, int y0, double amp,
+               unsigned int seed, unsigned long long draw) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x;
   const int y = blockIdx.y * blockDim.y + threadIdx.y;
   const int l = blockIdx.z;
   if (x >= g.nx || y >= g.ny) return;
-  const unsigned long long idx = ((unsigned long long)l * g.ny + y) * g.nx + x;
+  const unsigned long long idx = ((unsigned long long)l * n + y0 + y) * n + x0 + x;
   unsigned int c[4] = {(unsigned int)idx, (unsigned int)(idx >> 32), (unsigned int)draw, (unsigned int)(draw >> 32)};
   philox4x32_10(c, seed, 0x6d737167u);
   const double u1 = (((double)c[0]) * 4294967296. + (double)c[1] + 0.5) * (1. / 18446744073709551616.);
@@ -705,5 +708,7 @@ k_noise_philox(double *__restrict__ noise, const double *__restrict__ sigma, Geo
   const double v = amp * sigma[cc] * gsn;
   double *p = noise + (size_t)l * g.plane;
   p[GIDX(g.pitch, y, x)] = v;
+  /* the ghosts of the reference's boundary(n_stochl); nothing reads them (the stochastic terms of k_rhs and k_advance
+     are pointwise), so on a tile the ring is left as written here and never exchanged with the neighbours */
   write_ghosts(p, g, x, y, v, -1.);
 }

@@ -73,8 +73,16 @@ def tile_box(N, px, py, rank):
 
 
 class Group:
-    def __init__(self, params, px, py, agg_n, device=0, backend="local", rank=0, nranks=1, uid=None, smoother="lex"):
+    def __init__(self, params, px, py, agg_n, device=0, backend="local", rank=0, nranks=1, uid=None, smoother="lex",
+                 noise=None, seed=1):
+        """noise, seed: the noise stream of a group with stochastic forcing (params.stochastic), required there:
+        'philox' draws each tile's cells on the device (production), 'libc' replays the reference's rand() stream after
+        srand(seed) on every tile (parity; each tile pays the host time of the whole N^2 nl stream per draw).  Every tile
+        is seeded alike here; under NCCL every rank passes the same values."""
         self.L = _bind()
+        if params.stochastic and noise not in ("libc", "philox"):
+            raise G.MsqgError(G.ERR_ARG, "stochastic forcing on a group needs its noise stream: noise='philox' (device) or "
+                                         "'libc' (host replay of the whole rand() stream on every tile), and the seed")
         self.p, self.px, self.py, self.agg_n = params, px, py, agg_n
         self.N, self.nl = params.N, params.nl
         h = C.c_void_p()
@@ -93,6 +101,9 @@ class Group:
             info = (C.c_int * 6)()
             self.L.msqg_group_tile_info(self.h, t, info)
             self.boxes.append(tuple(info))
+        if params.stochastic:
+            self.set_noise_mode(noise)
+            self.seed_noise(seed)
 
     def close(self):
         if getattr(self, "h", None):
@@ -131,6 +142,22 @@ class Group:
 
     def set_const(self):
         G.check(self.L.msqg_group_set_const(self.h))
+
+    def _tiles(self):
+        return [self.L.msqg_group_tile(self.h, t) for t in range(self.ntiles)]
+
+    def seed_noise(self, seed):
+        """stochastic forcing: seed the noise stream of every local tile like srand(seed) (libc mode) or as the Philox
+        key (philox mode); the tiles then draw, each for its window, the field of the undecomposed model.  Under
+        NCCL every rank calls this with the same seed (the group refuses to step otherwise)."""
+        for h in self._tiles():
+            self.L.msqg_seed_noise(h, seed)
+
+    def set_noise_mode(self, mode):
+        """'libc' replays the reference's rand() stream (every tile replays all N^2 nl draws, host time), 'philox'
+        draws the field on the device (production).  Under NCCL every rank calls this with the same mode."""
+        for h in self._tiles():
+            G.check(self.L.msqg_set_noise_mode(h, {"libc": 0, "philox": 1}[mode]))
 
     def invertq(self, q_id=G.Q):
         G.check(self.L.msqg_group_invertq(self.h, q_id))
@@ -188,8 +215,9 @@ def broadcast_bytes(payload, nbytes, device=None):
     return bytes(t.cpu().numpy().tobytes())
 
 
-def nccl_group(params, agg_n, device, smoother="lex"):
-    """One tile per rank of the default torch.distributed process group (torch only carries the NCCL id)."""
+def nccl_group(params, agg_n, device, smoother="lex", noise=None, seed=1):
+    """One tile per rank of the default torch.distributed process group (torch only carries the NCCL id).
+    noise, seed: as Group (stochastic forcing), the same on every rank."""
     import torch.distributed as dist
     L = _bind()
     rank, world = dist.get_rank(), dist.get_world_size()
@@ -198,4 +226,4 @@ def nccl_group(params, agg_n, device, smoother="lex"):
     if rank == 0:
         G.check(L.msqg_nccl_unique_id(buf))
     uid = broadcast_bytes(buf.raw, 128, device)
-    return Group(params, px, py, agg_n, device, "nccl", rank, world, uid, smoother=smoother)
+    return Group(params, px, py, agg_n, device, "nccl", rank, world, uid, smoother=smoother, noise=noise, seed=seed)
