@@ -155,8 +155,6 @@ int msqg_get_smoother(msqg_model *m);
  * other compile-time switch of qg.h, _LS_RV = 0, needs no entry point: it is the arithmetic of flsrv = 0. */
 int msqg_set_energy_conserv(msqg_model *m, int on);
 int msqg_get_energy_conserv(msqg_model *m);
-/* 1 if the library was built with -DMSQG_EXPERIMENTS (rejected kernel variants kept for A/B measurements) */
-int msqg_has_experiments(void);
 /* reset_layer_var (layer.h:37-41): zero the interior, ghost ring untouched */
 int msqg_reset_field(msqg_model *m, int id);
 /* layer thicknesses dhf (qg.h:895-896; overridden by dh_%dl.bin, qg.h:940-948) */

@@ -2,7 +2,7 @@
 // n x n x 4 level: builds in seconds (one instantiation), prints the per-step time of worker 0, the
 // lag between neighbouring workers and a checksum of the result (must not change between variants).
 //   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -fmad=false -o relax_bench relax_bench.cu
-//   ./relax_bench [n=4096] [nsweeps=4]
+//   ./relax_bench [n=4096] [nsweeps=4] [repetitions=0]
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -46,12 +46,9 @@ int main(int argc, char **argv) {
   CKC(cudaMemset(err, 0, 4));
   k_fill<<<592, 256>>>(mail, words, MAIL_EMPTY);
   RelaxArgs A;
-  A.da = da; A.res = res; A.g = g; A.nsweeps = nsw; A.mailbox = mail; A.err = err; A.dbg = dbg; A.flags = argc > 3 ? atoi(argv[3]) : 0; A.w_base = 0;
-#ifndef BMW
-#define BMW 0
-#endif
-  constexpr int NTHR = 64 * BWPC + (BMW ? 32 : 0);
-  auto kern = k_relax_ws<NL, K, BWPC, false, false, 1, BMW != 0>;
+  A.da = da; A.res = res; A.g = g; A.nsweeps = nsw; A.mailbox = mail; A.err = err; A.dbg = dbg; A.w_base = 0;
+  constexpr int NTHR = 64 * BWPC;
+  auto kern = k_relax_ws<NL, K, BWPC, false, false>;
   const size_t smem = Cfg::smem_per_worker * BWPC;
   CKC(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int mb = 0; CKC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&mb, kern, NTHR, smem));
@@ -88,8 +85,8 @@ int main(int argc, char **argv) {
          ms, herr, (d[1] - d[0]) / 1e3 / steps, (d[1] - d[0]) / 1e3 / steps * 1965, lag[lag.size() / 2],
          lag[lag.size() / 2] - Cfg::W * (d[1] - d[0]) / 1e3 / steps, cs);
   // determinism stress: the strips synchronise through counters and self-validating mailbox entries only; repeat
-  // the launch and compare the result bit for bit (argv[4] = repetitions)
-  const int reps = argc > 4 ? atoi(argv[4]) : 0;
+  // the launch and compare the result bit for bit (argv[3] = repetitions)
+  const int reps = argc > 3 ? atoi(argv[3]) : 0;
   int bad = 0;
   for (int r = 0; r < reps; r++) {
     CKC(cudaMemcpy(da, h.data(), nd * 8, cudaMemcpyHostToDevice));

@@ -460,33 +460,25 @@ def test_wavelet_filter(gpu, N, nl, afilt, modal):
     assert np.array_equal(mg.get(G.Q), mo.get(O.Q))
 
 
-@pytest.mark.parametrize("mode", ["MSQG_MG=rr", "MSQG_MG=fused", "MSQG_RELAX_CS=2", "MSQG_RELAX_CS=4", "MSQG_RELAX=v3", "MSQG_RHS=gather"])
-def test_fused_cycle_tail_variants(gpu, mode):
-    """Measured-and-rejected variants kept behind environment switches (read once per process, hence the subprocess)
-    give the same bits, cycle counts and dt as the oracle: MSQG_MG=rr / fused (k_corr_res fusions of correction +
-    residual + first restriction) and MSQG_RELAX_CS=2 / 4 (relax hand-off between the CTAs of a thread-block cluster
-    through distributed shared memory), MSQG_RELAX=v3 (single-warp wavefront k_relax_lex) and MSQG_RHS=gather
-    (L1-gather right-hand side k_rhs instead of the tiled k_rhs_t).  All but MSQG_RHS=gather exist only in a library built
-    with `make EXPERIMENTS=1` (the default library carries one relax kernel per smoother)."""
+@pytest.mark.parametrize("smoother", ["lex", "rb"])
+@pytest.mark.parametrize("N,nl", [(128, 3), (256, 4), (32, 2)])
+def test_rhs_gather_variant(gpu, N, nl, smoother):
+    """MSQG_RHS=gather (L1-gather right-hand side k_rhs instead of the tiled k_rhs_t; the switch is read once per
+    process, hence the subprocess) gives the same bits, cycle counts and dt as the oracle, with both sweep orders."""
     import subprocess, sys
-    from msom_b200 import capi as G0
-    G0.lib().msqg_has_experiments.restype = int
-    if mode != "MSQG_RHS=gather" and not G0.lib().msqg_has_experiments():
-        pytest.skip("rejected variant: built with EXPERIMENTS=1 only")
     code = (
         "import sys, numpy as np\n"
         "sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
         "from common import make_pair\n"
         "from oracle import oracle as O\n"
         "from msom_b200 import capi as G\n"
-        "for N, nl in ((128, 3), (256, 4), (32, 2)):\n"
-        "    mo, mg, _ = make_pair(N, nl)\n"
-        "    mo.set_const(); mg.set_const()\n"
-        "    for _ in range(3):\n"
-        "        assert mg.step() == mo.step()\n"
-        "    assert np.array_equal(mg.get(G.Q), mo.get(O.Q)) and np.array_equal(mg.get(G.PSI), mo.get(O.PSI))\n"
-        "    assert mg.total_cycles == mo.L.orc_total_cycles(mo.h)\n"
-        "print('ok')\n") % (ROOT, os.path.join(ROOT, "tests"))
-    env = dict(os.environ, **dict([mode.split("=")]))
+        "mo, mg, _ = make_pair(%d, %d, smoother=%r)\n"
+        "mo.set_const(); mg.set_const()\n"
+        "for _ in range(3):\n"
+        "    assert mg.step() == mo.step()\n"
+        "assert np.array_equal(mg.get(G.Q), mo.get(O.Q)) and np.array_equal(mg.get(G.PSI), mo.get(O.PSI))\n"
+        "assert mg.total_cycles == mo.L.orc_total_cycles(mo.h)\n"
+        "print('ok')\n") % (ROOT, os.path.join(ROOT, "tests"), N, nl, smoother)
+    env = dict(os.environ, MSQG_RHS="gather")
     out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
     assert out.returncode == 0 and "ok" in out.stdout, out.stdout + out.stderr
