@@ -263,9 +263,9 @@ double msqg_ensemble_time(msqg_ensemble *e, int k);
 
 /* ---- (1b) 2-D domain decomposition: one tile per GPU, halo exchange == boundary() -------------
  * The semantics of the reference built with -D_MPI=1 (msqg/qg.c:12-19): px x py tiles on every
- * multigrid level whose global size is >= agg_n (coarser levels are agglomerated on tile (0,0)),
- * lexicographic Gauss-Seidel inside each tile with the neighbours' pre-sweep halo, halo exchange
- * after every sweep.  `local` keeps all tiles in one process on one device (tests / emulation),
+ * multigrid level whose global size is >= agg_n (coarser levels are gathered onto one tile per
+ * process and solved there with the undecomposed arithmetic), lexicographic Gauss-Seidel inside
+ * each tile with the neighbours' pre-sweep halo, halo exchange after every sweep.  `local` keeps all tiles in one process on one device (tests / emulation),
  * `nccl` is one tile per process: rank = iy*px + ix, uid from msqg_nccl_unique_id on rank 0.
  * Field buffers are the TILE's [nf][ny][nx] block of the global [nf][N][N] array. */
 typedef struct msqg_group msqg_group;
@@ -281,8 +281,8 @@ int msqg_group_create_nccl(const msqg_params *p, int device, int px, int py, int
  * cells per side there: at nl >= 10 a grid of 4 or more tiles across (4 x 2, 2 x 4, ...) is refused (MSQG_ERR_ARG).
  * The same with the smoother named (msqg_set_smoother): 1 = red-black.  A red-black group gives the bits of the
  * single-GPU red-black solve whatever px, py and agg_n are (a half-sweep is decomposition independent); levels with
- * fewer than agg_n cells per side are replicated on every GPU (all-gather of the restricted residual, redundant coarse
- * solve) and the sweeps of a distributed level need ONE halo exchange (deep halos, communication-avoiding).
+ * fewer than agg_n cells per side are solved once per process (under NCCL: all-gather of the restricted residual,
+ * redundant coarse solve on every GPU) and the sweeps of a distributed level need ONE halo exchange (deep halos, communication-avoiding).
  * Groups run the layer-coupled inversion; a closed-basin red-black group also runs the vertical-mode inversion
  * (p->mode_pv_invert) when the modes are uniform: varRo <= 0 and the same Fr on every tile (msqg_group_set_const checks
  * it).  Stochastic forcing (p->stochastic) runs on every group, periodic or closed, both smoothers: each tile draws its
@@ -294,7 +294,8 @@ int msqg_group_create_local_sm(const msqg_params *p, int device, int px, int py,
 int msqg_group_create_nccl_sm(const msqg_params *p, int device, int px, int py, int agg_n, int smoother, int rank, int nranks,
                               const void *uid128, msqg_group **out);
 int msqg_group_smoother(msqg_group *g);
-/* 1: halos move by direct stores into the neighbours' memory (CUDA IPC over NVLink, dist_rb.cuh); 0: ncclSend/ncclRecv */
+/* either smoother: 1: halos move by direct stores into the neighbours' memory (CUDA IPC over NVLink, dist_rb.cuh);
+ * 0: staged device copies (local) or ncclSend/ncclRecv (environment MSQG_P2P=0, and periodic groups) */
 int msqg_group_transport(msqg_group *g);
 void msqg_group_destroy(msqg_group *g);
 int msqg_group_ntiles(msqg_group *g);                       /* tiles held by this process */

@@ -1,19 +1,22 @@
 /*
  * dist_impl.cuh -- 2-D domain decomposition of the msqg timestep (included by model.cu).
  *
- * Semantics = the reference built with -D_MPI=1 (msqg/qg.c:12-19): every rank owns a px x py tile on
- * each multigrid level; a relaxation sweep is lexicographic Gauss-Seidel INSIDE the tile with the
- * neighbours' pre-sweep values in the halo, refreshed after every sweep (boundary_level ==
- * halo exchange, [BASILISK] C3 of SURVEY.md 2c); every other operator is order-independent.  Levels
- * whose global size is below `agg_n` are agglomerated onto tile (0,0) and swept serially there.
- * This is exactly what oracle/msqg_oracle.c emulates with orc_set_decomp(px, py, agg_n), so the
- * decomposed GPU path is checked bit for bit against the CPU oracle.
+ * Every group runs on the same tile machinery: the 8-neighbour halo exchange, the coarse levels and the cycle of
+ * dist_rb.cuh.  Only the sweeps of a distributed level depend on the smoother:
+ *   lexicographic (smoother 0): the reference built with -D_MPI=1 (msqg/qg.c:12-19).  A relaxation sweep is
+ *     lexicographic Gauss-Seidel INSIDE the tile with the neighbours' pre-sweep values in a one-cell halo, refreshed
+ *     after every sweep (boundary_level == halo exchange, [BASILISK] C3 of SURVEY.md 2c); every other operator is
+ *     order-independent.  This is exactly what oracle/msqg_oracle.c emulates with orc_set_decomp(px, py, agg_n), so
+ *     the decomposed GPU path is checked bit for bit against the CPU oracle;
+ *   red-black (smoother 1): decomposition independent, deep halos, one exchange per level and cycle (dist_rb.cuh).
+ * Levels whose global size is below `agg_n` are gathered onto one tile per process and solved there by the
+ * undecomposed multigrid (mg_levels): the arithmetic of the reference's serial solve of those levels.
  *
- * Two exchange back-ends behind the same driver:
- *   local : all tiles live in this process on one device (tests, 1-GPU emulation): device copies
- *   nccl  : one tile per process/GPU: grouped ncclSend/ncclRecv on the model stream (NVLink),
- *           ncclAllReduce for the 8-byte reductions.  NCCL is loaded lazily with dlopen.
- * Halo exchange is x-phase then y-phase (rows include the ghost columns) so corner ghosts propagate.
+ * Two back-ends behind the same driver:
+ *   local : all tiles live in this process on one device (tests, 1-GPU emulation): direct stores or device copies
+ *   nccl  : one tile per process/GPU: direct stores into the neighbours' memory (CUDA IPC) or grouped
+ *           ncclSend/ncclRecv on the model stream (NVLink), ncclAllReduce for the 8-byte reductions.  NCCL is loaded
+ *           lazily with dlopen.
  */
 #pragma once
 
@@ -68,41 +71,7 @@ extern "C" int msqg_nccl_unique_id(void *out128) {
   return MSQG_OK;
 }
 
-/* ------------------------------------------------------------------ exchange kernels */
-__global__ void k_pack_cols(const double *__restrict__ a, int nf, Geom g, double *__restrict__ bl, double *__restrict__ br) {
-  const int y = blockIdx.x * blockDim.x + threadIdx.x, f = blockIdx.y;
-  if (y >= g.ny) return;
-  const double *p = a + (size_t)f * g.plane;
-  bl[(size_t)f * g.ny + y] = p[GIDX(g.pitch, y, 0)];
-  br[(size_t)f * g.ny + y] = p[GIDX(g.pitch, y, g.nx - 1)];
-}
-__global__ void k_unpack_cols(double *__restrict__ a, int nf, Geom g, const double *__restrict__ fl, const double *__restrict__ fr) {
-  const int y = blockIdx.x * blockDim.x + threadIdx.x, f = blockIdx.y;
-  if (y >= g.ny) return;
-  double *p = a + (size_t)f * g.plane;
-  if (g.bc & 1) p[GIDX(g.pitch, y, -1)] = fl[(size_t)f * g.ny + y];
-  if (g.bc & 2) p[GIDX(g.pitch, y, g.nx)] = fr[(size_t)f * g.ny + y];
-}
-__global__ void k_pack_rows(const double *__restrict__ a, int nf, Geom g, double *__restrict__ bb, double *__restrict__ bt) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x - 1, f = blockIdx.y;
-  if (x > g.nx) return;
-  const double *p = a + (size_t)f * g.plane;
-  bb[(size_t)f * (g.nx + 2) + x + 1] = p[GIDX(g.pitch, 0, x)];
-  bt[(size_t)f * (g.nx + 2) + x + 1] = p[GIDX(g.pitch, g.ny - 1, x)];
-}
-__global__ void k_unpack_rows(double *__restrict__ a, int nf, Geom g, const double *__restrict__ fb, const double *__restrict__ ft) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x - 1, f = blockIdx.y;
-  if (x > g.nx) return;
-  double *p = a + (size_t)f * g.plane;
-  if (g.bc & 4) p[GIDX(g.pitch, -1, x)] = fb[(size_t)f * (g.nx + 2) + x + 1];
-  if (g.bc & 8) p[GIDX(g.pitch, g.ny, x)] = ft[(size_t)f * (g.nx + 2) + x + 1];
-}
-/* gather: contiguous tile block [nf][hy][hx] -> interior of the full padded level at (ox, oy) */
-__global__ void k_place(double *__restrict__ full, Geom gfull, const double *__restrict__ src, int hx, int hy, int ox, int oy) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y, f = blockIdx.z;
-  if (x >= hx || y >= hy) return;
-  full[(size_t)f * gfull.plane + GIDX(gfull.pitch, oy + y, ox + x)] = src[((size_t)f * hy + y) * hx + x];
-}
+/* ------------------------------------------------------------------ coarse-level patch kernels */
 /* scatter: (hx+2) x (hy+2) patch around the tile block of the full level; values outside the
  * domain are the homogeneous-dirichlet ghosts of da (coarse_at with bc = 0) */
 __global__ void k_extract_patch(const double *__restrict__ full, Geom gfull, double *__restrict__ dst, int hx, int hy, int ox, int oy,
@@ -126,8 +95,8 @@ __global__ void k_load_patch(double *__restrict__ dst, Geom gp, const double *__
 struct msqg_group {
   msqg_params p;
   int px, py, agg_n, device, kind; /* kind 0 local, 1 nccl */
-  int rb;                          /* red-black smoother: replicated coarse levels, deep halos (dist_rb.cuh) */
-  int p2p;                         /* halo exchange by direct stores into the neighbours' memory (CUDA IPC) instead of NCCL */
+  int rb;                          /* red-black smoother (deep halos, dist_rb.cuh); 0: lexicographic */
+  int p2p;                         /* halo exchange by direct stores into the neighbours' memory instead of staged copies / NCCL */
   int rank, nranks;
   std::vector<msqg_model *> tiles; /* local: all tiles, index iy*px+ix; nccl: this rank's tile */
   cudaStream_t stream;
@@ -148,89 +117,11 @@ static inline int tile_rank(msqg_group *G, int ix, int iy) { return ((iy + G->py
 static inline msqg_model *tile_at(msqg_group *G, int ix, int iy) {
   return G->kind == 0 ? G->tiles[tile_rank(G, ix, iy)] : G->tiles[0];
 }
-static inline msqg_model *root_tile(msqg_group *G) { return (G->kind == 0 || G->rank == 0) ? G->tiles[0] : nullptr; }
-
-typedef double *(*tile_ptr_fn)(msqg_model *, int);
-static double *ptr_da(msqg_model *m, int l) { return m->da.lev[l]; }
-static double *ptr_patch(msqg_model *m, int) { return m->da_patch; }
-
-/* halo exchange of `nf` planes of the array ptr(tile) with geometry geo(tile) */
-static int halo_exchange(msqg_group *G, std::vector<double *> &arr, std::vector<Geom> &geo, int nf) {
-  G->exchanges++;
-  const int nt = (int)G->tiles.size();
-  for (int phase = 0; phase < 2; phase++) {
-    /* pack */
-    for (int t = 0; t < nt; t++) {
-      msqg_model *m = G->tiles[t];
-      const Geom &g = geo[t];
-      if (phase == 0) k_pack_cols<<<dim3((g.ny + 127) / 128, nf), 128, 0, G->stream>>>(arr[t], nf, g, m->halo_send[0], m->halo_send[1]);
-      else k_pack_rows<<<dim3((g.nx + 2 + 127) / 128, nf), 128, 0, G->stream>>>(arr[t], nf, g, m->halo_send[2], m->halo_send[3]);
-    }
-    CK(cudaGetLastError());
-    /* transfer: side 0 <-> neighbour's side 1 (x), side 2 <-> neighbour's side 3 (y) */
-    if (G->kind == 0) {
-      for (int t = 0; t < nt; t++) {
-        msqg_model *m = G->tiles[t];
-        const Geom &g = geo[t];
-        const size_t cnt = (size_t)nf * (phase == 0 ? g.ny : g.nx + 2) * sizeof(double);
-        const int lo = phase == 0 ? 0 : 2, hi = lo + 1;
-        if (g.bc & (phase == 0 ? 1 : 4)) { /* neighbour on the low side: its high-side send -> my low-side recv */
-          msqg_model *nb = phase == 0 ? tile_at(G, m->ix - 1, m->iy) : tile_at(G, m->ix, m->iy - 1);
-          CK(cudaMemcpyAsync(m->halo_recv[lo], nb->halo_send[hi], cnt, cudaMemcpyDeviceToDevice, G->stream));
-        }
-        if (g.bc & (phase == 0 ? 2 : 8)) {
-          msqg_model *nb = phase == 0 ? tile_at(G, m->ix + 1, m->iy) : tile_at(G, m->ix, m->iy + 1);
-          CK(cudaMemcpyAsync(m->halo_recv[hi], nb->halo_send[lo], cnt, cudaMemcpyDeviceToDevice, G->stream));
-        }
-      }
-    } else {
-      msqg_model *m = G->tiles[0];
-      const Geom &g = geo[0];
-      const size_t cnt = (size_t)nf * (phase == 0 ? g.ny : g.nx + 2);
-      const int lo = phase == 0 ? 0 : 2, hi = lo + 1;
-      NCK(G->nccl->GroupStart());
-      if (g.bc & (phase == 0 ? 1 : 4)) {
-        const int peer = phase == 0 ? tile_rank(G, m->ix - 1, m->iy) : tile_rank(G, m->ix, m->iy - 1);
-        NCK(G->nccl->Send(m->halo_send[lo], cnt, NCCL_DOUBLE, peer, G->comm, G->stream));
-        NCK(G->nccl->Recv(m->halo_recv[lo], cnt, NCCL_DOUBLE, peer, G->comm, G->stream));
-      }
-      if (g.bc & (phase == 0 ? 2 : 8)) {
-        const int peer = phase == 0 ? tile_rank(G, m->ix + 1, m->iy) : tile_rank(G, m->ix, m->iy + 1);
-        NCK(G->nccl->Send(m->halo_send[hi], cnt, NCCL_DOUBLE, peer, G->comm, G->stream));
-        NCK(G->nccl->Recv(m->halo_recv[hi], cnt, NCCL_DOUBLE, peer, G->comm, G->stream));
-      }
-      NCK(G->nccl->GroupEnd());
-    }
-    /* unpack */
-    for (int t = 0; t < nt; t++) {
-      msqg_model *m = G->tiles[t];
-      const Geom &g = geo[t];
-      if (phase == 0) k_unpack_cols<<<dim3((g.ny + 127) / 128, nf), 128, 0, G->stream>>>(arr[t], nf, g, m->halo_recv[0], m->halo_recv[1]);
-      else k_unpack_rows<<<dim3((g.nx + 2 + 127) / 128, nf), 128, 0, G->stream>>>(arr[t], nf, g, m->halo_recv[2], m->halo_recv[3]);
-    }
-    CK(cudaGetLastError());
-  }
-  return MSQG_OK;
-}
 static int exchange_one(msqg_group *G, int id, int lev, int w, int ring);
 static int exchange_list(msqg_group *G, int id, int lev) {
-  /* red-black groups: the 8-neighbour exchange, which also carries the ghost ring of the physical sides along the
-     tile edges, so every halo cell (corners included) holds exactly the value of the undecomposed field */
-  if (G->rb) return exchange_one(G, id, lev, 1, 1);
-  std::vector<double *> arr;
-  std::vector<Geom> geo;
-  int nf = 0;
-  for (msqg_model *m : G->tiles) {
-    List *L = list_by_id(m, id);
-    arr.push_back(L->lev[lev]); geo.push_back(m->g[lev]); nf = L->nf;
-  }
-  return halo_exchange(G, arr, geo, nf);
-}
-static int exchange_da(msqg_group *G, int lev) {
-  std::vector<double *> arr;
-  std::vector<Geom> geo;
-  for (msqg_model *m : G->tiles) { arr.push_back(m->da.lev[lev]); geo.push_back(m->g[lev]); }
-  return halo_exchange(G, arr, geo, G->p.nl);
+  /* the 8-neighbour exchange, which also carries the ghost ring of the physical sides along the tile edges, so every
+     halo cell (corners included) holds exactly the value of the undecomposed field */
+  return exchange_one(G, id, lev, 1, 1);
 }
 
 /* max over tiles/ranks of n doubles that every tile holds at d_scal + off: enqueue (capturable in a CUDA graph),
@@ -354,7 +245,8 @@ static int group_create(const msqg_params *p, int device, int px, int py, int ag
     for (int iy = 0; iy < py; iy++)
       for (int ix = 0; ix < px; ix++) {
         msqg_model *m;
-        if ((rc = create_model(p, device, px, py, ix, iy, agg_n, G->stream, &m, G->rb))) return rc;
+        /* the levels below agg_n live on tiles[0] only (the solver tile of the process) */
+        if ((rc = create_model(p, device, px, py, ix, iy, agg_n, G->stream, &m, G->rb, G->tiles.empty()))) return rc;
         m->smoother = G->rb;
         m->tile_index = (int)G->tiles.size();
         G->tiles.push_back(m);
@@ -366,21 +258,20 @@ static int group_create(const msqg_params *p, int device, int px, int py, int ag
     memcpy(&id, uid, 128);
     NCK(G->nccl->CommInitRank(&G->comm, nranks, id, rank));
     msqg_model *m;
-    if ((rc = create_model(p, device, px, py, rank % px, rank / px, agg_n, G->stream, &m, G->rb))) return rc;
+    if ((rc = create_model(p, device, px, py, rank % px, rank / px, agg_n, G->stream, &m, G->rb, true))) return rc;
     m->smoother = G->rb;
     G->tiles.push_back(m);
   }
   G->p2p = 0;
-  if (G->rb) {
-    int want = 1;
-    { const char *e = getenv("MSQG_P2P"); if (e && atoi(e) == 0) want = 0; }
-    if (per) want = 0; /* a tile may be its own neighbour in several directions: staged device copies */
-    if (want && (rc = group_setup_p2p(G))) return rc;
-  }
+  int want = 1;
+  { const char *e = getenv("MSQG_P2P"); if (e && atoi(e) == 0) want = 0; }
+  if (per) want = 0; /* a tile may be its own neighbour in several directions: staged device copies */
+  if (want && (rc = group_setup_p2p(G))) return rc;
   *out = G;
   return MSQG_OK;
 }
-extern "C" int msqg_group_transport(msqg_group *G) { return G->p2p; } /* 1: peer-memory halo exchange, 0: NCCL send/recv */
+/* 1: peer-memory halo exchange, 0: staged device copies (local group) or NCCL send/recv */
+extern "C" int msqg_group_transport(msqg_group *G) { return G->p2p; }
 extern "C" int msqg_group_create_local(const msqg_params *p, int device, int px, int py, int agg_n, msqg_group **out) {
   return group_create(p, device, px, py, agg_n, 0, 0, 1, nullptr, out);
 }
@@ -470,106 +361,6 @@ static int g_relax_level(msqg_group *G, msqg_model *m, int l, int nsweeps) {
   return rc;
 }
 
-static int g_cycle(msqg_group *G, int nrelax) {
-  msqg_model *m0 = G->tiles[0];
-  const int D = m0->depth, La = m0->agg_level, nl = G->p.nl;
-  dim3 b(32, 8);
-  /* restriction(res) on the distributed levels, then onto this tile's share of level La-1 */
-  for (msqg_model *m : G->tiles) {
-    for (int l = D - 1; l >= La; l--) {
-      k_restrict<<<grid2(m->g[l].nx, m->g[l].ny, b, nl), b, 0, G->stream>>>(m->res.lev[l + 1], m->res.lev[l], m->g[l + 1], m->g[l], -1., 0);
-      m->launches++;
-    }
-    k_restrict<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nl), b, 0, G->stream>>>(m->res.lev[La], m->res_patch, m->g[La], m->gpatch, -1., 0);
-    k_unpack<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nl), b, 0, G->stream>>>(m->patch_stage, m->res_patch, nl, m->gpatch);
-    m->launches += 2;
-  }
-  CK(cudaGetLastError());
-  /* gather onto tile (0,0) */
-  msqg_model *root = root_tile(G);
-  const int hx = m0->gpatch.nx, hy = m0->gpatch.ny;
-  const size_t blk = (size_t)nl * hx * hy;
-  if (G->kind == 0) {
-    for (msqg_model *m : G->tiles) {
-      k_place<<<grid2(hx, hy, b, nl), b, 0, G->stream>>>(root->res.lev[La - 1], root->g[La - 1], m->patch_stage, hx, hy, m->ix * hx, m->iy * hy);
-      root->launches++;
-    }
-  } else {
-    if (G->rank == 0) {
-      k_place<<<grid2(hx, hy, b, nl), b, 0, G->stream>>>(root->res.lev[La - 1], root->g[La - 1], root->patch_stage, hx, hy, 0, 0);
-      for (int r = 1; r < G->nranks; r++) {
-        NCK(G->nccl->Recv(root->d_stage, blk, NCCL_DOUBLE, r, G->comm, G->stream));
-        k_place<<<grid2(hx, hy, b, nl), b, 0, G->stream>>>(root->res.lev[La - 1], root->g[La - 1], root->d_stage, hx, hy, (r % G->px) * hx, (r / G->px) * hy);
-      }
-    } else
-      NCK(G->nccl->Send(m0->patch_stage, blk, NCCL_DOUBLE, 0, G->comm, G->stream));
-  }
-  CK(cudaGetLastError());
-  int rc;
-  if (root) {
-    /* agglomerated levels: serial reference sweep on one GPU */
-    for (int l = La - 2; l >= 1; l--) {
-      k_restrict<<<grid2(root->g[l].nx, root->g[l].ny, b, nl), b, 0, G->stream>>>(root->res.lev[l + 1], root->res.lev[l], root->g[l + 1], root->g[l], -1., 0);
-      root->launches++;
-    }
-    for (int l = 1; l <= La - 1; l++) {
-      const Geom &g = root->g[l];
-      if (l == 1) CK(cudaMemsetAsync(root->da.lev[l], 0, (size_t)nl * g.plane * sizeof(double), G->stream));
-      else {
-        launch_prolong(G->stream, nl, root->da.lev[l - 1], root->da.lev[l], root->g[l - 1], g);
-        root->launches++;
-      }
-      if ((rc = g_relax_level(G, root, l, nrelax))) return rc;
-    }
-  }
-  /* scatter level La-1 of da: each tile gets its block plus a one-cell ring */
-  const size_t pblk = (size_t)nl * (hx + 2) * (hy + 2);
-  if (G->kind == 0) {
-    for (msqg_model *m : G->tiles) {
-      k_extract_patch<<<grid2(hx + 2, hy + 2, b, nl), b, 0, G->stream>>>(root->da.lev[La - 1], root->g[La - 1], m->patch_stage, hx, hy, m->ix * hx, m->iy * hy, 0);
-      k_load_patch<<<grid2(hx + 2, hy + 2, b, nl), b, 0, G->stream>>>(m->da_patch, m->gpatch, m->patch_stage);
-      m->launches += 2;
-    }
-  } else {
-    if (G->rank == 0) {
-      for (int r = 1; r < G->nranks; r++) {
-        k_extract_patch<<<grid2(hx + 2, hy + 2, b, nl), b, 0, G->stream>>>(root->da.lev[La - 1], root->g[La - 1], root->d_stage, hx, hy, (r % G->px) * hx, (r / G->px) * hy, 0);
-        NCK(G->nccl->Send(root->d_stage, pblk, NCCL_DOUBLE, r, G->comm, G->stream));
-      }
-      k_extract_patch<<<grid2(hx + 2, hy + 2, b, nl), b, 0, G->stream>>>(root->da.lev[La - 1], root->g[La - 1], root->patch_stage, hx, hy, 0, 0, 0);
-    } else
-      NCK(G->nccl->Recv(m0->patch_stage, pblk, NCCL_DOUBLE, 0, G->comm, G->stream));
-    k_load_patch<<<grid2(hx + 2, hy + 2, b, nl), b, 0, G->stream>>>(m0->da_patch, m0->gpatch, m0->patch_stage);
-  }
-  CK(cudaGetLastError());
-  /* distributed levels: prolong, halo, nrelax x { one sweep inside the tile, halo } */
-  for (int l = La; l <= D; l++) {
-    for (msqg_model *m : G->tiles) {
-      const Geom &g = m->g[l];
-      ProfScope ps(m, PROF_PROLONG, l);
-      if (l == La) launch_prolong(G->stream, nl, m->da_patch, m->da.lev[l], m->gpatch, g);
-      else launch_prolong(G->stream, nl, m->da.lev[l - 1], m->da.lev[l], m->g[l - 1], g);
-      m->launches++;
-    }
-    CK(cudaGetLastError());
-    if ((rc = exchange_da(G, l))) return rc;
-    for (int s = 0; s < nrelax; s++) {
-      for (msqg_model *m : G->tiles)
-        if ((rc = g_relax_level(G, m, l, 1))) return rc;
-      if ((rc = exchange_da(G, l))) return rc;
-    }
-  }
-  /* a += da ; boundary(a) */
-  for (msqg_model *m : G->tiles) {
-    const Geom &g = m->g[D];
-    ProfScope ps(m, PROF_CORRECT, 0);
-    k_correct<<<grid2(g.nx, g.ny, b, nl), b, 0, G->stream>>>(m->psi.lev[D], m->da.lev[D], g);
-    m->launches++;
-  }
-  CK(cudaGetLastError());
-  return exchange_list(G, MSQG_PSI, D);
-}
-
 static int g_check_err(msqg_group *G) {
   for (msqg_model *m : G->tiles) {
     int rc = check_relax_err(m);
@@ -590,26 +381,21 @@ static int g_solve(msqg_group *G, const std::vector<MgProblem> &P, msqg_mgstats 
   if ((rc = g_residual(G, P, &resb))) return rc;
   s.resb = s.resa = resb;
   for (s.i = 0; s.i < 100 && (s.i < 1 || s.resa > 1e-3); s.i++) {
-    if (G->rb) {
-      /* one cycle + residual + its all-reduce: a single graph launch (keyed by nrelax, the mode, the unknown and the
-         right-hand side of tile 0 and the current da buffers of every tile) */
-      msqg_model *m0 = G->tiles[0];
-      unsigned long long mask = 0;
-      for (msqg_model *m : G->tiles) mask = mask * 1315423911ull + da_parity_mask(m);
-      bool graphed = m0->use_graphs != 0;
-      for (msqg_model *m : G->tiles) graphed = graphed && !m->prof_on;
-      GraphKey key(s.nrelax, P[0].mode, (const void *)P[0].a, (const void *)P[0].b, mask);
-      rc = run_graphed(G->stream, G->graphs, key, G->tiles, &G->exchanges, graphed, [&]() -> int {
-        int r2 = g_cycle_rb(G, P, s.nrelax);
-        if (r2) return r2;
-        return g_residual_enqueue(G, P);
-      });
-      if (rc) return rc;
-      if ((rc = reduce_max_finish(G, 1, &s.resa))) return rc;
-    } else {
-      if ((rc = g_cycle(G, s.nrelax))) return rc;
-      if ((rc = g_residual(G, P, &s.resa))) return rc;
-    }
+    /* one cycle + residual + its all-reduce: with the red-black smoother a single graph launch (keyed by nrelax, the
+       mode, the unknown and the right-hand side of tile 0 and the current da buffers of every tile) */
+    msqg_model *m0 = G->tiles[0];
+    unsigned long long mask = 0;
+    for (msqg_model *m : G->tiles) mask = mask * 1315423911ull + da_parity_mask(m);
+    bool graphed = G->rb && m0->use_graphs != 0;
+    for (msqg_model *m : G->tiles) graphed = graphed && !m->prof_on;
+    GraphKey key(s.nrelax, P[0].mode, (const void *)P[0].a, (const void *)P[0].b, mask);
+    rc = run_graphed(G->stream, G->graphs, key, G->tiles, &G->exchanges, graphed, [&]() -> int {
+      int r2 = g_cycle(G, P, s.nrelax);
+      if (r2) return r2;
+      return g_residual_enqueue(G, P);
+    });
+    if (rc) return rc;
+    if ((rc = reduce_max_finish(G, 1, &s.resa))) return rc;
     if (s.resa > 1e-3) {
       if (resb / s.resa < 1.2 && s.nrelax < 100) s.nrelax++;
       else if (resb / s.resa > 10 && s.nrelax > 2) s.nrelax--;

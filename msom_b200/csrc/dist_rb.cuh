@@ -1,22 +1,28 @@
 /*
- * dist_rb.cuh -- multigrid cycle of a px x py group of tiles with the red-black smoother (included by model.cu).
+ * dist_rb.cuh -- halo exchange and multigrid cycle of a px x py group of tiles (included by model.cu), for both smoothers.
  *
  * A red-black half-sweep only reads cells of the other colour, so a decomposed sweep gives the SAME bits as the
  * undecomposed one provided every tile sees current values in its halo -- unlike the reference's lexicographic sweep,
  * whose result depends on the MPI decomposition (msqg/poisson_layer.h:55-65; run as `mpirun -np 16`, msqg/qg.c:12-19).
- * The group therefore reproduces the single-GPU red-black result bit for bit on 1, 2, 4 and 8 GPUs, and it does so with
- * ONE halo exchange per level and cycle instead of one per sweep:
+ * The red-black group therefore reproduces the single-GPU red-black result bit for bit on 1, 2, 4 and 8 GPUs, and it
+ * does so with ONE halo exchange per level and cycle instead of one per sweep:
  *
  *   - the planes of a tile carry a frame of MSQG_FRAME cells (layout.cuh); before the nrelax sweeps of a level the
  *     tiles exchange a halo of 2 nrelax + 1 cells of da (and, once per cycle for all levels, 2 nrelax cells of res);
  *     k_relax_rb then runs all sweeps on tile + halo, recomputing the neighbours' border cells: after h half-sweeps the
  *     outermost h halo cells are stale and are simply not used any more (communication-avoiding smoothing);
- *   - one halo cell survives the sweeps, which is what the bilinear prolongation to the next level reads;
- *   - the exchange moves the 4 sides and 4 corners in ONE grouped ncclSend/ncclRecv (8 neighbours) -- corners go
- *     straight to the diagonal neighbour, no x-phase/y-phase;
- *   - levels below the agglomeration threshold (global size < agg_n) are REPLICATED: the restricted residual is
- *     all-gathered (ncclAllGather) and every GPU runs the small coarse solve redundantly, so nothing is scattered back
- *     and no GPU idles while one of them works (SURVEY.md section 5).
+ *   - one halo cell survives the sweeps, which is what the bilinear prolongation to the next level reads.
+ * The lexicographic group exchanges a one-cell halo of da before its first sweep and after every one (block Gauss-Seidel).
+ *
+ * Shared by both smoothers:
+ *   - the exchange moves the 4 sides and 4 corners in ONE step (8 neighbours): direct stores into the neighbours'
+ *     memory, or staged device copies / one grouped ncclSend/ncclRecv -- corners go straight to the diagonal
+ *     neighbour, no x-phase/y-phase;
+ *   - levels below the agglomeration threshold (global size < agg_n) are solved ONCE PER PROCESS, on its tiles[0]:
+ *     the restricted residual is gathered there (under NCCL all-gathered, so every GPU runs the small coarse solve
+ *     redundantly, nothing is scattered back and no GPU idles while one of them works, SURVEY.md section 5), and each
+ *     tile takes its block of the result;
+ *   - the correction updates the one halo cell of psi that da still holds, so psi needs no exchange after a cycle.
  * Scalars: one ncclAllReduce(max) per cycle for the residual norm.
  */
 #pragma once
@@ -353,10 +359,11 @@ __global__ void k_correct_ring(double *__restrict__ a, const double *__restrict_
 }
 
 /* one cycle of the problem P[t] of every tile t: the layer-coupled solve (nl, -1, psi, q) or the scalar Helmholtz
- * solve of one vertical mode (1, mode, plane `mode` of pm, of qm) */
-static int g_cycle_rb(msqg_group *G, const std::vector<MgProblem> &P, int nrelax) {
-  msqg_model *m0 = G->tiles[0];
-  const int D = m0->depth, La = m0->agg_level, nf = P[0].nf, mode = P[0].mode;
+ * solve of one vertical mode (1, mode, plane `mode` of pm, of qm; red-black only) */
+static int g_cycle(msqg_group *G, const std::vector<MgProblem> &P, int nrelax) {
+  /* S = tiles[0] (this rank's tile under NCCL) solves the levels below agg_level; every tile has its geometry */
+  msqg_model *S = G->tiles[0];
+  const int D = S->depth, La = S->agg_level, nf = P[0].nf, mode = P[0].mode;
   const int nt = (int)G->tiles.size(), nranks = G->px * G->py;
   dim3 b(32, 8);
   int rc;
@@ -372,31 +379,36 @@ static int g_cycle_rb(msqg_group *G, const std::vector<MgProblem> &P, int nrelax
     m->launches += 2;
   }
   CK(cudaGetLastError());
-  /* every tile receives every tile's block of level La-1 (all-gather) and assembles the full level */
-  const int hx = m0->gpatch.nx, hy = m0->gpatch.ny;
+  /* the solver tile receives every tile's block of level La-1 (under NCCL every rank's tile: all-gather) */
+  const int hx = S->gpatch.nx, hy = S->gpatch.ny;
   const size_t blk = (size_t)nf * hx * hy;
   if (G->kind == 0) {
-    for (msqg_model *m : G->tiles)
-      for (int r = 0; r < nt; r++)
-        CK(cudaMemcpyAsync(m->gather_buf + (size_t)r * blk, G->tiles[r]->patch_stage, blk * sizeof(double), cudaMemcpyDeviceToDevice, G->stream));
+    for (int r = 0; r < nt; r++)
+      CK(cudaMemcpyAsync(S->gather_buf + (size_t)r * blk, G->tiles[r]->patch_stage, blk * sizeof(double), cudaMemcpyDeviceToDevice, G->stream));
   } else {
-    ProfScope ps_g(m0, PROF_XCHG, 100);
-    NCK(G->nccl->AllGather(m0->patch_stage, m0->gather_buf, blk, NCCL_DOUBLE, G->comm, G->stream));
+    ProfScope ps_g(S, PROF_XCHG, 100);
+    NCK(G->nccl->AllGather(S->patch_stage, S->gather_buf, blk, NCCL_DOUBLE, G->comm, G->stream));
   }
-  const int chunk0 = nrelax < 7 ? nrelax : 7;
-  /* replicated coarse levels: every tile solves levels 1 .. La-1 (same arithmetic, same bits everywhere) */
+  /* levels 1 .. La-1 on the solver tile: the undecomposed multigrid, whose arithmetic does not depend on the tiles */
+  k_place_all<<<grid2(hx, hy, b, nranks * nf), b, 0, G->stream>>>(S->res.lev[La - 1], S->g[La - 1], S->gather_buf, hx, hy, G->px, nranks, nf);
+  S->launches++;
+  if ((rc = mg_levels(S, nf, mode, nrelax, La - 1, La - 1))) return rc;
+  /* every tile's block of level La-1 plus a one-cell ring (homogeneous dirichlet ghosts evaluated on the fly) */
   for (msqg_model *m : G->tiles) {
-    k_place_all<<<grid2(hx, hy, b, nranks * nf), b, 0, G->stream>>>(m->res.lev[La - 1], m->g[La - 1], m->gather_buf, hx, hy, G->px, nranks, nf);
-    m->launches++;
-    if ((rc = mg_levels(m, nf, mode, nrelax, La - 1, La - 1))) return rc;
-    /* this tile's block of level La-1 plus a one-cell ring (homogeneous dirichlet ghosts evaluated on the fly) */
-    k_extract_patch<<<grid2(hx + 2, hy + 2, b, nf), b, 0, G->stream>>>(m->da.lev[La - 1], m->g[La - 1], m->patch_stage, hx, hy, m->ix * hx, m->iy * hy,
+    k_extract_patch<<<grid2(hx + 2, hy + 2, b, nf), b, 0, G->stream>>>(S->da.lev[La - 1], S->g[La - 1], m->patch_stage, hx, hy, m->ix * hx, m->iy * hy,
                                                                         m->periodic);
     k_load_patch<<<grid2(hx + 2, hy + 2, b, nf), b, 0, G->stream>>>(m->da_patch, m->gpatch, m->patch_stage);
     m->launches += 2;
   }
   CK(cudaGetLastError());
-  /* distributed levels: prolongation, ONE halo exchange, all sweeps on tile + halo */
+  const int chunk0 = nrelax < 7 ? nrelax : 7;
+  auto da_item = [&](int l, int w) { /* da of level l with a halo of w cells */
+    XItem X;
+    for (msqg_model *m : G->tiles) { X.arr.push_back(m->da.lev[l]); X.geo.push_back(m->g[l]); }
+    X.nf = nf; X.w = w; X.ring = 0;
+    return X;
+  };
+  /* distributed levels: prolongation, then the sweeps of the smoother */
   for (int l = La; l <= D; l++) {
     for (msqg_model *m : G->tiles) {
       ProfScope ps(m, PROF_PROLONG, l);
@@ -405,18 +417,28 @@ static int g_cycle_rb(msqg_group *G, const std::vector<MgProblem> &P, int nrelax
       m->launches++;
     }
     CK(cudaGetLastError());
+    if (!G->rb) {
+      /* lexicographic: block Gauss-Seidel, a one-cell halo of da refreshed before the first sweep and after every one */
+      std::vector<XItem> items{da_item(l, 1)};
+      if ((rc = exchange_multi(G, items))) return rc;
+      for (int s = 0; s < nrelax; s++) {
+        for (msqg_model *m : G->tiles)
+          if ((rc = g_relax_level(G, m, l, 1))) return rc;
+        if ((rc = exchange_multi(G, items))) return rc;
+      }
+      continue;
+    }
+    /* red-black: ONE halo exchange, all sweeps on tile + halo */
     int left = nrelax;
     while (left > 0) {
       const int c = left < 7 ? left : 7;       /* sweeps covered by one exchange: 2c + 1 <= 15 cells of halo */
       const int last = (left - c == 0);
       int w = 2 * c + (last ? 1 : 0);          /* one halo cell must survive the last sweep: the prolongation reads it */
-      const Geom &g0 = m0->g[l];
+      const Geom &g0 = S->g[l];
       if (w > g0.nx) w = g0.nx;
       if (w > g0.ny) w = g0.ny;
       if (w < 2 * c) FAIL(MSQG_ERR_ARG, "tiles of level %d are too small for %d fused sweeps (raise agg_n)", l, c);
-      std::vector<XItem> items(1);
-      for (msqg_model *m : G->tiles) { items[0].arr.push_back(m->da.lev[l]); items[0].geo.push_back(m->g[l]); }
-      items[0].nf = nf; items[0].w = w; items[0].ring = 0;
+      std::vector<XItem> items{da_item(l, w)};
       if (l == La && left == nrelax) {
         /* the halo of res on ALL distributed levels (the sweeps recompute up to 2 nrelax border cells of the neighbours)
            rides in the same exchange: one neighbour synchronisation less per cycle */
@@ -424,8 +446,8 @@ static int g_cycle_rb(msqg_group *G, const std::vector<MgProblem> &P, int nrelax
           XItem X;
           for (msqg_model *m : G->tiles) { X.arr.push_back(m->res.lev[l2]); X.geo.push_back(m->g[l2]); }
           X.nf = nf; X.w = 2 * chunk0; X.ring = 0;
-          if (X.w > m0->g[l2].nx) X.w = m0->g[l2].nx;
-          if (X.w > m0->g[l2].ny) X.w = m0->g[l2].ny;
+          if (X.w > S->g[l2].nx) X.w = S->g[l2].nx;
+          if (X.w > S->g[l2].ny) X.w = S->g[l2].ny;
           items.push_back(X);
         }
       }

@@ -75,8 +75,8 @@ struct GraphCache {
 struct msqg_model {
   msqg_params p;
   int N, nl, depth, device;
-  /* tile of a px x py decomposition (single GPU: 1 x 1).  Levels < agg_level exist only on tile (0,0),
-     as full square grids (agglomerated coarse levels); finest tile is tnx x tny cells at (x0, y0). */
+  /* tile of a px x py decomposition (single GPU: 1 x 1).  Levels < agg_level exist only on the tile that solves them
+     for its process (tiles[0] of the group), as full square grids; finest tile is tnx x tny cells at (x0, y0). */
   int px, py, ix, iy, agg_level, tnx, tny, x0, y0;
   bool has_lev[MSQG_MAXLEV + 1];
   int fy[MSQG_MAXLEV + 1];     /* frame rows around the cells of a plane: 1 (the ghost ring) on undecomposed levels,
@@ -96,12 +96,11 @@ struct msqg_model {
   struct msqg_group *group;    /* a periodic model made by msqg_create: the 1 x 1 group that owns this tile (else NULL) */
   int periodic;                /* sbc == -1 (periodic(right); periodic(top), qg.h:842-846): every side of every tile is an
                                   internal side whose halo comes from the opposite tile (or from the tile itself) */
-  int rb_dist;                 /* tile of a red-black group: the levels below agg_level are REPLICATED on every tile */
   Geom gpatch;                 /* level agg_level-1 restricted to this tile (+ halo ring): scatter/gather scratch */
   double *da_patch, *res_patch; /* [nl] planes of gpatch */
-  double *halo_send[4], *halo_recv[4], *patch_stage; /* contiguous exchange buffers */
-  size_t halo_doubles, patch_doubles;
-  double *xsend[9], *xrecv[9]; /* red-black group: one buffer per neighbour direction (dist_rb.cuh), xcap doubles each */
+  double *patch_stage;         /* contiguous gather / scatter block */
+  size_t patch_doubles;
+  double *xsend[9], *xrecv[9]; /* halo exchange: one buffer per neighbour direction (dist_rb.cuh), xcap doubles each */
   size_t xcap;
   /* peer-memory halo exchange (dist_rb.cuh): ONE allocation that neighbours map (CUDA IPC) and write into directly:
      [2 parities][9 directions][xcap] doubles of receive space, then 16 arrival flags, the exchange counter, block
@@ -110,7 +109,7 @@ struct msqg_model {
   size_t xarea_bytes;
   double *peer_area[9];        /* the neighbours' xarea (mapped), by direction; NULL where there is no neighbour */
   void *ipc_opened[9];
-  double *gather_buf;          /* all-gathered blocks of level agg_level-1, [px*py][nl][hy][hx] */
+  double *gather_buf;          /* solver tile: gathered blocks of level agg_level-1, [px*py][nl][hy][hx] */
   cudaStream_t stream;
   bool own_stream;
   Geom g[MSQG_MAXLEV + 1];
@@ -407,13 +406,13 @@ static int coarse_max_level(int nf) {
 }
 
 static int create_model(const msqg_params *p, int device, int px, int py, int ix, int iy, int agg_n, cudaStream_t shared,
-                        msqg_model **out, int rb_dist = 0) {
+                        msqg_model **out, int smoother = 0, bool coarse = true) {
   *out = nullptr;
   if (p->nl < 2 || p->nl > MSQG_NLMAX) FAIL(MSQG_ERR_ARG, "nl must be in [2,%d] (nl==1 is not functional in the reference)", MSQG_NLMAX);
   if (p->N < 8 || (p->N & (p->N - 1))) FAIL(MSQG_ERR_ARG, "N must be a power of two >= 8");
   const int per = p->sbc == -1;
   if (p->sbc < 0 && !per) FAIL(MSQG_ERR_ARG, "sbc is >= 0 (free / partial slip) or -1 (doubly periodic, qg.h:80)");
-  if (per && !rb_dist)
+  if (per && smoother != 1)
     FAIL(MSQG_ERR_ARG, "periodic boundaries (sbc = -1) run on the tile machinery with the red-black smoother: "
                        "msqg_create does that by itself (a 1 x 1 group); tiles: msqg_group_create_local_sm(p, device, px, py, 0, 1, &group)");
   if (per && (p->mode_pv_invert || p->nptr > 0))
@@ -446,7 +445,6 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
   m->agg_level = 0;
   m->periodic = per; m->group = nullptr;
   const bool tiled = px * py > 1 || per;
-  m->rb_dist = tiled ? rb_dist : 0;
   if (per) {
     /* the replicated levels must all be swept by k_coarse_rb, the only kernel of those levels with wrap-around
        neighbours: levels up to 32^2 for nl <= 9, up to 16^2 for nl >= 10; everything above lives on tiles */
@@ -467,7 +465,7 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
            p->N, p->nl, 1 << la, px, py, MSQG_FRAME);
     }
     else if (((1 << la) / px) < 8 || ((1 << la) / py) < 8) why = "tiles must keep >= 8 cells per side on every distributed level (raise agg_n)";
-    else if (rb_dist && (((1 << la) / px) < MSQG_FRAME || ((1 << la) / py) < MSQG_FRAME))
+    else if (smoother == 1 && (((1 << la) / px) < MSQG_FRAME || ((1 << la) / py) < MSQG_FRAME))
       why = "red-black tiles must keep >= 16 cells per side on every distributed level (raise agg_n)";
     else if (la < 2) why = "agg_n too small";
     if (why) { delete m; FAIL(MSQG_ERR_ARG, "%s", why); }
@@ -485,7 +483,7 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
       g.pitch = ((g.nx + MSQG_OX + MSQG_FRAME + 15) / 16) * 16;
     } else {
       g.nx = g.ny = 1 << l; g.bc = 0;
-      m->has_lev[l] = (ix == 0 && iy == 0) || m->rb_dist; /* a red-black group solves the coarse levels redundantly on every tile */
+      m->has_lev[l] = coarse;
       m->fy[l] = 1;
       g.pitch = msqg_pitch(g.nx);
     }
@@ -495,7 +493,6 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
   m->tnx = m->g[depth].nx; m->tny = m->g[depth].ny;
   m->x0 = ix * m->tnx; m->y0 = iy * m->tny;
   m->da_patch = m->res_patch = m->patch_stage = nullptr;
-  for (int k = 0; k < 4; k++) m->halo_send[k] = m->halo_recv[k] = nullptr;
   for (int k = 0; k < 9; k++) m->xsend[k] = m->xrecv[k] = nullptr;
   m->gather_buf = nullptr; m->xcap = 0; m->xarea = nullptr; m->xarea_bytes = 0;
   for (int k = 0; k < 9; k++) { m->peer_area[k] = nullptr; m->ipc_opened[k] = nullptr; }
@@ -526,10 +523,6 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
   int maxnf = p->mode_pv_invert ? nl * nl : nl;
   if (nl * p->nptr > maxnf) maxnf = nl * p->nptr;
   m->stage_doubles = (size_t)maxnf * m->tnx * m->tny;
-  if (m->has_lev[0]) { /* tile (0,0) also stages the agglomerated square levels */
-    const size_t sq0 = m->agg_level > 0 ? (size_t)nl * (1 << (m->agg_level - 1)) * (1 << (m->agg_level - 1)) : 0;
-    if (sq0 > m->stage_doubles) m->stage_doubles = sq0;
-  }
   CK(cudaMalloc(&m->d_stage, m->stage_doubles * sizeof(double)));
   CK(cudaMalloc(&m->d_scal, 64 * sizeof(double)));
   CK(cudaHostAlloc(&m->h_scal, 64 * sizeof(double), cudaHostAllocMapped | cudaHostAllocPortable));
@@ -585,7 +578,7 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
     std::vector<double> one(tc, 1.);
     if ((rc = pack_to(m, m->rd, one.data()))) { msqg_destroy(m); return rc; }
   }
-  if (tiled) { /* exchange / scatter-gather scratch */
+  if (tiled) { /* exchange / gather-scatter scratch */
     const int la = m->agg_level;
     Geom &gp = m->gpatch;
     gp.nx = m->g[la].nx / 2; gp.ny = m->g[la].ny / 2; gp.bc = 15;
@@ -597,24 +590,17 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
     CK(cudaMemsetAsync(m->res_patch, 0, (size_t)nl * gp.plane * sizeof(double), m->stream));
     m->patch_doubles = (size_t)nl * (gp.nx + 2) * (gp.ny + 2);
     CK(cudaMalloc(&m->patch_stage, m->patch_doubles * sizeof(double)));
-    m->halo_doubles = (size_t)nl * ((m->tnx > m->tny ? m->tnx : m->tny) + 2);
-    for (int k = 0; k < 4; k++) {
-      CK(cudaMalloc(&m->halo_send[k], m->halo_doubles * sizeof(double)));
-      CK(cudaMalloc(&m->halo_recv[k], m->halo_doubles * sizeof(double)));
+    /* one exchange carries at most: MSQG_FRAME-wide halos of one list on every distributed level (sizes halve per level) */
+    m->xcap = (size_t)nl * MSQG_FRAME * 2 * ((m->tnx > m->tny ? m->tnx : m->tny) + 2 * MSQG_FRAME);
+    for (int k = 0; k < 9; k++) {
+      if (k == 4) continue;
+      CK(cudaMalloc(&m->xsend[k], m->xcap * sizeof(double)));
+      CK(cudaMalloc(&m->xrecv[k], m->xcap * sizeof(double)));
     }
-    if (m->rb_dist) {
-      /* one exchange carries at most: MSQG_FRAME-wide halos of one list on every distributed level (sizes halve per level) */
-      m->xcap = (size_t)nl * MSQG_FRAME * 2 * ((m->tnx > m->tny ? m->tnx : m->tny) + 2 * MSQG_FRAME);
-      for (int k = 0; k < 9; k++) {
-        if (k == 4) continue;
-        CK(cudaMalloc(&m->xsend[k], m->xcap * sizeof(double)));
-        CK(cudaMalloc(&m->xrecv[k], m->xcap * sizeof(double)));
-      }
-      CK(cudaMalloc(&m->gather_buf, (size_t)px * py * nl * gp.nx * gp.ny * sizeof(double)));
-      m->xarea_bytes = (2 * 9 * m->xcap) * sizeof(double) + 4096;
-      CK(cudaMalloc(&m->xarea, m->xarea_bytes));
-      CK(cudaMemsetAsync(m->xarea, 0, m->xarea_bytes, m->stream));
-    }
+    if (coarse) CK(cudaMalloc(&m->gather_buf, (size_t)px * py * nl * gp.nx * gp.ny * sizeof(double)));
+    m->xarea_bytes = (2 * 9 * m->xcap) * sizeof(double) + 4096;
+    CK(cudaMalloc(&m->xarea, m->xarea_bytes));
+    CK(cudaMemsetAsync(m->xarea, 0, m->xarea_bytes, m->stream));
   }
   CK(cudaStreamSynchronize(m->stream));
   *out = m;
@@ -669,7 +655,6 @@ extern "C" void msqg_destroy(msqg_model *m) {
   if (m->da_patch) cudaFree(m->da_patch);
   if (m->res_patch) cudaFree(m->res_patch);
   if (m->patch_stage) cudaFree(m->patch_stage);
-  for (int k = 0; k < 4; k++) { if (m->halo_send[k]) cudaFree(m->halo_send[k]); if (m->halo_recv[k]) cudaFree(m->halo_recv[k]); }
   for (int k = 0; k < 9; k++) { if (m->xsend[k]) cudaFree(m->xsend[k]); if (m->xrecv[k]) cudaFree(m->xrecv[k]); }
   if (m->gather_buf) cudaFree(m->gather_buf);
   for (int k = 0; k < 9; k++) if (m->ipc_opened[k]) cudaIpcCloseMemHandle(m->ipc_opened[k]);

@@ -1,12 +1,13 @@
 """2-D domain decomposition of the msqg timestep (include/msqg.h layer 1b).
 
 smoother="rb" (throughput mode): red-black sweeps are decomposition independent, so the group reproduces the
-single-GPU red-black result bit for bit on any px x py; levels below `agg_n` are replicated on every GPU
-(all-gather + redundant coarse solve) and each distributed level needs one deep-halo exchange per cycle.
-smoother="lex" is the first-round decomposition of the reference-order sweep (block Gauss-Seidel, rank-0 coarse levels).
+single-GPU red-black result bit for bit on any px x py; each distributed level needs one deep-halo exchange per cycle.
+smoother="lex": the reference-order sweep decomposed (block Gauss-Seidel).
 
 `Group(params, px, py, agg_n)` is the reference built with -D_MPI=1: px x py tiles, halo exchange
-after every relaxation sweep, coarse levels below `agg_n` agglomerated on tile (0,0).
+after every relaxation sweep.  Both smoothers share the halo exchange (peer memory unless MSQG_P2P=0) and the coarse
+levels: those below `agg_n` are gathered onto one tile per process and solved there (under NCCL every GPU solves them
+from an all-gather, nothing is scattered back).
 
   * backend "local": all tiles in this process on one GPU (tests; emulates N ranks on one device)
   * backend "nccl" : one tile per process / GPU; torch.distributed only carries the 128-byte NCCL

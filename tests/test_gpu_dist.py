@@ -1,5 +1,5 @@
 """Domain decomposition (reference -D_MPI=1 semantics) on ONE GPU with the local exchange back-end:
-all tiles in one process, halo exchange by device copies.  Checked bit for bit against the oracle's
+all tiles in one process, halo exchange by direct stores or device copies.  Checked bit for bit against the oracle's
 emulation of the MPI block decomposition (orc_set_decomp)."""
 import numpy as np
 import pytest
@@ -24,11 +24,16 @@ def _pair(N, nl, px, py, agg_n, gpu):
     return mo, g, psi
 
 
-@pytest.mark.parametrize("N,nl,px,py,agg_n", [(128, 2, 2, 1, 32), (128, 3, 2, 2, 32), (256, 2, 4, 2, 64), (128, 4, 1, 2, 64)])
-def test_decomposed_invertq_and_steps(gpu, N, nl, px, py, agg_n):
+@pytest.mark.parametrize("p2p", [1, 0])
+@pytest.mark.parametrize("N,nl,px,py,agg_n", [(128, 2, 2, 1, 32), (128, 3, 2, 2, 32), (256, 2, 4, 2, 64), (128, 4, 1, 2, 64),
+                                              (128, 2, 4, 2, 32),    # 8-cell wide tiles on the first distributed level
+                                              (512, 3, 4, 2, 128)])  # larger tiles with inner columns on 4 x 2
+def test_decomposed_invertq_and_steps(gpu, N, nl, px, py, agg_n, p2p, monkeypatch):
     from oracle import oracle as O
     from msom_b200 import capi as G
+    monkeypatch.setenv("MSQG_P2P", str(p2p))   # halo transport: stores into the neighbours' receive areas / staged copies
     mo, g, psi = _pair(N, nl, px, py, agg_n, gpu)
+    assert g.transport == ("peer-memory" if p2p else "nccl")
     assert np.array_equal(g.get_global(G.Q), mo.get(O.Q))
     z = np.zeros_like(psi)
     mo.set(O.PSI, z); g.set_global(G.PSI, z)
