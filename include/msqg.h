@@ -233,6 +233,13 @@ int msqg_test_residual(msqg_model *m, const double *a, const double *b, double *
  * out receives res on levels D, D-1, .., *bottom one after another, each [nf][2^l][2^l] (at most 4/3 of level D) */
 int msqg_test_residual_levels(msqg_model *m, int mode, const double *a, const double *b, double *out, double *maxres,
                               int *bottom);
+/* ncycles multigrid cycles of the production solve loop with a fixed sweep schedule: cycle k relaxes nrelax[k] times
+ * per level, no tolerance stop and no nrelax adaptation; resa[k] receives the residual max norm after cycle k.  mode = -1
+ * the layer-coupled problem PSI <- Q, mode = l (mode_pv_invert) plane l of PM <- QM; the unknown is updated in place
+ * (msqg_get_field).  Red-black cycles go through the same CUDA graphs as msqg_invertq (MSQG_GRAPH), so a repeated
+ * nrelax runs eagerly, is recorded, then replayed.  A periodic handle runs its group.  MSQG_ERR_ARG for an nrelax
+ * outside 2..100 (the range mg_solve can reach) or a bad mode. */
+int msqg_test_cycles(msqg_model *m, int mode, const int *nrelax, int ncycles, double *resa);
 int msqg_test_restrict(msqg_model *m, int level, const double *fine, double *coarse);
 int msqg_test_prolong(msqg_model *m, int level, const double *coarse, double *fine);
 /* div_by() (exact division by a pivot with known reciprocal) next to IEEE x/d */
@@ -306,6 +313,8 @@ int msqg_group_get_field(msqg_group *g, int t, int id, double *host_tile);
 int msqg_group_set_const(msqg_group *g);
 int msqg_group_invertq(msqg_group *g, int q_id);
 int msqg_group_step(msqg_group *g, double t, double tnext, double *dt_out, double *tnext_out);
+/* msqg_test_cycles on the decomposed grid (every tile's PSI <- Q, or plane `mode` of PM <- QM) */
+int msqg_group_test_cycles(msqg_group *g, int mode, const int *nrelax, int ncycles, double *resa);
 int msqg_group_last_mgstats(msqg_group *g, msqg_mgstats *out);
 /* as msqg_last_mgstats: mode < 0 the last solve, else the solve of that vertical mode (mode_pv_invert) */
 int msqg_group_last_mode_mgstats(msqg_group *g, int mode, msqg_mgstats *out);

@@ -133,6 +133,7 @@ def lib():
     L.msqg_test_relax_scalar.argtypes = [vp, C.c_int, C.c_double, dp, dp, C.c_int]
     L.msqg_test_residual.argtypes = [vp, dp, dp, dp, pd]
     L.msqg_test_residual_levels.argtypes = [vp, C.c_int, dp, dp, dp, pd, C.POINTER(C.c_int)]
+    L.msqg_test_cycles.argtypes = [vp, C.c_int, np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS"), C.c_int, dp]
     L.msqg_test_restrict.argtypes = [vp, C.c_int, dp, dp]
     L.msqg_test_prolong.argtypes = [vp, C.c_int, dp, dp]
     L.msqg_test_div.argtypes = [C.c_int, dp, dp, dp, dp, C.c_int]
@@ -252,6 +253,14 @@ class Model:
         s = MgStats()
         check(self.L.msqg_last_mgstats(self.h, mode, C.byref(s)))
         return s
+
+    def test_cycles(self, nrelax, mode=-1):
+        """len(nrelax) multigrid cycles, cycle k with nrelax[k] sweeps per level (msqg_test_cycles): the unknown (PSI, or
+        plane `mode` of PM) is updated in place; returns the residual max norm after every cycle"""
+        sched = np.ascontiguousarray(nrelax, dtype=np.int32)
+        resa = np.zeros(len(sched))
+        check(self.L.msqg_test_cycles(self.h, mode, sched, len(sched), resa))
+        return resa
 
     def update(self, dtmax, q_id=Q):
         out = C.c_double()

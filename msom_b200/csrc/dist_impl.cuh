@@ -371,8 +371,10 @@ static int g_check_err(msqg_group *G) {
 
 #include "dist_rb.cuh"
 
-/* mg_solve on the decomposed grid: problem P[t] on tile t (NITERMIN 1, NITERMAX 100, nrelax starts at 4) */
-static int g_solve(msqg_group *G, const std::vector<MgProblem> &P, msqg_mgstats *st) {
+/* mg_solve on the decomposed grid: problem P[t] on tile t (NITERMIN 1, NITERMAX 100, nrelax starts at 4); sched as
+ * mg_solve's */
+static int g_solve(msqg_group *G, const std::vector<MgProblem> &P, msqg_mgstats *st, const int *sched = nullptr,
+                   int ncycles = 0, double *resa_out = nullptr) {
   int rc;
   msqg_mgstats s;
   memset(&s, 0, sizeof(s));
@@ -380,7 +382,8 @@ static int g_solve(msqg_group *G, const std::vector<MgProblem> &P, msqg_mgstats 
   double resb;
   if ((rc = g_residual(G, P, &resb))) return rc;
   s.resb = s.resa = resb;
-  for (s.i = 0; s.i < 100 && (s.i < 1 || s.resa > 1e-3); s.i++) {
+  for (s.i = 0; sched ? s.i < ncycles : s.i < 100 && (s.i < 1 || s.resa > 1e-3); s.i++) {
+    if (sched) s.nrelax = sched[s.i];
     /* one cycle + residual + its all-reduce: with the red-black smoother a single graph launch (keyed by nrelax, the
        mode, the unknown and the right-hand side of tile 0 and the current da buffers of every tile) */
     msqg_model *m0 = G->tiles[0];
@@ -396,7 +399,8 @@ static int g_solve(msqg_group *G, const std::vector<MgProblem> &P, msqg_mgstats 
     });
     if (rc) return rc;
     if ((rc = reduce_max_finish(G, 1, &s.resa))) return rc;
-    if (s.resa > 1e-3) {
+    if (sched) resa_out[s.i] = s.resa;
+    else if (s.resa > 1e-3) {
       if (resb / s.resa < 1.2 && s.nrelax < 100) s.nrelax++;
       else if (resb / s.resa > 10 && s.nrelax > 2) s.nrelax--;
     }
@@ -456,6 +460,18 @@ static int g_invertq(msqg_group *G, int q_id) {
 extern "C" int msqg_group_invertq(msqg_group *G, int q_id) {
   CK(cudaSetDevice(G->device));
   return g_invertq(G, q_id);
+}
+extern "C" int msqg_group_test_cycles(msqg_group *G, int mode, const int *nrelax, int ncycles, double *resa) {
+  CK(cudaSetDevice(G->device));
+  int rc = check_cycle_schedule(G->p.nl, G->p.mode_pv_invert, mode, nrelax, ncycles, resa);
+  if (rc) return rc;
+  for (msqg_model *m : G->tiles) {
+    if (!m->const_set) FAIL(MSQG_ERR_ARG, "set_const must be called before the cycles");
+    if (mode < 0 && !m->s_uniform) FAIL(MSQG_ERR_ARG, "horizontally varying stretching is not supported by the relax kernel yet");
+  }
+  if ((rc = exchange_list(G, mode < 0 ? MSQG_PSI : MSQG_PM, G->tiles[0]->depth))) return rc; /* the start's ring, as g_invertq */
+  msqg_mgstats st;
+  return g_solve(G, g_problem(G, mode, MSQG_Q), &st, nrelax, ncycles, resa);
 }
 
 /* ------------------------------------------------------------------ fields, set_const */

@@ -1485,8 +1485,11 @@ static int mg_cycle(msqg_model *m, const MgProblem &P, int nrelax) {
   return MSQG_OK;
 }
 
-/* mg_solve, mspg/elliptic.h:145-229: NITERMIN=1, NITERMAX=100, nrelax starts at 4 */
-static int mg_solve(msqg_model *m, const MgProblem &P, double tolerance, msqg_mgstats *st) {
+/* mg_solve, mspg/elliptic.h:145-229: NITERMIN=1, NITERMAX=100, nrelax starts at 4.  sched != NULL (msqg_test_cycles):
+ * exactly ncycles cycles, cycle k with sched[k] sweeps per level, no tolerance stop and no adaptation; resa_out[k] is the
+ * residual after cycle k */
+static int mg_solve(msqg_model *m, const MgProblem &P, double tolerance, msqg_mgstats *st, const int *sched = nullptr,
+                    int ncycles = 0, double *resa_out = nullptr) {
   msqg_mgstats s;
   memset(&s, 0, sizeof(s));
   s.nrelax = 4;
@@ -1496,7 +1499,8 @@ static int mg_solve(msqg_model *m, const MgProblem &P, double tolerance, msqg_mg
   s.resb = s.resa = resb;
   const bool graphed = m->smoother == 1 && m->use_graphs && !m->prof_on; /* coefficient tables are fixed between set_const calls */
   std::vector<msqg_model *> self(1, m);
-  for (s.i = 0; s.i < 100 && (s.i < 1 || s.resa > tolerance); s.i++) {
+  for (s.i = 0; sched ? s.i < ncycles : s.i < 100 && (s.i < 1 || s.resa > tolerance); s.i++) {
+    if (sched) s.nrelax = sched[s.i];
     /* one cycle + the residual that follows it: a single graph launch in red-black mode */
     GraphKey key(s.nrelax, P.mode, (const void *)P.a, (const void *)P.b, da_parity_mask(m));
     rc = run_graphed(m->stream, m->graphs, key, self, nullptr, graphed, [&]() -> int {
@@ -1507,7 +1511,8 @@ static int mg_solve(msqg_model *m, const MgProblem &P, double tolerance, msqg_mg
     if (rc) return rc;
     CK(cudaStreamSynchronize(m->stream));
     s.resa = m->h_scal[0];
-    if (s.resa > tolerance) {
+    if (sched) resa_out[s.i] = s.resa;
+    else if (s.resa > tolerance) {
       if (resb / s.resa < 1.2 && s.nrelax < 100) s.nrelax++;
       else if (resb / s.resa > 10 && s.nrelax > 2) s.nrelax--;
     }
@@ -2494,6 +2499,28 @@ extern "C" int msqg_test_prolong(msqg_model *m, int level, const double *coarse,
   launch_prolong(m->stream, m->nl, m->da.lev[level - 1], m->da.lev[level], m->g[level - 1], m->g[level]);
   CK(cudaGetLastError());
   return download_level(m, fine, m->da.lev[level], m->nl, level);
+}
+
+/* arguments of msqg_test_cycles / msqg_group_test_cycles: nrelax in 2..100, the range mg_solve can produce */
+static int check_cycle_schedule(int nl, int mode_pv_invert, int mode, const int *nrelax, int ncycles, const double *resa) {
+  if (mode < -1 || mode >= nl || (mode >= 0 && !mode_pv_invert)) FAIL(MSQG_ERR_ARG, "mode %d needs mode_pv_invert and mode < nl", mode);
+  if (ncycles < 1 || !nrelax || !resa) FAIL(MSQG_ERR_ARG, "a schedule of ncycles >= 1 sweep counts and a resa buffer");
+  for (int k = 0; k < ncycles; k++)
+    if (nrelax[k] < 2 || nrelax[k] > 100) FAIL(MSQG_ERR_ARG, "nrelax[%d] = %d is outside 2..100", k, nrelax[k]);
+  return MSQG_OK;
+}
+extern "C" int msqg_test_cycles(msqg_model *m, int mode, const int *nrelax, int ncycles, double *resa) {
+  CK(cudaSetDevice(m->device));
+  int rc = check_cycle_schedule(m->nl, m->p.mode_pv_invert, mode, nrelax, ncycles, resa);
+  if (rc) return rc;
+  if (m->group) return msqg_group_test_cycles(m->group, mode, nrelax, ncycles, resa);
+  if (!m->const_set) FAIL(MSQG_ERR_ARG, "set_const must be called before the cycles");
+  const int D = m->depth;
+  const size_t pl = m->g[D].plane;
+  MgProblem P = mode < 0 ? MgProblem{m->nl, -1, m->psi.lev[D], m->q.lev[D]}
+                         : MgProblem{1, mode, m->pm.lev[D] + (size_t)mode * pl, m->qm.lev[D] + (size_t)mode * pl};
+  msqg_mgstats st;
+  return mg_solve(m, P, 1e-3, &st, nrelax, ncycles, resa);
 }
 
 /* exact-division self test: out[i] = div_by(x[i], d[i], 1/d[i]) next to x[i]/d[i] */

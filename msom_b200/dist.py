@@ -48,6 +48,7 @@ def _bind():
     L.msqg_group_set_const.argtypes = [vp]
     L.msqg_group_invertq.argtypes = [vp, C.c_int]
     L.msqg_group_step.argtypes = [vp, C.c_double, C.c_double, pd, pd]
+    L.msqg_group_test_cycles.argtypes = [vp, C.c_int, np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS"), C.c_int, dp]
     L.msqg_group_last_mgstats.argtypes = [vp, C.POINTER(G.MgStats)]
     L.msqg_group_last_mode_mgstats.argtypes = [vp, C.c_int, C.POINTER(G.MgStats)]
     for f in ("msqg_group_total_cycles", "msqg_group_exchanges", "msqg_group_launches"):
@@ -162,6 +163,13 @@ class Group:
 
     def invertq(self, q_id=G.Q):
         G.check(self.L.msqg_group_invertq(self.h, q_id))
+
+    def test_cycles(self, nrelax, mode=-1):
+        """G.Model.test_cycles on the decomposed grid (msqg_group_test_cycles)"""
+        sched = np.ascontiguousarray(nrelax, dtype=np.int32)
+        resa = np.zeros(len(sched))
+        G.check(self.L.msqg_group_test_cycles(self.h, mode, sched, len(sched), resa))
+        return resa
 
     def mgstats(self, mode=-1):
         """statistics of the last solve (mode < 0), or of vertical mode `mode` of the last modal inversion"""

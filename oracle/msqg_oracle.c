@@ -831,7 +831,9 @@ static void mg_cycle(mgctx *c, flist *a, flist *res, flist *da, flist *old, int 
   boundary(a);
 }
 
-static orc_mgstats mg_solve(mgctx *c, flist *a, flist *b, double tolerance) {
+/* sched != NULL: exactly ncycles cycles, cycle k with sched[k] sweeps per level, no tolerance stop and no adaptation;
+ * resa_out[k] is the residual after cycle k */
+static orc_mgstats mg_solve(mgctx *c, flist *a, flist *b, double tolerance, const int *sched, int ncycles, double *resa_out) {
   orc_model *m = c->m;
   int D = m->depth, n = m->N;
   flist da = fl_new(a->nf, a->bc, D);   /* homogeneous version of a's BC: same */
@@ -847,10 +849,12 @@ static orc_mgstats mg_solve(mgctx *c, flist *a, flist *b, double tolerance) {
   s.nrelax = 4;
   double resb;
   resb = s.resb = s.resa = mg_residual(c, a, b, &res);
-  for (s.i = 0; s.i < 100 && (s.i < 1 || s.resa > tolerance); s.i++) {
+  for (s.i = 0; sched ? s.i < ncycles : s.i < 100 && (s.i < 1 || s.resa > tolerance); s.i++) {
+    if (sched) s.nrelax = sched[s.i];
     mg_cycle(c, a, &res, &da, &old, s.nrelax, 1, D);
     s.resa = mg_residual(c, a, b, &res);
-    if (s.resa > tolerance) {
+    if (sched) resa_out[s.i] = s.resa;
+    else if (s.resa > tolerance) {
       if (resb / s.resa < 1.2 && s.nrelax < 100) s.nrelax++;
       else if (resb / s.resa > 10 && s.nrelax > 2) s.nrelax--;
     }
@@ -884,7 +888,7 @@ static void invertq(orc_model *m, flist *pl, flist *ql) {
       flist lam = m->iBul; lam.nf = 1; lam.d = m->iBul.d + l * (D + 1);
       restriction(&lam);
       c.scalar_mode = 1; c.mode = l;
-      m->mgmode[l] = m->mgpsi = mg_solve(&c, &pm, &qm, 1e-3);
+      m->mgmode[l] = m->mgpsi = mg_solve(&c, &pm, &qm, 1e-3, NULL, 0, NULL);
     }
     for (int i = 0; i < n; i++)
       for (int j = 0; j < n; j++) {
@@ -898,11 +902,31 @@ static void invertq(orc_model *m, flist *pl, flist *ql) {
   } else {
     /* poisson_layer, poisson_layer.h:263-306: restriction(strl) every call */
     restriction(&m->strl);
-    m->mgpsi = mg_solve(&c, pl, ql, 1e-3);
+    m->mgpsi = mg_solve(&c, pl, ql, 1e-3, NULL, 0, NULL);
   }
   boundary(pl);
 }
 void orc_invertq(orc_model *m) { invertq(m, &m->pol, &m->qol); }
+int orc_test_cycles(orc_model *m, int mode, const int *nrelax, int ncycles, double *resa) {
+  if (mode < -1 || mode >= m->nl || (mode >= 0 && !m->p.mode_pv_invert) || ncycles < 1 || !nrelax || !resa) return -1;
+  for (int k = 0; k < ncycles; k++)
+    if (nrelax[k] < 2 || nrelax[k] > 100) return -1;
+  mgctx c; c.m = m; c.scalar_mode = 0; c.mode = 0;
+  if (mode < 0) {
+    restriction(&m->strl); /* as invertq */
+    mg_solve(&c, &m->pol, &m->qol, 1e-3, nrelax, ncycles, resa);
+    boundary(&m->pol);
+    return 0;
+  }
+  const int D = m->depth;
+  flist pm = m->pom, qm = m->qom, lam = m->iBul; /* views on plane `mode` */
+  pm.nf = qm.nf = lam.nf = 1;
+  pm.d = m->pom.d + mode * (D + 1); qm.d = m->qom.d + mode * (D + 1); lam.d = m->iBul.d + mode * (D + 1);
+  restriction(&lam);
+  c.scalar_mode = 1; c.mode = mode;
+  mg_solve(&c, &pm, &qm, 1e-3, nrelax, ncycles, resa);
+  return 0;
+}
 orc_mgstats orc_last_mgstats(orc_model *m, int mode) { return mode < 0 ? m->mgpsi : m->mgmode[mode]; }
 int orc_total_cycles(orc_model *m) { return m->total_cycles; }
 

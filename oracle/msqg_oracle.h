@@ -99,6 +99,11 @@ void orc_invertq(orc_model *m);                  /* invertq(pol,qol) */
 void orc_comp_q(orc_model *m);                   /* comp_q(pol,qol) */
 orc_mgstats orc_last_mgstats(orc_model *m, int mode);
 int  orc_total_cycles(orc_model *m);
+/* ncycles multigrid cycles with a fixed sweep schedule: cycle k relaxes nrelax[k] times per level, no tolerance stop and
+   no nrelax adaptation; resa[k] is the residual max norm after cycle k.  mode = -1: the layer-coupled problem, PSI <- Q
+   (the stretching restricted first, as invertq); mode = l (mode_pv_invert): plane l of PM <- QM (lambda restricted
+   first).  The unknown is updated in place.  Returns -1 for a bad mode or an nrelax outside 2..100. */
+int  orc_test_cycles(orc_model *m, int mode, const int *nrelax, int ncycles, double *resa);
 
 /* update_qg on the model's q (evolving) -> DQ; returns dtmax */
 double orc_update(orc_model *m, double dtmax);

@@ -101,6 +101,8 @@ def lib(omp=False):
     L.orc_last_mgstats.restype = MgStats
     L.orc_total_cycles.argtypes = [vp]
     L.orc_total_cycles.restype = C.c_int
+    L.orc_test_cycles.argtypes = [vp, C.c_int, np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS"), C.c_int, dp]
+    L.orc_test_cycles.restype = C.c_int
     L.orc_update.argtypes = [vp, C.c_double]
     L.orc_update.restype = C.c_double
     L.orc_step.argtypes = [vp]
@@ -223,6 +225,15 @@ class Model:
 
     def mgstats(self, mode=-1):
         return self.L.orc_last_mgstats(self.h, mode)
+
+    def test_cycles(self, nrelax, mode=-1):
+        """len(nrelax) multigrid cycles, cycle k with nrelax[k] sweeps per level (orc_test_cycles): the unknown (PSI, or
+        plane `mode` of PM) is updated in place; returns the residual max norm after every cycle"""
+        sched = np.ascontiguousarray(nrelax, dtype=np.int32)
+        resa = np.zeros(len(sched))
+        if self.L.orc_test_cycles(self.h, mode, sched, len(sched), resa):
+            raise ValueError("orc_test_cycles refused mode %d / schedule %s" % (mode, list(sched)))
+        return resa
 
     def update(self, dtmax):
         return self.L.orc_update(self.h, dtmax)

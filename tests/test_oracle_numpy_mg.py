@@ -38,8 +38,10 @@ def residual(a, b, s, idh0, idh1, D, bc=-1):
     return r, float(np.abs(r).max())
 
 
-def numpy_solve(a, b, s_fine, dh, L0, tol=1e-3, bc=-1):
-    """bc = -1: closed basin (dirichlet(0)); bc = 0: doubly periodic (sbc = -1, qg.h:842-846)"""
+def numpy_solve(a, b, s_fine, dh, L0, tol=1e-3, bc=-1, schedule=None):
+    """bc = -1: closed basin (dirichlet(0)); bc = 0: doubly periodic (sbc = -1, qg.h:842-846).
+    schedule: exactly len(schedule) cycles, cycle k with schedule[k] sweeps per level, no tolerance stop and no nrelax
+    adaptation (orc_test_cycles).  stats["resas"] holds the residual after every cycle."""
     nl, N = a.shape[0], a.shape[1]
     depth = int(np.log2(N))
     dhc = 0.5 * (dh[:-1] + dh[1:])
@@ -51,8 +53,10 @@ def numpy_solve(a, b, s_fine, dh, L0, tol=1e-3, bc=-1):
     a = a.copy()
     hist = []
     res, resb = residual(a, b, s_fine, idh0, idh1, L0 / N, bc)
-    stats = dict(resb=resb, resa=resb, nrelax=4, i=0)
-    while stats["i"] < 100 and (stats["i"] < 1 or stats["resa"] > tol):
+    stats = dict(resb=resb, resa=resb, nrelax=4, i=0, resas=[])
+    while (stats["i"] < len(schedule)) if schedule is not None else (stats["i"] < 100 and (stats["i"] < 1 or stats["resa"] > tol)):
+        if schedule is not None:
+            stats["nrelax"] = schedule[stats["i"]]
         # mg_cycle with minlevel = 1
         r_lev = {depth: res}
         for l in range(depth - 1, 0, -1):
@@ -66,7 +70,8 @@ def numpy_solve(a, b, s_fine, dh, L0, tol=1e-3, bc=-1):
         hist.append(stats["nrelax"])
         res, resa = residual(a, b, s_fine, idh0, idh1, L0 / N, bc)
         stats["resa"] = resa
-        if resa > tol:
+        stats["resas"].append(resa)
+        if schedule is None and resa > tol:
             if resb / resa < 1.2 and stats["nrelax"] < 100:
                 stats["nrelax"] += 1
             elif resb / resa > 10 and stats["nrelax"] > 2:
