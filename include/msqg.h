@@ -155,6 +155,11 @@ int msqg_get_smoother(msqg_model *m);
  * other compile-time switch of qg.h, _LS_RV = 0, needs no entry point: it is the arithmetic of flsrv = 0. */
 int msqg_set_energy_conserv(msqg_model *m, int on);
 int msqg_get_energy_conserv(msqg_model *m);
+/* How the layer-coupled relaxation reads the stretching strl = (Fr/Ro)^2 (valid after set_const): 0 per-level constants
+ * (uniform), 1 per-row coefficient tables (it varies with y only: varRo > 0), 2 per-cell tables (it varies with x too:
+ * a Fr(x, y) field).  On a tile of a group (and a periodic model) this is the group's decision over the whole field.
+ * MSQG_ERR_ARG before set_const. */
+int msqg_stretch_tables(msqg_model *m);
 /* reset_layer_var (layer.h:37-41): zero the interior, ghost ring untouched */
 int msqg_reset_field(msqg_model *m, int id);
 /* layer thicknesses dhf (qg.h:895-896; overridden by dh_%dl.bin, qg.h:940-948) */
@@ -296,7 +301,11 @@ int msqg_group_create_nccl(const msqg_params *p, int device, int px, int py, int
  * window of the undecomposed noise field (Philox: global counter; libc: every tile replays the whole N^2 nl rand() stream,
  * O(N^2 nl) host time per draw and tile).  Seed every tile alike (msqg_seed_noise / msqg_set_noise_mode on each
  * msqg_group_tile, on every rank under NCCL): msqg_group_step refuses tiles that disagree on noise mode, seed or draw
- * count (MSQG_ERR_ARG).  Refused with MSQG_ERR_ARG: modal inversion on a lexicographic or periodic group. */
+ * count (MSQG_ERR_ARG).  Horizontally varying stretching (varRo > 0, a Fr(x, y) field through MSQG_FR) runs on red-black
+ * groups, periodic ones included, at nl <= 6 with the bits of the undecomposed red-black model: msqg_group_set_const
+ * decides constants / per-row / per-cell tables for the whole group (msqg_stretch_tables of any tile reports it).
+ * Refused with MSQG_ERR_ARG: modal inversion on a lexicographic or periodic group; varying stretching on a lexicographic
+ * group or at nl >= 7 (at the first invertq). */
 int msqg_group_create_local_sm(const msqg_params *p, int device, int px, int py, int agg_n, int smoother, msqg_group **out);
 int msqg_group_create_nccl_sm(const msqg_params *p, int device, int px, int py, int agg_n, int smoother, int rank, int nranks,
                               const void *uid128, msqg_group **out);

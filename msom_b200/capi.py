@@ -109,6 +109,7 @@ def lib():
     L.msqg_get_field_async.argtypes = [vp, C.c_int, dp]
     L.msqg_io_wait.argtypes = [vp]
     L.msqg_get_energy_conserv.argtypes = [vp]
+    L.msqg_stretch_tables.argtypes = [vp]
     L.msqg_set_keep_dq.argtypes = [vp, C.c_int]
     L.msqg_set_dissipation.argtypes = [vp, C.c_double, C.c_double, C.c_double, C.c_double]
     L.msqg_set_const.argtypes = [vp]
@@ -313,6 +314,16 @@ class Model:
         ms = (C.c_double * 9)(); cnt = (C.c_long * 9)(); aux = (C.c_long * 9)()
         check(self.L.msqg_profile_read(self.h, ms, cnt, aux))
         return {k: dict(ms=ms[i], count=cnt[i], aux=aux[i]) for i, k in enumerate(self.PROF_CATS)}
+
+    STRETCHING = ("uniform", "rows", "cells")
+
+    @property
+    def stretching(self):
+        """how the relaxation reads the stretching (after set_const): "uniform" (per-level constants), "rows" (per-row
+        tables: it varies with y only, varRo > 0) or "cells" (per-cell tables: a Fr(x, y) field)"""
+        rc = self.L.msqg_stretch_tables(self.h)
+        check(min(rc, 0))
+        return self.STRETCHING[rc]
 
     @property
     def total_cycles(self):

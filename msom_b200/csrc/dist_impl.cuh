@@ -91,6 +91,17 @@ __global__ void k_load_patch(double *__restrict__ dst, Geom gp, const double *__
   dst[(size_t)f * gp.plane + GIDX(gp.pitch, y, x)] = src[((size_t)f * (gp.ny + 2) + y + 1) * (gp.nx + 2) + x + 1];
 }
 
+/* does the stretching (planes 0 .. nf-1) vary over the cells [x0, x1) x [y0, y1) of a level?  flags[0] = 1: it is not
+ * one value per plane; flags[1] = 1: it varies along x (a row holds more than one value) */
+__global__ void k_stretch_varies(const double *__restrict__ s, Geom g, int x0, int x1, int y0, int y1, double *flags) {
+  const int x = x0 + blockIdx.x * blockDim.x + threadIdx.x, y = y0 + blockIdx.y * blockDim.y + threadIdx.y, f = blockIdx.z;
+  if (x >= x1 || y >= y1) return;
+  const double *p = s + (size_t)f * g.plane;
+  const double v = p[GIDX(g.pitch, y, x)];
+  if (v != p[GIDX(g.pitch, y0, x0)]) flags[0] = 1.;
+  if (v != p[GIDX(g.pitch, y, x0)]) flags[1] = 1.;
+}
+
 /* ------------------------------------------------------------------ the group */
 struct msqg_group {
   msqg_params p;
@@ -413,15 +424,15 @@ static int g_solve(msqg_group *G, const std::vector<MgProblem> &P, msqg_mgstats 
   return MSQG_OK;
 }
 
+static int g_check_stretching(msqg_group *G);
 /* poisson_layer + invertq on the decomposed grid (invertq_list's order) */
 static int g_invertq(msqg_group *G, int q_id) {
-  for (msqg_model *m : G->tiles) {
+  for (msqg_model *m : G->tiles)
     if (!m->const_set) FAIL(MSQG_ERR_ARG, "set_const must be called before invertq");
-    if (!m->s_uniform) FAIL(MSQG_ERR_ARG, "horizontally varying stretching is not supported by the relax kernel yet");
-  }
   const int D = G->tiles[0]->depth;
   int rc;
   if (!G->p.mode_pv_invert) {
+    if ((rc = g_check_stretching(G))) return rc;
     if ((rc = exchange_list(G, MSQG_PSI, D))) return rc; /* the warm start's ring */
     return g_solve(G, g_problem(G, -1, q_id), &G->mgpsi);
   }
@@ -465,10 +476,9 @@ extern "C" int msqg_group_test_cycles(msqg_group *G, int mode, const int *nrelax
   CK(cudaSetDevice(G->device));
   int rc = check_cycle_schedule(G->p.nl, G->p.mode_pv_invert, mode, nrelax, ncycles, resa);
   if (rc) return rc;
-  for (msqg_model *m : G->tiles) {
+  for (msqg_model *m : G->tiles)
     if (!m->const_set) FAIL(MSQG_ERR_ARG, "set_const must be called before the cycles");
-    if (mode < 0 && !m->s_uniform) FAIL(MSQG_ERR_ARG, "horizontally varying stretching is not supported by the relax kernel yet");
-  }
+  if (mode < 0 && (rc = g_check_stretching(G))) return rc;
   if ((rc = exchange_list(G, mode < 0 ? MSQG_PSI : MSQG_PM, G->tiles[0]->depth))) return rc; /* the start's ring, as g_invertq */
   msqg_mgstats st;
   return g_solve(G, g_problem(G, mode, MSQG_Q), &st, nrelax, ncycles, resa);
@@ -510,14 +520,88 @@ static int g_check_modes_agree(msqg_group *G) {
                          "everywhere (uniform vertical modes)", k / 4);
   return MSQG_OK;
 }
+/* One stretching path for the whole group: constants, per-row tables or per-cell tables, decided as the undecomposed
+ * model decides it over the whole field.  Each tile only knows its own cells, and a field that is constant on every
+ * tile but differs between tiles must not pass for uniform.  So the stretching of every distributed level gets the
+ * halo the sweeps of one exchange reach (g_cycle: 2 * 7 + 1 cells), each tile tests its own cells plus that halo, and
+ * the "varies" flags are combined over all tiles and ranks (max).  The windows of neighbouring tiles overlap, so
+ * "uniform on every window" is "uniform everywhere", and likewise for "uniform along x".
+ * Varying stretching on a red-black group: tables over own cells + halo on the distributed levels; the solver tile
+ * receives the stretching of level La-1 the way the cycle gathers res, restricts it down to level 1 and builds the
+ * tables of those levels, so the coarse levels (k_coarse_rb included) run as on one grid. */
+static int g_stretching(msqg_group *G) {
+  msqg_model *S = G->tiles[0];
+  const int D = S->depth, La = S->agg_level, nl = G->p.nl;
+  int rc;
+  if (nl < 2) return MSQG_OK;
+  std::vector<XItem> items;
+  for (int l = La; l <= D; l++) {
+    XItem X;
+    for (msqg_model *m : G->tiles) { X.arr.push_back(m->str.lev[l]); X.geo.push_back(m->g[l]); }
+    X.nf = nl; X.ring = 1;
+    X.w = MSQG_FRAME - 1;
+    if (X.w > S->g[l].nx) X.w = S->g[l].nx;
+    if (X.w > S->g[l].ny) X.w = S->g[l].ny;
+    items.push_back(X);
+    if (items.size() == XCHG_MAXITEMS || l == D) {
+      if ((rc = exchange_multi(G, items))) return rc;
+      items.clear();
+    }
+  }
+  dim3 b(32, 8);
+  for (msqg_model *m : G->tiles) {
+    const Geom &g = m->g[D];
+    /* own cells plus one halo cell on the internal sides: enough for the windows of neighbours to overlap */
+    const int x0 = (g.bc & 1) ? -1 : 0, x1 = g.nx + ((g.bc & 2) ? 1 : 0), y0 = (g.bc & 4) ? -1 : 0, y1 = g.ny + ((g.bc & 8) ? 1 : 0);
+    CK(zero_words(G->stream, m->d_scal + 1, 2));
+    k_stretch_varies<<<grid2(x1 - x0, y1 - y0, b, nl - 1), b, 0, G->stream>>>(m->str.lev[D], g, x0, x1, y0, y1, m->d_scal + 1);
+    m->launches++;
+  }
+  CK(cudaGetLastError());
+  double varies[2];
+  if ((rc = reduce_max(G, 1, 2, varies))) return rc;
+  for (msqg_model *m : G->tiles) {
+    m->s_uniform = varies[0] == 0.;
+    m->s_rowuniform = varies[1] == 0.;
+    if (!m->s_uniform) m->s_lev.assign((size_t)(D + 1) * nl, 0.); /* a tile that is uniform on its own cells kept constants */
+  }
+  if (S->s_uniform || !G->rb) return MSQG_OK; /* lexicographic groups refuse varying stretching (g_check_stretching) */
+  for (msqg_model *m : G->tiles) {
+    if ((rc = build_stretch_tables(m, La, D))) return rc;
+    /* this tile's block of level La-1, staged for the gather */
+    k_restrict<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nl), b, 0, G->stream>>>(m->str.lev[La], m->res_patch, m->g[La], m->gpatch, 1., 1);
+    k_unpack<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nl), b, 0, G->stream>>>(m->patch_stage, m->res_patch, nl, m->gpatch);
+    m->launches += 2;
+  }
+  CK(cudaGetLastError());
+  if ((rc = g_gather_coarse(G, nl, S->str.lev[La - 1]))) return rc;
+  for (int l = La - 2; l >= 1; l--) {
+    k_restrict<<<grid2(S->g[l].nx, S->g[l].ny, b, nl), b, 0, G->stream>>>(S->str.lev[l + 1], S->str.lev[l], S->g[l + 1], S->g[l], 1., 1);
+    S->launches++;
+  }
+  CK(cudaGetLastError());
+  if (La > 1 && (rc = build_stretch_tables(S, 1, La - 1))) return rc;
+  CK(cudaStreamSynchronize(G->stream));
+  return MSQG_OK;
+}
+/* what the layer-coupled solve of a group cannot run */
+static int g_check_stretching(msqg_group *G) {
+  if (G->tiles[0]->s_uniform) return MSQG_OK;
+  if (!G->rb)
+    FAIL(MSQG_ERR_ARG, "horizontally varying stretching (varRo, frpg) on tiles needs the red-black smoother: the lexicographic "
+                       "tile sweep has no coefficient tables");
+  if (G->p.nl > 6) FAIL(MSQG_ERR_ARG, "varRo > 0 with the layer-coupled solver is built for nl <= 6 (nl = %d)", G->p.nl);
+  return MSQG_OK;
+}
 extern "C" int msqg_group_set_const(msqg_group *G) {
   CK(cudaSetDevice(G->device));
   G->graphs.clear();
   int rc;
   const int D = G->tiles[0]->depth;
   for (msqg_model *m : G->tiles)
-    if ((rc = set_const_local(m))) return rc;
+    if ((rc = set_const_local(m, false))) return rc;
   if (G->p.mode_pv_invert && (rc = g_check_modes_agree(G))) return rc;
+  if ((rc = g_stretching(G))) return rc;
   for (int id : {MSQG_PSI, MSQG_PSIPG, MSQG_TOPO})
     if ((rc = exchange_list(G, id, D))) return rc;
   for (msqg_model *m : G->tiles)

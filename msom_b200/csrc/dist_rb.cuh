@@ -323,7 +323,12 @@ static int relax_rb_tile(msqg_model *m, int lev, int sweeps, int h_in, const Rel
     const int ho = h - 2 * ns;
     if (ho < 0) FAIL(MSQG_ERR_ARG, "halo of %d cells is too thin for %d sweeps", h_in, sweeps);
     const int orange[4] = {(g.bc & 1) ? -ho : 0, g.nx + ((g.bc & 2) ? ho : 0), (g.bc & 4) ? -ho : 0, g.ny + ((g.bc & 8) ? ho : 0)};
-    int rc = launch_relax_rb_pass<NL, false>(m, m->da.lev[lev], m->res.lev[lev], lev, ns, C, orange, h);
+    int rc;
+    if (relax_uses_table<NL>(m)) { /* horizontally varying stretching: tables over own cells + halo (g_stretching) */
+      if constexpr (NL <= 6) rc = launch_relax_rb_pass<NL, true>(m, m->da.lev[lev], m->res.lev[lev], lev, ns, C, orange, h);
+      else FAIL(MSQG_ERR_ARG, "varRo > 0 with the layer-coupled solver is built for nl <= 6 (nl = %d)", NL);
+    } else
+      rc = launch_relax_rb_pass<NL, false>(m, m->da.lev[lev], m->res.lev[lev], lev, ns, C, orange, h);
     if (rc) return rc;
     left -= ns; h = ho;
   }
@@ -338,6 +343,27 @@ __global__ void k_place_all(double *__restrict__ full, Geom gfull, const double 
   if (x >= hx || y >= hy) return;
   const int ox = (r % px) * hx, oy = (r / px) * hy;
   full[(size_t)f * gfull.plane + GIDX(gfull.pitch, oy + y, ox + x)] = gathered[(((size_t)r * nf + f) * hy + y) * hx + x];
+}
+
+/* the solver tile receives every tile's patch_stage block (nf planes of gpatch) into its level La-1 field `full` (under
+ * NCCL every rank's tile: all-gather) */
+static int g_gather_coarse(msqg_group *G, int nf, double *full) {
+  msqg_model *S = G->tiles[0];
+  const int La = S->agg_level, nt = (int)G->tiles.size(), nranks = G->px * G->py;
+  const int hx = S->gpatch.nx, hy = S->gpatch.ny;
+  const size_t blk = (size_t)nf * hx * hy;
+  if (G->kind == 0) {
+    for (int r = 0; r < nt; r++)
+      CK(cudaMemcpyAsync(S->gather_buf + (size_t)r * blk, G->tiles[r]->patch_stage, blk * sizeof(double), cudaMemcpyDeviceToDevice, G->stream));
+  } else {
+    ProfScope ps_g(S, PROF_XCHG, 100);
+    NCK(G->nccl->AllGather(S->patch_stage, S->gather_buf, blk, NCCL_DOUBLE, G->comm, G->stream));
+  }
+  dim3 b(32, 8);
+  k_place_all<<<grid2(hx, hy, b, nranks * nf), b, 0, G->stream>>>(full, S->g[La - 1], S->gather_buf, hx, hy, G->px, nranks, nf);
+  S->launches++;
+  CK(cudaGetLastError());
+  return MSQG_OK;
 }
 
 /* a += da on the one-cell halo ring of the INTERNAL sides (cells owned by a neighbouring tile; corners included when both
@@ -364,7 +390,7 @@ static int g_cycle(msqg_group *G, const std::vector<MgProblem> &P, int nrelax) {
   /* S = tiles[0] (this rank's tile under NCCL) solves the levels below agg_level; every tile has its geometry */
   msqg_model *S = G->tiles[0];
   const int D = S->depth, La = S->agg_level, nf = P[0].nf, mode = P[0].mode;
-  const int nt = (int)G->tiles.size(), nranks = G->px * G->py;
+  const int nt = (int)G->tiles.size();
   dim3 b(32, 8);
   int rc;
   /* restriction(res) on the distributed levels, then onto this tile's share of level La-1 */
@@ -379,20 +405,10 @@ static int g_cycle(msqg_group *G, const std::vector<MgProblem> &P, int nrelax) {
     m->launches += 2;
   }
   CK(cudaGetLastError());
-  /* the solver tile receives every tile's block of level La-1 (under NCCL every rank's tile: all-gather) */
-  const int hx = S->gpatch.nx, hy = S->gpatch.ny;
-  const size_t blk = (size_t)nf * hx * hy;
-  if (G->kind == 0) {
-    for (int r = 0; r < nt; r++)
-      CK(cudaMemcpyAsync(S->gather_buf + (size_t)r * blk, G->tiles[r]->patch_stage, blk * sizeof(double), cudaMemcpyDeviceToDevice, G->stream));
-  } else {
-    ProfScope ps_g(S, PROF_XCHG, 100);
-    NCK(G->nccl->AllGather(S->patch_stage, S->gather_buf, blk, NCCL_DOUBLE, G->comm, G->stream));
-  }
+  if ((rc = g_gather_coarse(G, nf, S->res.lev[La - 1]))) return rc;
   /* levels 1 .. La-1 on the solver tile: the undecomposed multigrid, whose arithmetic does not depend on the tiles */
-  k_place_all<<<grid2(hx, hy, b, nranks * nf), b, 0, G->stream>>>(S->res.lev[La - 1], S->g[La - 1], S->gather_buf, hx, hy, G->px, nranks, nf);
-  S->launches++;
   if ((rc = mg_levels(S, nf, mode, nrelax, La - 1, La - 1))) return rc;
+  const int hx = S->gpatch.nx, hy = S->gpatch.ny;
   /* every tile's block of level La-1 plus a one-cell ring (homogeneous dirichlet ghosts evaluated on the fly) */
   for (msqg_model *m : G->tiles) {
     k_extract_patch<<<grid2(hx + 2, hy + 2, b, nf), b, 0, G->stream>>>(S->da.lev[La - 1], S->g[La - 1], m->patch_stage, hx, hy, m->ix * hx, m->iy * hy,

@@ -667,12 +667,15 @@ __device__ __forceinline__ void st_mail2_if(bool p, unsigned long long *a, unsig
 
 /* Per-row Thomas coefficients of one level for stretching that varies with y only (varRo > 0): the expressions
  * of relax_coef_layers() (msqg/poisson_layer.h:89-139, same order, IEEE division) evaluated with the level's
- * restricted stretching field at column 0 of every row.  out[j][6][NL] = t0, t2, t1p, rinv, cf, cb. */
+ * restricted stretching field at column 0 of every row.  out[j][6][NL] = t0, t2, t1p, rinv, cf, cb.
+ * The table covers rows y0 .. y0 + th - 1 and, per cell, columns x0 .. x0 + tw - 1: a tile's own cells plus the halo
+ * of its internal sides (x0, y0 < 0), the undecomposed level with x0 = y0 = 0, tw = nx, th = ny. */
 template <int NL>
-__global__ void k_rowcoef(const double *__restrict__ s, Geom g, LayerMetrics M, double *__restrict__ out, int cell) {
+__global__ void k_rowcoef(const double *__restrict__ s, Geom g, LayerMetrics M, double *__restrict__ out, int cell, int x0, int y0, int tw,
+                          int th) {
   const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; /* one thread per row, or per cell (x fastest) */
-  if (t >= (size_t)g.ny * (cell ? g.nx : 1)) return;
-  const int j = cell ? (int)(t / g.nx) : (int)t, ix = cell ? (int)(t % g.nx) : 0;
+  if (t >= (size_t)th * (cell ? tw : 1)) return;
+  const int j = y0 + (cell ? (int)(t / tw) : (int)t), ix = cell ? x0 + (int)(t % tw) : 0;
   const double D2 = g.Delta * g.Delta;
   double sv[NL], t0[NL], t1[NL], t2[NL];
 #pragma unroll

@@ -135,7 +135,9 @@ struct msqg_model {
   double sbcc;                 /* partial slip coefficient of comp_del2 (qg.h:185-198), 0 = free slip */
   bool s_uniform;
   bool s_rowuniform;           /* stretching depends on y only (varRo > 0): per-row relax coefficients */
-  double *rowcoef[MSQG_MAXLEV + 1]; /* device tables [ny][6][nl] per level, or NULL */
+  double *rowcoef[MSQG_MAXLEV + 1]; /* device tables [rows][6][nl] or [rows][cols][6][nl] per level, or NULL */
+  int coef_mx[MSQG_MAXLEV + 1], coef_my[MSQG_MAXLEV + 1]; /* margin of a table on the left / bottom side (tiles: the halo) */
+  int coef_w[MSQG_MAXLEV + 1];  /* cells per row of a per-cell table (own cells + margins) */
   std::vector<double> s_lev;   /* [(depth+1)][nl] */
   std::vector<double> h_fr;    /* host copy of Frl finest [nl][N][N] */
   /* modal */
@@ -534,7 +536,7 @@ static int create_model(const msqg_params *p, int device, int px, int py, int ix
   CK(cudaHostAlloc(&m->h_err, sizeof(int), cudaHostAllocMapped | cudaHostAllocPortable));
   m->mailbox = nullptr; m->mailbox_words = 0; m->d_dbg = nullptr;
   m->nme_ft = 0; m->energy_vars = 0; m->filter_vars = 0; m->siglev0 = 0.;
-  for (int l = 0; l <= MSQG_MAXLEV; l++) m->rowcoef[l] = nullptr;
+  for (int l = 0; l <= MSQG_MAXLEV; l++) { m->rowcoef[l] = nullptr; m->coef_mx[l] = m->coef_my[l] = m->coef_w[l] = 0; }
   for (int k = 0; k < MSQG_NLMAX; k++) for (int l = 0; l <= MSQG_MAXLEV; l++) m->modecoef[k][l] = nullptr;
   m->coef_mode = -1; m->modes_uniform = true;
   m->s_rowuniform = false;
@@ -707,6 +709,10 @@ extern "C" int msqg_set_energy_conserv(msqg_model *m, int on) {
 }
 extern "C" int msqg_get_energy_conserv(msqg_model *m) { return m->econs; }
 extern "C" int msqg_get_smoother(msqg_model *m) { return m->smoother; }
+extern "C" int msqg_stretch_tables(msqg_model *m) {
+  if (!m->const_set) FAIL(MSQG_ERR_ARG, "the stretching path is decided by set_const");
+  return m->s_uniform ? 0 : (m->s_rowuniform ? 1 : 2);
+}
 extern "C" int msqg_set_keep_dq(msqg_model *m, int keep) { m->keep_dq = keep; return MSQG_OK; }
 extern "C" int msqg_set_dissipation(msqg_model *m, double iRe, double iRe4, double Eks, double Ekb) {
   m->iRe = iRe; m->iRe4 = iRe4; m->Eks = Eks; m->Ekb = Ekb; /* pystep_bfn flips these, qg_bfn.h:34-44 */
@@ -932,10 +938,19 @@ static RelaxCoef<1> relax_coef_scalar(msqg_model *m, int lev, double lambda) {
 /* ------------------------------------------------------------------ relax launch */
 /* coefficient table of the current relax launch: the stretching tables of the layer-coupled solver (k_rowcoef), or
    the lambda tables of one vertical mode (k_modecoef) while a scalar solve with a lambda FIELD is running */
-static inline const double *relax_table(const msqg_model *m, int lev) {
-  return m->coef_mode >= 0 ? m->modecoef[m->coef_mode][lev] : m->rowcoef[lev];
-}
 static inline bool relax_table_per_cell(const msqg_model *m) { return m->coef_mode >= 0 || !m->s_rowuniform; }
+/* ... as a pointer to the entry of own cell (0, 0): the stretching tables of a tile also cover its halo (margins) */
+static inline const double *relax_table(const msqg_model *m, int lev) {
+  if (m->coef_mode >= 0) return m->modecoef[m->coef_mode][lev];
+  if (!m->rowcoef[lev]) return nullptr;
+  const bool cell = relax_table_per_cell(m);
+  return m->rowcoef[lev] + ((size_t)m->coef_my[lev] * (cell ? m->coef_w[lev] : 1) + (cell ? m->coef_mx[lev] : 0)) * 6 * m->nl;
+}
+/* entries per row of the table of relax_table (0: one entry per row) */
+static inline int relax_table_stride(const msqg_model *m, int lev) {
+  if (!relax_table_per_cell(m)) return 0;
+  return m->coef_mode >= 0 ? m->g[lev].nx : m->coef_w[lev];
+}
 /* does a relax launch on NL coupled unknowns read tables (true) or per-level constants (false)? */
 template <int NL>
 static inline bool relax_uses_table(const msqg_model *m) { return NL > 1 ? !m->s_uniform : m->coef_mode >= 0; }
@@ -1089,9 +1104,9 @@ static int launch_relax_rb_pass(msqg_model *m, double *da, const double *res, in
   A.ylo = (g.bc & 4) ? -halo : 0; A.yhi = g.ny + ((g.bc & 8) ? halo : 0);
   A.par0 = 0; /* tile origins are even on every distributed level (tiles keep >= 8 cells per side) */
   A.coef = RCOEF ? relax_table(m, lev) : nullptr;
-  A.coef_cell = (RCOEF && relax_table_per_cell(m)) ? 1 : 0;
+  A.coef_cell = RCOEF ? relax_table_stride(m, lev) : 0;
   A.reuse = m->rb_reuse;
-  if (RCOEF && (g.bc || !A.coef)) FAIL(MSQG_ERR_ARG, "horizontally varying stretching (varRo, frpg) is supported on undecomposed levels only");
+  if (RCOEF && !A.coef) FAIL(MSQG_ERR_ARG, "no coefficient table on level %d", lev);
   const int nxo_ = A.ox_hi - A.ox_lo, nyo_ = A.oy_hi - A.oy_lo;
   const bool fold = corr_a != nullptr;
   if (fold) {
@@ -1690,8 +1705,36 @@ static int max_face_speed(msqg_model *m, List &L, double *umax_host) {
   return MSQG_OK;
 }
 
-/* set_const up to (not including) comp_q: everything that is local to a tile */
-static int set_const_local(msqg_model *m) {
+/* varRo > 0: the stretching depends on y only -> per-row Thomas coefficients for the relax kernel, built on the device
+ * from the restricted stretching field of levels lo .. hi (same expressions as relax_coef_layers); stretching that varies
+ * with x as well (Fr from frpg_*.bas, qg.h:957-962): the same table per CELL.  On the levels of a tile the table also
+ * covers the halo of the internal sides, as deep as the sweeps of one exchange reach (g_cycle: at most MSQG_FRAME - 1
+ * cells, capped at the tile size); the stretching must have been exchanged there. */
+static int build_stretch_tables(msqg_model *m, int lo, int hi) {
+  const int nl = m->nl;
+  const LayerMetrics M = metrics_of(m);
+  const int cell = m->s_rowuniform ? 0 : 1;
+  for (int l = lo; l <= hi; l++) {
+    const Geom &gl = m->g[l];
+    if (m->rowcoef[l]) { CK(cudaFree(m->rowcoef[l])); m->rowcoef[l] = nullptr; }
+    int mg = MSQG_FRAME - 1;
+    if (mg > gl.nx) mg = gl.nx;
+    if (mg > gl.ny) mg = gl.ny;
+    const int mx = (gl.bc & 1) ? mg : 0, my = (gl.bc & 4) ? mg : 0;
+    const int tw = gl.nx + mx + ((gl.bc & 2) ? mg : 0), th = gl.ny + my + ((gl.bc & 8) ? mg : 0);
+    m->coef_mx[l] = mx; m->coef_my[l] = my; m->coef_w[l] = tw;
+    const size_t ent = (size_t)th * (cell ? tw : 1);
+    CK(cudaMalloc(&m->rowcoef[l], ent * 6 * nl * sizeof(double)));
+    NL_SWITCH(nl, k_rowcoef<NL><<<(unsigned)((ent + 127) / 128), 128, 0, m->stream>>>(m->str.lev[l], gl, M, m->rowcoef[l], cell, -mx, -my, tw, th));
+    m->launches++;
+  }
+  CK(cudaGetLastError());
+  return MSQG_OK;
+}
+
+/* set_const up to (not including) comp_q: everything that is local to a tile.  tables = false (tiles of a group): no
+ * stretching tables, the group builds them once it has decided the path for all tiles */
+static int set_const_local(msqg_model *m, bool tables = true) {
   CK(cudaSetDevice(m->device));
   m->graphs.clear(); /* recorded cycles hold the old coefficients */
   const int nl = m->nl, D = m->depth;
@@ -1761,22 +1804,9 @@ static int set_const_local(msqg_model *m) {
         m->s_lev[(size_t)lev * nl + l] = avg4(v, v, v, v);
       }
   }
-  /* varRo > 0: the stretching depends on y only -> per-row Thomas coefficients for the relax kernel, built on the
-     device from the restricted stretching field of every level (same expressions as relax_coef_layers) */
   for (int l = 0; l <= MSQG_MAXLEV; l++) if (m->rowcoef[l]) { CK(cudaFree(m->rowcoef[l])); m->rowcoef[l] = nullptr; }
-  if (!uniform && m->g[D].bc == 0 && m->agg_level <= 1) {
-    /* stretching that varies with x as well (Fr from frpg_*.bas, qg.h:957-962): the same table per CELL */
-    const LayerMetrics M = metrics_of(m);
-    const int cell = rowuniform ? 0 : 1;
-    for (int l = 1; l <= D; l++) {
-      const Geom &gl = m->g[l];
-      const size_t ent = (size_t)gl.ny * (cell ? gl.nx : 1);
-      CK(cudaMalloc(&m->rowcoef[l], ent * 6 * nl * sizeof(double)));
-      NL_SWITCH(nl, k_rowcoef<NL><<<(unsigned)((ent + 127) / 128), 128, 0, m->stream>>>(m->str.lev[l], gl, M, m->rowcoef[l], cell));
-      m->launches++;
-    }
-    CK(cudaGetLastError());
-  }
+  /* a group decides uniform / per-row / per-cell for all its tiles together and builds their tables itself (g_stretching) */
+  if (tables && !uniform && (rc = build_stretch_tables(m, 1, D))) return rc;
   /* wind forcing table, qg.h:451, host libm so that sin() matches the reference */
   {
     std::vector<double> w(ty);

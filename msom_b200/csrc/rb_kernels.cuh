@@ -51,8 +51,9 @@ struct RbArgs {
   int ox_lo, ox_hi, oy_lo, oy_hi; /* cells stored by this launch (own cells; a tile may add a ring of halo cells) */
   int xlo, xhi, ylo, yhi;         /* cells that exist in memory: own cells + deep halo on internal sides */
   int par0;           /* parity of the tile origin (x0 + y0) & 1 */
-  const double *coef; /* RCOEF: per-row [ny][6][NL] or per-cell [ny][nx][6][NL] Thomas coefficients (k_rowcoef) */
-  int coef_cell;
+  const double *coef; /* RCOEF: per-row [rows][6][NL] or per-cell [rows][coef_cell][6][NL] Thomas coefficients (k_rowcoef),
+                         pointing at the entry of cell (0, 0); a tile's table also holds its halo */
+  int coef_cell;      /* RCOEF: entries per row of a per-cell table, 0 = per-row table */
   int reuse;          /* 1: south / in-pair neighbours from registers (default); 0: always from shared memory */
   double *a;          /* k_relax_rb<..., FOLD = true>, last pass on the finest level of an undecomposed grid: the store is
                          a += da with the dirichlet ghost ring of a (k_correct) instead of da_out = da; da_out is not
@@ -253,10 +254,11 @@ k_relax_rb(RbArgs A, RelaxCoef<NL> C) {
 #pragma unroll
         for (int l = NL - 2; l >= 0; l--) out[l] = div_by(rhs[l] - C.t2[l] * out[l + 1], C.t1p[l], C.rinv[l]);
       } else {
-        /* horizontally varying stretching: coefficients of this row / cell from the k_rowcoef table (own cells only) */
+        /* horizontally varying stretching: coefficients of this row / cell from the k_rowcoef table, which covers the
+           cells that exist (a tile's table also covers its halo); window cells beyond them are garbage anyway */
         const int j = jw0 + r, gx = upd ? gxb : gxa;
-        const int jc = j < 0 ? 0 : (j > ny - 1 ? ny - 1 : j), xc = gx < 0 ? 0 : (gx > nx - 1 ? nx - 1 : gx);
-        const double *ct = A.coef + (A.coef_cell ? (size_t)jc * nx + xc : (size_t)jc) * 6 * NL;
+        const int jc = min(max(j, A.ylo), A.yhi - 1), xc = min(max(gx, A.xlo), A.xhi - 1);
+        const double *ct = A.coef + (A.coef_cell ? (long long)jc * A.coef_cell + xc : (long long)jc) * 6 * NL;
         double t0[NL], t2[NL], t1p[NL], rinv[NL];
 #pragma unroll
         for (int l = 0; l < NL; l++) { t0[l] = ct[l]; t2[l] = ct[NL + l]; t1p[l] = ct[2 * NL + l]; rinv[l] = ct[3 * NL + l]; }
@@ -529,8 +531,8 @@ k_relax_rb_tile(RbArgs A, RelaxCoef<NL> C) {
         out[NL - 1] = div_by(rhs[NL - 1], C.t1p[NL - 1], C.rinv[NL - 1]);
 #pragma unroll
         for (int f = NL - 2; f >= 0; f--) out[f] = div_by(rhs[f] - C.t2[f] * out[f + 1], C.t1p[f], C.rinv[f]);
-      } else { /* coefficients of this row / cell from the k_rowcoef / k_modecoef table (undecomposed levels: gx, gy are own cells) */
-        const double *ct = A.coef + (A.coef_cell ? (size_t)gy * nx + gx : (size_t)gy) * 6 * NL;
+      } else { /* coefficients of this row / cell from the k_rowcoef / k_modecoef table (it covers every cell of the window) */
+        const double *ct = A.coef + (A.coef_cell ? (long long)gy * A.coef_cell + gx : (long long)gy) * 6 * NL;
         double t0[NL], t2[NL], t1p[NL], rinv[NL];
 #pragma unroll
         for (int f = 0; f < NL; f++) { t0[f] = ct[f]; t2[f] = ct[NL + f]; t1p[f] = ct[2 * NL + f]; rinv[f] = ct[3 * NL + f]; }

@@ -58,6 +58,7 @@ def _bind():
     L.msqg_group_timer.argtypes = [vp, C.c_int, pd]
     L.msqg_group_profile_enable.argtypes = [vp, C.c_int]
     L.msqg_group_profile_read.argtypes = [vp, pd, C.POINTER(C.c_long), C.POINTER(C.c_long)]
+    L.msqg_stretch_tables.argtypes = [vp]
     _bound = True
     return L
 
@@ -198,6 +199,13 @@ class Group:
         ms = (C.c_double * 9)(); cnt = (C.c_long * 9)(); aux = (C.c_long * 9)()
         G.check(self.L.msqg_group_profile_read(self.h, ms, cnt, aux))
         return {k: dict(ms=ms[i], count=cnt[i], aux=aux[i]) for i, k in enumerate(G.Model.PROF_CATS)}
+
+    @property
+    def stretching(self):
+        """G.Model.stretching of the group: one decision for all tiles and ranks, read from tile 0"""
+        rc = self.L.msqg_stretch_tables(self.L.msqg_group_tile(self.h, 0))
+        G.check(min(rc, 0))
+        return G.Model.STRETCHING[rc]
 
     @property
     def total_cycles(self):

@@ -1,8 +1,9 @@
-"""torchrun --nproc-per-node N scripts/dist_check.py [lex|rb|rbper|rbmodal|rbstoch|rbperstoch] : the NCCL back-end of
+"""torchrun --nproc-per-node N scripts/dist_check.py [lex|rb|rbper|rbmodal|rbstoch|rbperstoch|rbvary] : the NCCL back-end of
 the domain decomposition against the CPU oracle's emulation of the same decomposition, bit for bit, on every rank.
 rbmodal: the vertical-mode inversion (mode_pv_invert = 1) on red-black tiles, every mode's statistics compared too.
 rbstoch / rbperstoch: stochastic forcing with libc noise on the closed basin / the periodic domain: every rank replays
-the reference's rand() stream from the same seed and keeps its tile's cells; the oracle draws from srand(seed)."""
+the reference's rand() stream from the same seed and keeps its tile's cells; the oracle draws from srand(seed).
+rbvary: horizontally varying stretching, varRo > 0 together with a Fr(x, y) field (per-cell coefficient tables)."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -25,10 +26,14 @@ stoch = sm in ("rbstoch", "rbperstoch")
 if stoch:
     sm = "rbper" if sm == "rbperstoch" else "rb"
 STOCH = dict(stochastic=1, tr_stoch=10., amp_stoch=1.) if stoch else {}
+vary = sm == "rbvary"
+if vary:
+    sm = "rb"
+VARY = dict(varRo=1) if vary else {}
 SEED = 2024
 if sm == "rb":
     agg_n = 128 if world > 2 else 64
-kw = base_kw(N, nl, mode_pv_invert=1) if modal else base_kw(N, nl, **STOCH)
+kw = base_kw(N, nl, mode_pv_invert=1) if modal else base_kw(N, nl, **STOCH, **VARY)
 periodic = sm == "rbper"   # doubly periodic domain (sbc = -1) on the process grid: neighbours wrap around
 if periodic:
     sm = "rb"
@@ -42,15 +47,22 @@ if periodic:
 sig = np.full((nl, N, N), 1e-3) * (1 + np.arange(nl)[:, None, None])
 if stoch:
     g.set_global(G.SSTOCH, sig)
+fr = None
+if vary:
+    from test_gpu_dist_stretching import _fr_field
+    fr = _fr_field(N, nl)
+    g.set_global(G.FR, fr)
 g.set_global(G.PSI, psi); g.set_const()
 mo = O.Model(O.make_params(**kw)); mo.L.orc_set_decomp(mo.h, px, py, agg_n); mo.set_smoother(sm)
 mo.set(O.PSI, psi)
+if vary:
+    mo.set(O.FR, fr)
 if stoch:
     mo.set(O.SSTOCH, sig)
     import ctypes
     ctypes.CDLL(None).srand(SEED)
 mo.set_const()
-ok = True
+ok = not vary or g.stretching == "cells"
 for s in range(3):
     ok &= (g.step() == mo.step())
 if modal:
@@ -64,7 +76,7 @@ ok &= (g.total_cycles == mo.L.orc_total_cycles(mo.h))
 t = torch.tensor([1 if ok else 0], device="cuda")
 dist.all_reduce(t, op=dist.ReduceOp.MIN)
 if rank == 0:
-    print("DIST_CHECK", "PASS" if int(t.item()) == 1 else "FAIL", sm + ("-periodic" if periodic else "") + ("-modal" if modal else "") + ("-stochastic" if stoch else ""), g.transport, "world", world, "grid %dx%d" % (px, py), "exchanges", g.exchanges)
+    print("DIST_CHECK", "PASS" if int(t.item()) == 1 else "FAIL", sm + ("-periodic" if periodic else "") + ("-modal" if modal else "") + ("-stochastic" if stoch else "") + ("-varying-stretching" if vary else ""), g.transport, "world", world, "grid %dx%d" % (px, py), "exchanges", g.exchanges)
 g.close()
 dist.destroy_process_group()
 sys.exit(0 if int(t.item()) == 1 else 1)
