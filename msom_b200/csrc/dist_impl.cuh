@@ -115,7 +115,6 @@ struct msqg_group {
   NcclApi *nccl;
   ncclComm_t comm;
   double *d_red, *h_red; /* reduction scratch (device / pinned host), 64 doubles */
-  double ts_previous;
   msqg_mgstats mgpsi, mgmode[MSQG_MAXL]; /* last solve; per vertical mode (mode_pv_invert) */
   long total_cycles;
   double umax_pg[MSQG_MAXL];
@@ -243,7 +242,7 @@ static int group_create(const msqg_params *p, int device, int px, int py, int ag
   msqg_group *G = new msqg_group();
   G->p = *p; G->px = px; G->py = py; G->agg_n = agg_n; G->device = device; G->kind = kind;
   G->rank = rank; G->nranks = nranks; G->nccl = nullptr; G->comm = nullptr; G->rb = smoother == 1;
-  G->ts_previous = 0.; G->total_cycles = 0; G->exchanges = 0;
+  G->total_cycles = 0; G->exchanges = 0;
   memset(&G->mgpsi, 0, sizeof(G->mgpsi));
   memset(G->mgmode, 0, sizeof(G->mgmode));
   memset(G->umax_pg, 0, sizeof(G->umax_pg));
@@ -340,36 +339,13 @@ static std::vector<MgProblem> g_problem(msqg_group *G, int mode, int q_id) {
   }
   return P;
 }
+/* a tile's stream is the group's (create_model, pg_set_stream) */
 static int g_residual_enqueue(msqg_group *G, const std::vector<MgProblem> &P) {
   for (int t = 0; t < (int)G->tiles.size(); t++) {
-    msqg_model *m = G->tiles[t];
-    const int D = m->depth;
-    const Geom &g = m->g[D];
-    CK(zero_words(G->stream, m->d_scal, 1));
-    dim3 b(64, 4);
-    ProfScope ps(m, PROF_RESIDUAL, 0);
-    if (P[t].mode < 0) {
-      LayerMetrics M = metrics_of(m);
-      NL_SWITCH(m->nl, k_residual<NL><<<grid2(g.nx, g.ny, b), b, 0, G->stream>>>(P[t].a, P[t].b, m->res.lev[D], m->str.lev[D], g, M, m->d_scal));
-    } else
-      k_residual_scalar<<<grid2(g.nx, g.ny, b), b, 0, G->stream>>>(P[t].a, P[t].b, m->res.lev[D], m->ibu.lev[D] + (size_t)P[t].mode * g.plane, g,
-                                                                   m->d_scal);
-    m->launches++;
+    int rc = launch_residual(G->tiles[t], P[t]);
+    if (rc) return rc;
   }
-  CK(cudaGetLastError());
   return reduce_max_enqueue(G, 0, 1);
-}
-static int g_residual(msqg_group *G, const std::vector<MgProblem> &P, double *maxres) {
-  int rc = g_residual_enqueue(G, P);
-  if (rc) return rc;
-  return reduce_max_finish(G, 1, maxres);
-}
-
-static int g_relax_level(msqg_group *G, msqg_model *m, int l, int nsweeps) {
-  int rc;
-  ProfScope ps(m, l == m->depth ? PROF_RELAX_FINE : PROF_RELAX_COARSE, nsweeps);
-  NL_SWITCH(m->nl, { auto C = relax_coef_layers<NL>(m, l); rc = launch_relax<NL>(m, m->da.lev[l], m->res.lev[l], l, nsweeps, C); });
-  return rc;
 }
 
 static int g_check_err(msqg_group *G) {
@@ -382,42 +358,18 @@ static int g_check_err(msqg_group *G) {
 
 #include "dist_rb.cuh"
 
-/* mg_solve on the decomposed grid: problem P[t] on tile t (NITERMIN 1, NITERMAX 100, nrelax starts at 4); sched as
- * mg_solve's */
-static int g_solve(msqg_group *G, const std::vector<MgProblem> &P, msqg_mgstats *st, const int *sched = nullptr,
-                   int ncycles = 0, double *resa_out = nullptr) {
-  int rc;
+/* mg_solve on the decomposed grid: problem P[t] on tile t; the residual norm is the max over tiles and ranks.  sched,
+ * ncycles, resa_out as mg_solve_loop's */
+static int g_solve(msqg_group *G, const std::vector<MgProblem> &P, double tolerance, msqg_mgstats *st,
+                   const int *sched = nullptr, int ncycles = 0, double *resa_out = nullptr) {
+  bool graphed = G->rb && G->tiles[0]->use_graphs != 0;
+  for (msqg_model *m : G->tiles) graphed = graphed && !m->prof_on;
   msqg_mgstats s;
-  memset(&s, 0, sizeof(s));
-  s.nrelax = 4;
-  double resb;
-  if ((rc = g_residual(G, P, &resb))) return rc;
-  s.resb = s.resa = resb;
-  for (s.i = 0; sched ? s.i < ncycles : s.i < 100 && (s.i < 1 || s.resa > 1e-3); s.i++) {
-    if (sched) s.nrelax = sched[s.i];
-    /* one cycle + residual + its all-reduce: with the red-black smoother a single graph launch (keyed by nrelax, the
-       mode, the unknown and the right-hand side of tile 0 and the current da buffers of every tile) */
-    msqg_model *m0 = G->tiles[0];
-    unsigned long long mask = 0;
-    for (msqg_model *m : G->tiles) mask = mask * 1315423911ull + da_parity_mask(m);
-    bool graphed = G->rb && m0->use_graphs != 0;
-    for (msqg_model *m : G->tiles) graphed = graphed && !m->prof_on;
-    GraphKey key(s.nrelax, P[0].mode, (const void *)P[0].a, (const void *)P[0].b, mask);
-    rc = run_graphed(G->stream, G->graphs, key, G->tiles, &G->exchanges, graphed, [&]() -> int {
-      int r2 = g_cycle(G, P, s.nrelax);
-      if (r2) return r2;
-      return g_residual_enqueue(G, P);
-    });
-    if (rc) return rc;
-    if ((rc = reduce_max_finish(G, 1, &s.resa))) return rc;
-    if (sched) resa_out[s.i] = s.resa;
-    else if (s.resa > 1e-3) {
-      if (resb / s.resa < 1.2 && s.nrelax < 100) s.nrelax++;
-      else if (resb / s.resa > 10 && s.nrelax > 2) s.nrelax--;
-    }
-    resb = s.resa;
-  }
-  if ((rc = g_check_err(G))) return rc;
+  int rc = mg_solve_loop(G->stream, G->graphs, G->tiles, &G->exchanges, graphed, P[0], tolerance, &s, sched, ncycles,
+                         resa_out, [&]() { return g_residual_enqueue(G, P); },
+                         [&](int nrelax) { return g_cycle(G, P, nrelax); },
+                         [&](double *r) { return reduce_max_finish(G, 1, r); });
+  if (rc || (rc = g_check_err(G))) return rc;
   if ((rc = group_check_p2p(G))) return rc;
   G->total_cycles += s.i;
   *st = s;
@@ -434,36 +386,24 @@ static int g_invertq(msqg_group *G, int q_id) {
   if (!G->p.mode_pv_invert) {
     if ((rc = g_check_stretching(G))) return rc;
     if ((rc = exchange_list(G, MSQG_PSI, D))) return rc; /* the warm start's ring */
-    return g_solve(G, g_problem(G, -1, q_id), &G->mgpsi);
+    return g_solve(G, g_problem(G, -1, q_id), 1e-3, &G->mgpsi);
   }
   /* vertical modes (uniform on tiles: group_create and set_const refuse the others, so the matrices are constants) */
   if ((rc = exchange_list(G, MSQG_PM, D))) return rc; /* the warm start's ring, every mode */
-  dim3 b(64, 4), bg(32, 8);
-  for (msqg_model *m : G->tiles) {
-    const Geom &g = m->g[D];
-    NL_SWITCH(m->nl, {
-      ModeMat<NL> M;
-      for (int k = 0; k < NL * NL; k++) M.a[k] = m->h_cl2m[k];
-      k_project<NL><<<grid2(g.nx, g.ny, b), b, 0, G->stream>>>(list_by_id(m, q_id)->lev[D], m->qm.lev[D], g, M, nullptr, 0);
-    });
-    m->launches++;
-  }
-  CK(cudaGetLastError());
+  dim3 bg(32, 8);
+  for (msqg_model *m : G->tiles)
+    if ((rc = launch_project(m, list_by_id(m, q_id)->lev[D], m->qm.lev[D], m->h_cl2m, nullptr, false, 0))) return rc;
   for (int l = 0; l < G->p.nl; l++) {
-    if ((rc = g_solve(G, g_problem(G, l, q_id), &G->mgmode[l]))) return rc;
+    if ((rc = g_solve(G, g_problem(G, l, q_id), 1e-3, &G->mgmode[l]))) return rc;
     G->mgpsi = G->mgmode[l];
   }
   /* psi on the interior and on the ring of the internal sides: each mode's k_correct_ring left the owner's bits of pm
      there, so the neighbour's psi needs no exchange; then the ghosts of the physical sides */
   for (msqg_model *m : G->tiles) {
     const Geom &g = m->g[D];
-    NL_SWITCH(m->nl, {
-      ModeMat<NL> M;
-      for (int k = 0; k < NL * NL; k++) M.a[k] = m->h_cm2l[k];
-      k_project<NL, true><<<grid2(g.nx + 2, g.ny + 2, b), b, 0, G->stream>>>(m->pm.lev[D], m->psi.lev[D], g, M, nullptr, 0);
-    });
+    if ((rc = launch_project(m, m->pm.lev[D], m->psi.lev[D], m->h_cm2l, nullptr, true, 0))) return rc;
     k_ghosts<<<grid2(g.nx + 2, g.ny + 2, bg, m->nl), bg, 0, G->stream>>>(m->psi.lev[D], m->nl, g, -1.);
-    m->launches += 2;
+    m->launches++;
   }
   CK(cudaGetLastError());
   return MSQG_OK;
@@ -481,7 +421,7 @@ extern "C" int msqg_group_test_cycles(msqg_group *G, int mode, const int *nrelax
   if (mode < 0 && (rc = g_check_stretching(G))) return rc;
   if ((rc = exchange_list(G, mode < 0 ? MSQG_PSI : MSQG_PM, G->tiles[0]->depth))) return rc; /* the start's ring, as g_invertq */
   msqg_mgstats st;
-  return g_solve(G, g_problem(G, mode, MSQG_Q), &st, nrelax, ncycles, resa);
+  return g_solve(G, g_problem(G, mode, MSQG_Q), 1e-3, &st, nrelax, ncycles, resa);
 }
 
 /* ------------------------------------------------------------------ fields, set_const */
@@ -491,33 +431,45 @@ extern "C" int msqg_group_set_field(msqg_group *G, int t, int id, const double *
 extern "C" int msqg_group_get_field(msqg_group *G, int t, int id, double *host_tile) {
   return msqg_get_field(G->tiles[t], id, host_tile);
 }
+/* Do n 32-bit words agree on every tile and rank?  words: n per tile, tile after tile.  *differs: the index of the first
+ * word that is not the same everywhere, or -1.  reduce_max takes maxima of non-negative values, so each word h goes in
+ * with its complement 2^32 - 1 - h: max(h) + max(2^32 - 1 - h) = 2^32 - 1 exactly when h is the same everywhere. */
+static int g_words_agree(msqg_group *G, const std::vector<uint32_t> &words, int n, int *differs) {
+  const int nt = (int)G->tiles.size();
+  const double ones = 4294967295.;
+  std::vector<double> w((size_t)nt * 2 * n), out(2 * n);
+  for (int t = 0; t < nt; t++) {
+    double *wt = &w[(size_t)t * 2 * n];
+    for (int k = 0; k < n; k++) { const double h = words[(size_t)t * n + k]; wt[2 * k] = h; wt[2 * k + 1] = ones - h; }
+    CK(cudaMemcpyAsync(G->tiles[t]->d_scal + 1, wt, 2 * n * sizeof(double), cudaMemcpyHostToDevice, G->stream));
+  }
+  int rc = reduce_max(G, 1, 2 * n, out.data());
+  if (rc) return rc;
+  *differs = -1;
+  for (int k = 0; k < n && *differs < 0; k++)
+    if (out[2 * k] + out[2 * k + 1] != ones) *differs = k;
+  return MSQG_OK;
+}
 /* Uniform vertical modes are computed by every tile from its own Fr (set_const_local): a Fr field that is constant on
  * each tile but differs between tiles would give the tiles different matrices and a wrong result without any error.
- * So every tile and rank must have used the same Fr bits.  reduce_max takes maxima of non-negative words, so each value
- * goes in as its two 32-bit halves h and their complements 2^32 - 1 - h: max(h) + max(2^32 - 1 - h) = 2^32 - 1 exactly
- * when h is the same everywhere. */
+ * So every tile and rank must have used the same Fr bits: the two 32-bit halves of each interface's value agree. */
 static int g_check_modes_agree(msqg_group *G) {
-  const int nl = G->p.nl, n = 4 * (nl - 1), nt = (int)G->tiles.size();
-  const double ones = 4294967295.;
-  std::vector<double> w((size_t)nt * n), out(n);
-  for (int t = 0; t < nt; t++) {
-    msqg_model *m = G->tiles[t];
+  const int nl = G->p.nl, n = 2 * (nl - 1);
+  std::vector<uint32_t> words;
+  for (msqg_model *m : G->tiles) {
     const size_t tc = (size_t)m->tnx * m->tny;
-    double *wt = &w[(size_t)t * n];
     for (int l = 0; l < nl - 1; l++) {
       unsigned long long u;
       memcpy(&u, &m->h_fr[(size_t)l * tc], sizeof(u));
-      const double hi = (double)(u >> 32), lo = (double)(u & 0xffffffffull);
-      wt[4 * l] = hi; wt[4 * l + 1] = ones - hi; wt[4 * l + 2] = lo; wt[4 * l + 3] = ones - lo;
+      words.push_back((uint32_t)(u >> 32));
+      words.push_back((uint32_t)u);
     }
-    CK(cudaMemcpyAsync(m->d_scal + 1, wt, n * sizeof(double), cudaMemcpyHostToDevice, G->stream));
   }
-  int rc = reduce_max(G, 1, n, out.data());
+  int k, rc = g_words_agree(G, words, n, &k);
   if (rc) return rc;
-  for (int k = 0; k < n; k += 2)
-    if (out[k] + out[k + 1] != ones)
-      FAIL(MSQG_ERR_ARG, "Fr of interface %d differs between tiles: the vertical-mode inversion on tiles needs the same Fr "
-                         "everywhere (uniform vertical modes)", k / 4);
+  if (k >= 0)
+    FAIL(MSQG_ERR_ARG, "Fr of interface %d differs between tiles: the vertical-mode inversion on tiles needs the same Fr "
+                       "everywhere (uniform vertical modes)", k / 2);
   return MSQG_OK;
 }
 /* One stretching path for the whole group: constants, per-row tables or per-cell tables, decided as the undecomposed
@@ -536,13 +488,7 @@ static int g_stretching(msqg_group *G) {
   if (nl < 2) return MSQG_OK;
   std::vector<XItem> items;
   for (int l = La; l <= D; l++) {
-    XItem X;
-    for (msqg_model *m : G->tiles) { X.arr.push_back(m->str.lev[l]); X.geo.push_back(m->g[l]); }
-    X.nf = nl; X.ring = 1;
-    X.w = MSQG_FRAME - 1;
-    if (X.w > S->g[l].nx) X.w = S->g[l].nx;
-    if (X.w > S->g[l].ny) X.w = S->g[l].ny;
-    items.push_back(X);
+    items.push_back(level_item(G, &msqg_model::str, l, nl, MSQG_FRAME - 1, 1));
     if (items.size() == XCHG_MAXITEMS || l == D) {
       if ((rc = exchange_multi(G, items))) return rc;
       items.clear();
@@ -566,15 +512,9 @@ static int g_stretching(msqg_group *G) {
     if (!m->s_uniform) m->s_lev.assign((size_t)(D + 1) * nl, 0.); /* a tile that is uniform on its own cells kept constants */
   }
   if (S->s_uniform || !G->rb) return MSQG_OK; /* lexicographic groups refuse varying stretching (g_check_stretching) */
-  for (msqg_model *m : G->tiles) {
+  for (msqg_model *m : G->tiles)
     if ((rc = build_stretch_tables(m, La, D))) return rc;
-    /* this tile's block of level La-1, staged for the gather */
-    k_restrict<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nl), b, 0, G->stream>>>(m->str.lev[La], m->res_patch, m->g[La], m->gpatch, 1., 1);
-    k_unpack<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nl), b, 0, G->stream>>>(m->patch_stage, m->res_patch, nl, m->gpatch);
-    m->launches += 2;
-  }
-  CK(cudaGetLastError());
-  if ((rc = g_gather_coarse(G, nl, S->str.lev[La - 1]))) return rc;
+  if ((rc = g_restrict_gather(G, &msqg_model::str, La, nl, 1., 1, S->str.lev[La - 1]))) return rc;
   for (int l = La - 2; l >= 1; l--) {
     k_restrict<<<grid2(S->g[l].nx, S->g[l].ny, b, nl), b, 0, G->stream>>>(S->str.lev[l + 1], S->str.lev[l], S->g[l + 1], S->g[l], 1., 1);
     S->launches++;
@@ -652,45 +592,26 @@ static int g_rhs_prepare(msqg_group *G, double *umax) {
   }
   return reduce_max(G, 1, G->p.nl, umax);
 }
-static double g_dt_chain(msqg_group *G, const double *umax, double dtmax) {
-  msqg_model *m = G->tiles[0];
-  const double Delta = m->g[m->depth].Delta;
-  m->ts_previous = G->ts_previous;
-  for (int l = 0; l < m->nl; l++) {
-    dtmax = timestep_chain(m, umax[l], dtmax, Delta);
-    dtmax = timestep_chain(m, G->umax_pg[l], dtmax, Delta);
-  }
-  G->ts_previous = m->ts_previous;
-  return dtmax;
-}
 /* Stochastic forcing: every tile keeps its own corrector flag, noise mode, seed and draw counter (msqg_seed_noise and
  * msqg_set_noise_mode act on one tile) and all of them advance identically, so the tiles draw, each for its window,
  * the field of the undecomposed model.  Tiles seeded differently would give wrong bits without any error, so at the
  * first stochastic step after a tile's seed or mode changed the group compares mode, seed and draw count across all
- * tiles and ranks, with the complement trick of g_check_modes_agree.  Under NCCL every rank seeds its tile with the
+ * tiles and ranks (g_words_agree).  Under NCCL every rank seeds its tile with the
  * same arguments, so every rank takes this check at the same step. */
 static int g_check_noise_agree(msqg_group *G) {
   bool pending = false;
   for (msqg_model *m : G->tiles) pending |= !m->noise_agreed;
   if (!pending) return MSQG_OK;
-  const int n = 8, nt = (int)G->tiles.size();
-  const double ones = 4294967295.;
-  std::vector<double> w((size_t)nt * n), out(n);
-  for (int t = 0; t < nt; t++) {
-    msqg_model *m = G->tiles[t];
-    const double h[4] = {(double)m->noise_mode, (double)m->noise_seed, (double)(m->noise_draw >> 32),
-                         (double)(m->noise_draw & 0xffffffffull)};
-    double *wt = &w[(size_t)t * n];
-    for (int k = 0; k < 4; k++) { wt[2 * k] = h[k]; wt[2 * k + 1] = ones - h[k]; }
-    CK(cudaMemcpyAsync(m->d_scal + 1, wt, n * sizeof(double), cudaMemcpyHostToDevice, G->stream));
-  }
-  int rc = reduce_max(G, 1, n, out.data());
+  std::vector<uint32_t> words;
+  for (msqg_model *m : G->tiles)
+    for (uint32_t h : {(uint32_t)m->noise_mode, (uint32_t)m->noise_seed, (uint32_t)(m->noise_draw >> 32), (uint32_t)m->noise_draw})
+      words.push_back(h);
+  int k, rc = g_words_agree(G, words, 4, &k);
   if (rc) return rc;
   static const char *what[4] = {"noise mode", "noise seed", "noise draw count", "noise draw count"};
-  for (int k = 0; k < n; k += 2)
-    if (out[k] + out[k + 1] != ones)
-      FAIL(MSQG_ERR_ARG, "the %s differs between tiles: seed every tile of a stochastic group alike (msqg_seed_noise, "
-                         "msqg_set_noise_mode on every tile and rank, with the same arguments)", what[k / 2]);
+  if (k >= 0)
+    FAIL(MSQG_ERR_ARG, "the %s differs between tiles: seed every tile of a stochastic group alike (msqg_seed_noise, "
+                       "msqg_set_noise_mode on every tile and rank, with the same arguments)", what[k]);
   for (msqg_model *m : G->tiles) m->noise_agreed = 1;
   return MSQG_OK;
 }
@@ -702,20 +623,8 @@ extern "C" int msqg_group_step(msqg_group *G, double t, double tnext_event, doub
   double umax[MSQG_MAXL];
   if ((rc = g_invertq(G, MSQG_Q))) return rc;
   if ((rc = g_rhs_prepare(G, umax))) return rc;
-  double dt = g_dt_chain(G, umax, G->p.DT);
   double tnext;
-  if (tnext_event >= 0 && tnext_event > t) {
-    unsigned int nn = (tnext_event - t) / dt;
-    tnext = tnext_event;
-    if (nn == 0) dt = tnext_event - t;
-    else {
-      const double dt1 = (tnext_event - t) / nn;
-      if (dt1 > dt * (1. + 1e-9)) dt = (tnext_event - t) / (nn + 1);
-      else if (dt1 < dt) dt = dt1;
-      tnext = t + dt;
-    }
-  } else
-    tnext = t + dt;
+  double dt = dtnext(t, tnext_event, dt_chain(G->tiles[0], umax, G->umax_pg, G->p.DT), &tnext);
   for (msqg_model *m : G->tiles) { /* msqg_step: the noise of each stage is drawn before its right-hand side */
     const int D = m->depth;
     float dts = 0.f;
@@ -731,7 +640,7 @@ extern "C" int msqg_group_step(msqg_group *G, double t, double tnext_event, doub
     if ((rc = rhs_launch(m, m->qpred, m->q.lev[D], m->q.lev[D], nullptr, dt, dts))) return rc;
   }
   CK(cudaStreamSynchronize(G->stream));
-  (void)g_dt_chain(G, umax, dt);
+  (void)dt_chain(G->tiles[0], umax, G->umax_pg, dt);
   if (dt_out) *dt_out = dt;
   if (tnext_out) *tnext_out = tnext;
   return MSQG_OK;
@@ -803,7 +712,7 @@ static int pg_update(msqg_group *G, msqg_model *m, int q_id, double dtmax, doubl
   if ((rc = g_rhs_prepare(G, umax))) return rc;
   if ((rc = rhs_launch(m, *list_by_id(m, q_id), nullptr, nullptr, m->dq.lev[m->depth], 0., 0.f))) return rc;
   CK(cudaStreamSynchronize(G->stream));
-  if (dtmax_out) *dtmax_out = g_dt_chain(G, umax, dtmax);
+  if (dtmax_out) *dtmax_out = dt_chain(G->tiles[0], umax, G->umax_pg, dtmax);
   return MSQG_OK;
 }
 static int pg_step(msqg_group *G, msqg_model *m, double t, double tnext_event, double *dt_out, double *tnext_out) {

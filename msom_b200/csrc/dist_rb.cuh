@@ -308,31 +308,15 @@ static int exchange_one(msqg_group *G, int id, int lev, int w, int ring) {
   X.w = w; X.ring = ring;
   return exchange_multi(G, items);
 }
-
-/* ------------------------------------------------------------------ relax on a tile with deep halos */
-/* `sweeps` red-black sweeps on tile + halo: the halo holds h_in valid cells on the internal sides on entry and
- * h_in - 2 sweeps on exit (split into passes of at most NSMAX sweeps; bit-identical to sweeping the whole level) */
-template <int NL>
-static int relax_rb_tile(msqg_model *m, int lev, int sweeps, int h_in, const RelaxCoef<NL> &C) {
-  constexpr int NSMAX = RbCfg<NL>::NSMAX;
-  const Geom &g = m->g[lev];
-  int left = sweeps, h = h_in;
-  while (left > 0) {
-    const int passes = (left + NSMAX - 1) / NSMAX;
-    const int ns = (left + passes - 1) / passes;
-    const int ho = h - 2 * ns;
-    if (ho < 0) FAIL(MSQG_ERR_ARG, "halo of %d cells is too thin for %d sweeps", h_in, sweeps);
-    const int orange[4] = {(g.bc & 1) ? -ho : 0, g.nx + ((g.bc & 2) ? ho : 0), (g.bc & 4) ? -ho : 0, g.ny + ((g.bc & 8) ? ho : 0)};
-    int rc;
-    if (relax_uses_table<NL>(m)) { /* horizontally varying stretching: tables over own cells + halo (g_stretching) */
-      if constexpr (NL <= 6) rc = launch_relax_rb_pass<NL, true>(m, m->da.lev[lev], m->res.lev[lev], lev, ns, C, orange, h);
-      else FAIL(MSQG_ERR_ARG, "varRo > 0 with the layer-coupled solver is built for nl <= 6 (nl = %d)", NL);
-    } else
-      rc = launch_relax_rb_pass<NL, false>(m, m->da.lev[lev], m->res.lev[lev], lev, ns, C, orange, h);
-    if (rc) return rc;
-    left -= ns; h = ho;
-  }
-  return MSQG_OK;
+/* the list `list` of level l on every tile, nf planes, a halo of w cells but at most the level's size */
+static XItem level_item(msqg_group *G, List msqg_model::*list, int l, int nf, int w, int ring) {
+  const Geom &g0 = G->tiles[0]->g[l];
+  XItem X;
+  for (msqg_model *m : G->tiles) { X.arr.push_back((m->*list).lev[l]); X.geo.push_back(m->g[l]); }
+  X.nf = nf; X.ring = ring;
+  X.w = w < g0.nx ? w : g0.nx;
+  if (X.w > g0.ny) X.w = g0.ny;
+  return X;
 }
 
 __global__ void k_place_all(double *__restrict__ full, Geom gfull, const double *__restrict__ gathered, int hx, int hy, int px,
@@ -365,6 +349,25 @@ static int g_gather_coarse(msqg_group *G, int nf, double *full) {
   CK(cudaGetLastError());
   return MSQG_OK;
 }
+/* the list `list` of every tile restricted from level `from` down to La, then onto the tile's block of level La-1, and
+ * gathered into `full` on the solver tile; sg, flag: k_restrict's last two arguments */
+static int g_restrict_gather(msqg_group *G, List msqg_model::*list, int from, int nf, double sg, int flag, double *full) {
+  dim3 b(32, 8);
+  for (msqg_model *m : G->tiles) {
+    List &L = m->*list;
+    const int La = m->agg_level;
+    for (int l = from - 1; l >= La; l--) {
+      ProfScope ps(m, PROF_RESTRICT, l);
+      k_restrict<<<grid2(m->g[l].nx, m->g[l].ny, b, nf), b, 0, G->stream>>>(L.lev[l + 1], L.lev[l], m->g[l + 1], m->g[l], sg, flag);
+      m->launches++;
+    }
+    k_restrict<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nf), b, 0, G->stream>>>(L.lev[La], m->res_patch, m->g[La], m->gpatch, sg, flag);
+    k_unpack<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nf), b, 0, G->stream>>>(m->patch_stage, m->res_patch, nf, m->gpatch);
+    m->launches += 2;
+  }
+  CK(cudaGetLastError());
+  return g_gather_coarse(G, nf, full);
+}
 
 /* a += da on the one-cell halo ring of the INTERNAL sides (cells owned by a neighbouring tile; corners included when both
  * sides are internal); thread t walks the ring: bottom row, top row, left column, right column */
@@ -393,19 +396,8 @@ static int g_cycle(msqg_group *G, const std::vector<MgProblem> &P, int nrelax) {
   const int nt = (int)G->tiles.size();
   dim3 b(32, 8);
   int rc;
-  /* restriction(res) on the distributed levels, then onto this tile's share of level La-1 */
-  for (msqg_model *m : G->tiles) {
-    for (int l = D - 1; l >= La; l--) {
-      ProfScope ps(m, PROF_RESTRICT, l);
-      k_restrict<<<grid2(m->g[l].nx, m->g[l].ny, b, nf), b, 0, G->stream>>>(m->res.lev[l + 1], m->res.lev[l], m->g[l + 1], m->g[l], -1., 0);
-      m->launches++;
-    }
-    k_restrict<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nf), b, 0, G->stream>>>(m->res.lev[La], m->res_patch, m->g[La], m->gpatch, -1., 0);
-    k_unpack<<<grid2(m->gpatch.nx, m->gpatch.ny, b, nf), b, 0, G->stream>>>(m->patch_stage, m->res_patch, nf, m->gpatch);
-    m->launches += 2;
-  }
-  CK(cudaGetLastError());
-  if ((rc = g_gather_coarse(G, nf, S->res.lev[La - 1]))) return rc;
+  /* restriction(res) on the distributed levels, then onto this tile's share of level La-1, gathered on the solver tile */
+  if ((rc = g_restrict_gather(G, &msqg_model::res, D, nf, -1., 0, S->res.lev[La - 1]))) return rc;
   /* levels 1 .. La-1 on the solver tile: the undecomposed multigrid, whose arithmetic does not depend on the tiles */
   if ((rc = mg_levels(S, nf, mode, nrelax, La - 1, La - 1))) return rc;
   const int hx = S->gpatch.nx, hy = S->gpatch.ny;
@@ -418,12 +410,6 @@ static int g_cycle(msqg_group *G, const std::vector<MgProblem> &P, int nrelax) {
   }
   CK(cudaGetLastError());
   const int chunk0 = nrelax < 7 ? nrelax : 7;
-  auto da_item = [&](int l, int w) { /* da of level l with a halo of w cells */
-    XItem X;
-    for (msqg_model *m : G->tiles) { X.arr.push_back(m->da.lev[l]); X.geo.push_back(m->g[l]); }
-    X.nf = nf; X.w = w; X.ring = 0;
-    return X;
-  };
   /* distributed levels: prolongation, then the sweeps of the smoother */
   for (int l = La; l <= D; l++) {
     for (msqg_model *m : G->tiles) {
@@ -435,11 +421,13 @@ static int g_cycle(msqg_group *G, const std::vector<MgProblem> &P, int nrelax) {
     CK(cudaGetLastError());
     if (!G->rb) {
       /* lexicographic: block Gauss-Seidel, a one-cell halo of da refreshed before the first sweep and after every one */
-      std::vector<XItem> items{da_item(l, 1)};
+      std::vector<XItem> items{level_item(G, &msqg_model::da, l, nf, 1, 0)};
       if ((rc = exchange_multi(G, items))) return rc;
       for (int s = 0; s < nrelax; s++) {
-        for (msqg_model *m : G->tiles)
-          if ((rc = g_relax_level(G, m, l, 1))) return rc;
+        for (msqg_model *m : G->tiles) {
+          ProfScope ps(m, l == D ? PROF_RELAX_FINE : PROF_RELAX_COARSE, 1);
+          if ((rc = relax_level(m, mode, l, 1))) return rc;
+        }
         if ((rc = exchange_multi(G, items))) return rc;
       }
       continue;
@@ -449,32 +437,20 @@ static int g_cycle(msqg_group *G, const std::vector<MgProblem> &P, int nrelax) {
     while (left > 0) {
       const int c = left < 7 ? left : 7;       /* sweeps covered by one exchange: 2c + 1 <= 15 cells of halo */
       const int last = (left - c == 0);
-      int w = 2 * c + (last ? 1 : 0);          /* one halo cell must survive the last sweep: the prolongation reads it */
-      const Geom &g0 = S->g[l];
-      if (w > g0.nx) w = g0.nx;
-      if (w > g0.ny) w = g0.ny;
+      /* one halo cell must survive the last sweep: the prolongation reads it */
+      std::vector<XItem> items{level_item(G, &msqg_model::da, l, nf, 2 * c + (last ? 1 : 0), 0)};
+      const int w = items[0].w;
       if (w < 2 * c) FAIL(MSQG_ERR_ARG, "tiles of level %d are too small for %d fused sweeps (raise agg_n)", l, c);
-      std::vector<XItem> items{da_item(l, w)};
       if (l == La && left == nrelax) {
         /* the halo of res on ALL distributed levels (the sweeps recompute up to 2 nrelax border cells of the neighbours)
            rides in the same exchange: one neighbour synchronisation less per cycle */
-        for (int l2 = La; l2 <= D; l2++) {
-          XItem X;
-          for (msqg_model *m : G->tiles) { X.arr.push_back(m->res.lev[l2]); X.geo.push_back(m->g[l2]); }
-          X.nf = nf; X.w = 2 * chunk0; X.ring = 0;
-          if (X.w > S->g[l2].nx) X.w = S->g[l2].nx;
-          if (X.w > S->g[l2].ny) X.w = S->g[l2].ny;
-          items.push_back(X);
-        }
+        for (int l2 = La; l2 <= D; l2++) items.push_back(level_item(G, &msqg_model::res, l2, nf, 2 * chunk0, 0));
       }
       if ((rc = exchange_multi(G, items))) return rc;
       for (msqg_model *m : G->tiles) {
+        /* sweeps on tile + halo: the halo of w cells shrinks by 2 per sweep (launch_relax_rb) */
         ProfScope ps(m, l == D ? PROF_RELAX_FINE : PROF_RELAX_COARSE, c);
-        if (mode < 0) {
-          NL_SWITCH(m->nl, { auto C = relax_coef_layers<NL>(m, l); rc = relax_rb_tile<NL>(m, l, c, w, C); });
-        } else
-          rc = relax_rb_tile<1>(m, l, c, w, relax_coef_scalar(m, l, m->lam_lev[(size_t)l * m->nl + mode]));
-        if (rc) return rc;
+        if ((rc = relax_level(m, mode, l, c, w))) return rc;
       }
       left -= c;
     }

@@ -1044,11 +1044,12 @@ static int launch_relax_ws(msqg_model *m, double *da, const double *res, int lev
 }
 template <int NL>
 static int launch_relax_rb(msqg_model *m, double *da, const double *res, int lev, int nrelax, const RelaxCoef<NL> &C,
-                           const int *orange, int halo, double *corr_a);
+                           int halo, double *corr_a);
+/* halo (red-black tiles): valid cells of deep halo on the internal sides, see launch_relax_rb */
 template <int NL>
 static int launch_relax(msqg_model *m, double *da, const double *res, int lev, int nrelax, const RelaxCoef<NL> &C,
-                        double *corr_a = nullptr) {
-  if (m->smoother == 1) return launch_relax_rb<NL>(m, da, res, lev, nrelax, C, nullptr, 0, corr_a);
+                        int halo = 0, double *corr_a = nullptr) {
+  if (m->smoother == 1) return launch_relax_rb<NL>(m, da, res, lev, nrelax, C, halo, corr_a);
   if (corr_a) FAIL(MSQG_ERR_ARG, "the correction is folded into red-black passes only");
   int done = 0;
   while (done < nrelax) {
@@ -1081,7 +1082,7 @@ static bool rb_tiled(int nf, bool rcoef, long long cells) {
 }
 template <int NL, bool RCOEF>
 static int launch_relax_rb_pass(msqg_model *m, double *da, const double *res, int lev, int ns, const RelaxCoef<NL> &C,
-                                const int *orange /* optional {ox_lo, ox_hi, oy_lo, oy_hi} */, int halo,
+                                const int *orange /* {ox_lo, ox_hi, oy_lo, oy_hi} */, int halo,
                                 double *corr_a = nullptr /* k_relax_rb<..., FOLD = true>: a += da instead of da2 = da */) {
   using Cfg = RbCfg<NL>;
   const Geom &g = m->g[lev];
@@ -1097,8 +1098,7 @@ static int launch_relax_rb_pass(msqg_model *m, double *da, const double *res, in
   A.da = da; A.da_out = m->da2.lev[lev]; A.res = res; A.g = g; A.ns = ns;
   A.R = 2 * nh + 1 + RB_PF;
   A.TX = RB_WX - 2 * nh;
-  A.ox_lo = 0; A.ox_hi = g.nx; A.oy_lo = 0; A.oy_hi = g.ny;
-  if (orange) { A.ox_lo = orange[0]; A.ox_hi = orange[1]; A.oy_lo = orange[2]; A.oy_hi = orange[3]; }
+  A.ox_lo = orange[0]; A.ox_hi = orange[1]; A.oy_lo = orange[2]; A.oy_hi = orange[3];
   /* cells that exist: own cells, plus `halo` cells of deep halo on the sides that have a neighbouring tile */
   A.xlo = (g.bc & 1) ? -halo : 0; A.xhi = g.nx + ((g.bc & 2) ? halo : 0);
   A.ylo = (g.bc & 4) ? -halo : 0; A.yhi = g.ny + ((g.bc & 8) ? halo : 0);
@@ -1110,7 +1110,7 @@ static int launch_relax_rb_pass(msqg_model *m, double *da, const double *res, in
   const int nxo_ = A.ox_hi - A.ox_lo, nyo_ = A.oy_hi - A.oy_lo;
   const bool fold = corr_a != nullptr;
   if (fold) {
-    if (orange || halo || g.bc || rb_tiled(NL, RCOEF, (long long)nxo_ * nyo_))
+    if (halo || g.bc || rb_tiled(NL, RCOEF, (long long)nxo_ * nyo_))
       FAIL(MSQG_ERR_ARG, "the correction is folded into streaming passes over a whole undecomposed level only");
     if (!rb_can_fold(NL)) FAIL(MSQG_ERR_ARG, "nl = %d has no folded relax pass", NL);
     A.a = corr_a;
@@ -1177,26 +1177,33 @@ static int launch_relax_rb_pass(msqg_model *m, double *da, const double *res, in
   return MSQG_OK;
 }
 /* nrelax sweeps as ceil(nrelax / NSMAX) passes of (almost) equal length; the result does not depend on the split.
+ * halo (tiles, dist_rb.cuh): the deep halo holds `halo` valid cells on the internal sides on entry; each pass writes its
+ * own cells plus what stays valid after its ns sweeps, halo - 2 ns cells, so the halo holds halo - 2 nrelax cells on
+ * exit.  Without a halo on a level with internal sides only the own cells are swept.
  * corr_a (optional): the last pass adds da to this unknown instead of storing da (k_relax_rb<..., FOLD = true>). */
 template <int NL>
 static int launch_relax_rb(msqg_model *m, double *da, const double *res, int lev, int nrelax, const RelaxCoef<NL> &C,
-                           const int *orange = nullptr, int halo = 0, double *corr_a = nullptr) {
+                           int halo = 0, double *corr_a = nullptr) {
   constexpr int NSMAX = RbCfg<NL>::NSMAX;
-  int left = nrelax;
+  const Geom &g = m->g[lev];
+  const bool deep = g.bc && halo > 0;
+  int left = nrelax, h = halo;
   if (da != m->da.lev[lev]) FAIL(MSQG_ERR_ARG, "the rb relax pass works on the model's da list");
-  if (orange && nrelax > NSMAX) FAIL(MSQG_ERR_ARG, "a tile relax pass holds at most %d sweeps", NSMAX);
   while (left > 0) {
     const int passes = (left + NSMAX - 1) / NSMAX;
     const int ns = (left + passes - 1) / passes;
+    const int ho = deep ? h - 2 * ns : 0;
+    if (ho < 0) FAIL(MSQG_ERR_ARG, "halo of %d cells is too thin for %d sweeps", halo, nrelax);
+    const int orange[4] = {(g.bc & 1) ? -ho : 0, g.nx + ((g.bc & 2) ? ho : 0), (g.bc & 4) ? -ho : 0, g.ny + ((g.bc & 8) ? ho : 0)};
     double *ca = left == ns ? corr_a : nullptr;
     int rc;
-    if (relax_uses_table<NL>(m)) {
-      if constexpr (NL <= 6) rc = launch_relax_rb_pass<NL, true>(m, m->da.lev[lev], res, lev, ns, C, orange, halo, ca);
+    if (relax_uses_table<NL>(m)) { /* horizontally varying stretching: tables over own cells + halo on tiles (g_stretching) */
+      if constexpr (NL <= 6) rc = launch_relax_rb_pass<NL, true>(m, m->da.lev[lev], res, lev, ns, C, orange, h, ca);
       else FAIL(MSQG_ERR_ARG, "varRo > 0 with the layer-coupled solver is built for nl <= 6 (nl = %d)", NL);
     } else
-      rc = launch_relax_rb_pass<NL, false>(m, m->da.lev[lev], res, lev, ns, C, orange, halo, ca);
+      rc = launch_relax_rb_pass<NL, false>(m, m->da.lev[lev], res, lev, ns, C, orange, h, ca);
     if (rc) return rc;
-    left -= ns;
+    left -= ns; h = ho;
   }
   return MSQG_OK;
 }
@@ -1308,12 +1315,30 @@ static int residual_pyr_bottom(const msqg_model *m) {
   return D - PYR_MAXLEV > 1 ? D - PYR_MAXLEV : 1;
 }
 
-static int mg_residual_enqueue(msqg_model *m, const MgProblem &P) {
+/* res = b - A a on level D and its max norm in d_scal[0], without the restriction pyramid (one grid or one tile) */
+static int launch_residual(msqg_model *m, const MgProblem &P) {
   const int D = m->depth;
   const Geom &g = m->g[D];
   CK(zero_words(m->stream, m->d_scal, 1));
+  dim3 b(64, 4);
+  { ProfScope ps(m, PROF_RESIDUAL, 0);
+  if (P.mode < 0) {
+    LayerMetrics M = metrics_of(m);
+    NL_SWITCH(m->nl, k_residual<NL><<<grid2(g.nx, g.ny, b), b, 0, m->stream>>>(P.a, P.b, m->res.lev[D], m->str.lev[D], g, M, m->d_scal));
+  } else {
+    k_residual_scalar<<<grid2(g.nx, g.ny, b), b, 0, m->stream>>>(P.a, P.b, m->res.lev[D], m->ibu.lev[D] + (size_t)P.mode * g.plane, g, m->d_scal);
+  }
+  }
+  m->launches++;
+  CK(cudaGetLastError());
+  return MSQG_OK;
+}
+static int mg_residual_enqueue(msqg_model *m, const MgProblem &P) {
+  const int D = m->depth;
+  const Geom &g = m->g[D];
   const int bottom = residual_pyr_bottom(m);
   if (bottom < D) {
+    CK(zero_words(m->stream, m->d_scal, 1));
     PyrLevels L;
     L.nlev = D - bottom;
     for (int k = 0; k < PYR_MAXLEV; k++) {
@@ -1335,29 +1360,23 @@ static int mg_residual_enqueue(msqg_model *m, const MgProblem &P) {
     }
     m->launches++;
     CK(cudaGetLastError());
-    CK(to_host(m->stream, m->h_scal, m->d_scal, 1));
-    return MSQG_OK;
-  }
-  dim3 b(64, 4);
-  { ProfScope ps(m, PROF_RESIDUAL, 0);
-  if (P.mode < 0) {
-    LayerMetrics M = metrics_of(m);
-    NL_SWITCH(m->nl, k_residual<NL><<<grid2(g.nx, g.ny, b), b, 0, m->stream>>>(P.a, P.b, m->res.lev[D], m->str.lev[D], g, M, m->d_scal));
   } else {
-    k_residual_scalar<<<grid2(g.nx, g.ny, b), b, 0, m->stream>>>(P.a, P.b, m->res.lev[D], m->ibu.lev[D] + (size_t)P.mode * g.plane, g, m->d_scal);
+    int rc = launch_residual(m, P);
+    if (rc) return rc;
   }
-  }
-  m->launches++;
-  CK(cudaGetLastError());
   CK(to_host(m->stream, m->h_scal, m->d_scal, 1));
+  return MSQG_OK;
+}
+/* the residual norm that mg_residual_enqueue left in the pinned mirror */
+static int mg_residual_read(msqg_model *m, double *maxres) {
+  CK(cudaStreamSynchronize(m->stream));
+  *maxres = m->h_scal[0];
   return MSQG_OK;
 }
 static int mg_residual(msqg_model *m, const MgProblem &P, double *maxres) {
   int rc = mg_residual_enqueue(m, P);
   if (rc) return rc;
-  CK(cudaStreamSynchronize(m->stream));
-  *maxres = m->h_scal[0];
-  return MSQG_OK;
+  return mg_residual_read(m, maxres);
 }
 
 /* Run `body` (which only enqueues work on `st`) through a CUDA graph: the first use of a key runs eagerly (lazy
@@ -1412,6 +1431,20 @@ static unsigned long long da_parity_mask(msqg_model *m) {
  * (k_coarse_rb), which also does their restrictions. */
 /* MSQG_RB_FOLD=0: a separate k_correct launch instead of the correction folded into the last relax pass (A/B) */
 static bool rb_fold_enabled() { const char *e = getenv("MSQG_RB_FOLD"); return !(e && atoi(e) == 0); }
+/* nrelax sweeps on da / res of level l: the layer-coupled problem (mode < 0), or vertical mode `mode` with its lambda
+ * (per-cell tables while the modes vary horizontally).  halo, corr_a: launch_relax's */
+static int relax_level(msqg_model *m, int mode, int l, int nrelax, int halo = 0, double *corr_a = nullptr) {
+  int rc;
+  if (mode < 0) {
+    NL_SWITCH(m->nl, { auto C = relax_coef_layers<NL>(m, l); rc = launch_relax<NL>(m, m->da.lev[l], m->res.lev[l], l, nrelax, C, halo, corr_a); });
+  } else {
+    auto C = relax_coef_scalar(m, l, m->lam_lev[(size_t)l * m->nl + mode]);
+    m->coef_mode = m->modes_uniform ? -1 : mode;
+    rc = launch_relax<1>(m, m->da.lev[l], m->res.lev[l], l, nrelax, C, halo, corr_a);
+    m->coef_mode = -1;
+  }
+  return rc;
+}
 /* corrected != NULL (mg_cycle): when level D of an undecomposed grid goes through the streaming red-black kernel, its
  * last pass adds da to corr_a (no k_correct); *corrected tells the caller whether that happened.  Same bits. */
 static int mg_levels(msqg_model *m, int nf, int mode, int nrelax, int from, int top, double *corr_a = nullptr,
@@ -1468,15 +1501,7 @@ static int mg_levels(msqg_model *m, int nf, int mode, int nrelax, int from, int 
       CK(cudaGetLastError());
     }
     ProfScope ps(m, l == D ? PROF_RELAX_FINE : PROF_RELAX_COARSE, nrelax);
-    if (mode < 0) {
-      NL_SWITCH(m->nl, { auto C = relax_coef_layers<NL>(m, l); rc = launch_relax<NL>(m, m->da.lev[l], m->res.lev[l], l, nrelax, C, ca); });
-    } else {
-      auto C = relax_coef_scalar(m, l, m->lam_lev[(size_t)l * m->nl + mode]);
-      m->coef_mode = m->modes_uniform ? -1 : mode;
-      rc = launch_relax<1>(m, m->da.lev[l], m->res.lev[l], l, nrelax, C, ca);
-      m->coef_mode = -1;
-    }
-    if (rc) return rc;
+    if ((rc = relax_level(m, mode, l, nrelax, 0, ca))) return rc;
     if (ca) *corrected = true;
   }
   return MSQG_OK;
@@ -1500,32 +1525,34 @@ static int mg_cycle(msqg_model *m, const MgProblem &P, int nrelax) {
   return MSQG_OK;
 }
 
-/* mg_solve, mspg/elliptic.h:145-229: NITERMIN=1, NITERMAX=100, nrelax starts at 4.  sched != NULL (msqg_test_cycles):
- * exactly ncycles cycles, cycle k with sched[k] sweeps per level, no tolerance stop and no adaptation; resa_out[k] is the
- * residual after cycle k */
-static int mg_solve(msqg_model *m, const MgProblem &P, double tolerance, msqg_mgstats *st, const int *sched = nullptr,
-                    int ncycles = 0, double *resa_out = nullptr) {
+/* The solve loop of mg_solve and g_solve, mspg/elliptic.h:145-229: NITERMIN=1, NITERMAX=100, nrelax starts at 4 and
+ * adapts to the convergence rate.  sched != NULL (msqg_test_cycles): exactly ncycles cycles, cycle k with sched[k]
+ * sweeps per level, no tolerance stop and no adaptation; resa_out[k] is the residual after cycle k.
+ * residual() and cycle(nrelax) only enqueue work on `st`; read(&r) waits for the residual norm.  Each cycle and the
+ * residual that follows it run through run_graphed (one graph launch when `graphed`), keyed by nrelax, the problem
+ * (mode, unknown and right-hand side of P, the first tile's under a group) and the da buffers of every model. */
+template <class Residual, class Cycle, class Read>
+static int mg_solve_loop(cudaStream_t st, GraphCache &gc, std::vector<msqg_model *> &models, long *exchanges, bool graphed,
+                         const MgProblem &P, double tolerance, msqg_mgstats *out, const int *sched, int ncycles,
+                         double *resa_out, Residual residual, Cycle cycle, Read read) {
   msqg_mgstats s;
   memset(&s, 0, sizeof(s));
   s.nrelax = 4;
   double resb;
-  int rc = mg_residual(m, P, &resb);
-  if (rc) return rc;
+  int rc;
+  if ((rc = residual()) || (rc = read(&resb))) return rc;
   s.resb = s.resa = resb;
-  const bool graphed = m->smoother == 1 && m->use_graphs && !m->prof_on; /* coefficient tables are fixed between set_const calls */
-  std::vector<msqg_model *> self(1, m);
   for (s.i = 0; sched ? s.i < ncycles : s.i < 100 && (s.i < 1 || s.resa > tolerance); s.i++) {
     if (sched) s.nrelax = sched[s.i];
-    /* one cycle + the residual that follows it: a single graph launch in red-black mode */
-    GraphKey key(s.nrelax, P.mode, (const void *)P.a, (const void *)P.b, da_parity_mask(m));
-    rc = run_graphed(m->stream, m->graphs, key, self, nullptr, graphed, [&]() -> int {
-      int r2 = mg_cycle(m, P, s.nrelax);
+    unsigned long long mask = 0;
+    for (msqg_model *m : models) mask = mask * 1315423911ull + da_parity_mask(m);
+    GraphKey key(s.nrelax, P.mode, (const void *)P.a, (const void *)P.b, mask);
+    rc = run_graphed(st, gc, key, models, exchanges, graphed, [&]() -> int {
+      int r2 = cycle(s.nrelax);
       if (r2) return r2;
-      return mg_residual_enqueue(m, P);
+      return residual();
     });
-    if (rc) return rc;
-    CK(cudaStreamSynchronize(m->stream));
-    s.resa = m->h_scal[0];
+    if (rc || (rc = read(&s.resa))) return rc;
     if (sched) resa_out[s.i] = s.resa;
     else if (s.resa > tolerance) {
       if (resb / s.resa < 1.2 && s.nrelax < 100) s.nrelax++;
@@ -1533,9 +1560,41 @@ static int mg_solve(msqg_model *m, const MgProblem &P, double tolerance, msqg_mg
     }
     resb = s.resa;
   }
-  if ((rc = check_relax_err(m))) return rc;
+  *out = s;
+  return MSQG_OK;
+}
+
+/* mg_solve on one grid; sched, ncycles, resa_out as mg_solve_loop's */
+static int mg_solve(msqg_model *m, const MgProblem &P, double tolerance, msqg_mgstats *st, const int *sched = nullptr,
+                    int ncycles = 0, double *resa_out = nullptr) {
+  const bool graphed = m->smoother == 1 && m->use_graphs && !m->prof_on; /* coefficient tables are fixed between set_const calls */
+  std::vector<msqg_model *> self(1, m);
+  msqg_mgstats s;
+  int rc = mg_solve_loop(m->stream, m->graphs, self, nullptr, graphed, P, tolerance, &s, sched, ncycles, resa_out,
+                         [&]() { return mg_residual_enqueue(m, P); },
+                         [&](int nrelax) { return mg_cycle(m, P, nrelax); },
+                         [&](double *r) { return mg_residual_read(m, r); });
+  if (rc || (rc = check_relax_err(m))) return rc;
   m->total_cycles += s.i;
   *st = s;
+  return MSQG_OK;
+}
+
+/* layers <-> vertical modes on level D (k_project): out = M in with the host matrix h_mat, or with the per-column
+ * matrices of the field matf (non-null: horizontally varying modes).  ring: also the one-cell ring of a tile;
+ * ghosts: k_project's last argument */
+static int launch_project(msqg_model *m, const double *in, double *out, const double *h_mat, const double *matf, bool ring,
+                          int ghosts) {
+  const Geom &g = m->g[m->depth];
+  dim3 b(64, 4);
+  NL_SWITCH(m->nl, {
+    ModeMat<NL> M;
+    for (int k = 0; k < NL * NL; k++) M.a[k] = h_mat[k];
+    if (ring) k_project<NL, true><<<grid2(g.nx + 2, g.ny + 2, b), b, 0, m->stream>>>(in, out, g, M, matf, ghosts);
+    else k_project<NL><<<grid2(g.nx, g.ny, b), b, 0, m->stream>>>(in, out, g, M, matf, ghosts);
+  });
+  m->launches++;
+  CK(cudaGetLastError());
   return MSQG_OK;
 }
 
@@ -1552,26 +1611,13 @@ static int invertq_list(msqg_model *m, List &ql) {
     /* horizontally varying Fr/Ro: the projection matrices are fields (one eigmod per column), as in the reference */
     const double *matf_l2m = m->modes_uniform ? nullptr : m->cl2m.lev[D];
     const double *matf_m2l = m->modes_uniform ? nullptr : m->cm2l.lev[D];
-    dim3 b(64, 4);
-    NL_SWITCH(m->nl, {
-      ModeMat<NL> M;
-      for (int k = 0; k < NL * NL; k++) M.a[k] = m->h_cl2m[k];
-      k_project<NL><<<grid2(g.nx, g.ny, b), b, 0, m->stream>>>(ql.lev[D], m->qm.lev[D], g, M, matf_l2m, 0);
-    });
-    m->launches++;
-    CK(cudaGetLastError());
+    if ((rc = launch_project(m, ql.lev[D], m->qm.lev[D], m->h_cl2m, matf_l2m, false, 0))) return rc;
     for (int l = 0; l < m->nl; l++) {
       MgProblem P{1, l, m->pm.lev[D] + (size_t)l * g.plane, m->qm.lev[D] + (size_t)l * g.plane};
       if ((rc = mg_solve(m, P, 1e-3, &m->mgmode[l]))) return rc;
       m->mgpsi = m->mgmode[l];
     }
-    NL_SWITCH(m->nl, {
-      ModeMat<NL> M;
-      for (int k = 0; k < NL * NL; k++) M.a[k] = m->h_cm2l[k];
-      k_project<NL><<<grid2(g.nx, g.ny, b), b, 0, m->stream>>>(m->pm.lev[D], m->psi.lev[D], g, M, matf_m2l, 1);
-    });
-    m->launches++;
-    CK(cudaGetLastError());
+    if ((rc = launch_project(m, m->pm.lev[D], m->psi.lev[D], m->h_cm2l, matf_m2l, false, 1))) return rc;
   }
   return MSQG_OK;
 }
@@ -1968,14 +2014,32 @@ static int rhs_prepare(msqg_model *m) {
   CK(to_host(m->stream, m->h_scal + 1, m->d_scal + 1, m->nl));
   return MSQG_OK;
 }
-/* dtmax chain of advection_pv, qg.h:383-391 (needs the umax D2H to have completed) */
-static double dt_chain(msqg_model *m, double dtmax) {
+/* dtmax chain of advection_pv, qg.h:383-391: umax, the max face speeds of psi (needs their D2H to have completed), and
+ * umax_pg, those of the background flow, per layer.  timestep()'s state is m->ts_previous (a group's: its tiles[0]'s) */
+static double dt_chain(msqg_model *m, const double *umax, const double *umax_pg, double dtmax) {
   const double Delta = m->g[m->depth].Delta;
   for (int l = 0; l < m->nl; l++) {
-    dtmax = timestep_chain(m, m->h_scal[1 + l], dtmax, Delta);
-    dtmax = timestep_chain(m, m->umax_pg[l], dtmax, Delta);
+    dtmax = timestep_chain(m, umax[l], dtmax, Delta);
+    dtmax = timestep_chain(m, umax_pg[l], dtmax, Delta);
   }
   return dtmax;
+}
+/* dtnext(), [BASILISK] events: TEPS = 1e-9.  dt rounded so that t lands on tnext_event (negative: no pending event);
+ * *tnext is the time after the step */
+static double dtnext(double t, double tnext_event, double dt, double *tnext) {
+  if (tnext_event >= 0 && tnext_event > t) {
+    unsigned int nn = (tnext_event - t) / dt;
+    *tnext = tnext_event;
+    if (nn == 0) dt = tnext_event - t;
+    else {
+      const double dt1 = (tnext_event - t) / nn;
+      if (dt1 > dt * (1. + 1e-9)) dt = (tnext_event - t) / (nn + 1);
+      else if (dt1 < dt) dt = dt1;
+      *tnext = t + dt;
+    }
+  } else
+    *tnext = t + dt;
+  return dt;
 }
 
 static int rhs_launch(msqg_model *m, List &q_ev, const double *q_in, double *q_out, double *dq, double dt, float dts) {
@@ -2052,7 +2116,7 @@ extern "C" int msqg_update(msqg_model *m, int q_id, double dtmax, double *dtmax_
   if ((rc = rhs_launch(m, *L, nullptr, nullptr, m->dq.lev[m->depth], 0., 0.f))) return rc;
   if (m->p.nptr > 0 && (rc = ptr_launch(m, q_id == MSQG_QPRED ? m->ptr_pred : m->ptr, nullptr, nullptr, m->dptr.lev[m->depth], 0.))) return rc;
   CK(cudaStreamSynchronize(m->stream));
-  if (dtmax_out) *dtmax_out = dt_chain(m, dtmax);
+  if (dtmax_out) *dtmax_out = dt_chain(m, m->h_scal + 1, m->umax_pg, dtmax);
   return MSQG_OK;
 }
 
@@ -2151,21 +2215,8 @@ extern "C" int msqg_step(msqg_model *m, double t, double tnext_event, double *dt
   if ((rc = invertq_list(m, m->q))) return rc;
   if ((rc = rhs_prepare(m))) return rc;
   CK(cudaStreamSynchronize(m->stream));
-  double dt = dt_chain(m, m->p.DT);
   double tnext;
-  if (tnext_event >= 0 && tnext_event > t) {
-    /* dtnext(), [BASILISK] events: TEPS = 1e-9 */
-    unsigned int nn = (tnext_event - t) / dt;
-    tnext = tnext_event;
-    if (nn == 0) dt = tnext_event - t;
-    else {
-      const double dt1 = (tnext_event - t) / nn;
-      if (dt1 > dt * (1. + 1e-9)) dt = (tnext_event - t) / (nn + 1);
-      else if (dt1 < dt) dt = dt1;
-      tnext = t + dt;
-    }
-  } else
-    tnext = t + dt;
+  double dt = dtnext(t, tnext_event, dt_chain(m, m->h_scal + 1, m->umax_pg, m->p.DT), &tnext);
   float dts = 0.f;
   if (m->p.stochastic && (rc = stochastic_stage(m, sqrt(dt / 2.), &dts))) return rc;
   double *dqp = m->keep_dq ? m->dq.lev[D] : nullptr;
@@ -2178,7 +2229,7 @@ extern "C" int msqg_step(msqg_model *m, double t, double tnext_event, double *dt
   if ((rc = rhs_launch(m, m->qpred, m->q.lev[D], m->q.lev[D], dqp, dt, dts))) return rc;
   if (m->p.nptr > 0 && (rc = ptr_launch(m, m->ptr_pred, m->ptr.lev[D], m->ptr.lev[D], nullptr, dt))) return rc;
   CK(cudaStreamSynchronize(m->stream));
-  (void)dt_chain(m, dt); /* update()'s return value is ignored in stage 2; timestep()'s static state is not */
+  (void)dt_chain(m, m->h_scal + 1, m->umax_pg, dt); /* update()'s return value is ignored in stage 2; timestep()'s static state is not */
   if (dt_out) *dt_out = dt;
   if (tnext_out) *tnext_out = tnext;
   return MSQG_OK;
@@ -2428,7 +2479,7 @@ extern "C" int msqg_tendency_bfn(msqg_model *m, double direction) {
   m->has_qforc = hq;
   if (rc) return rc;
   CK(cudaStreamSynchronize(m->stream));
-  (void)dt_chain(m, m->p.DT); /* advection_pv still runs timestep(): static state advances */
+  (void)dt_chain(m, m->h_scal + 1, m->umax_pg, m->p.DT); /* advection_pv still runs timestep(): static state advances */
   return MSQG_OK;
 }
 

@@ -88,6 +88,30 @@ def test_periodic_through_the_single_model_entry_points(gpu):
     assert np.array_equal(mg.get(G.Q), mo.get(O.Q))
 
 
+@pytest.mark.parametrize("sbc", [0., -1.])
+def test_ts_previous_reset_is_honoured(gpu, sbc):
+    """msqg_set_ts_previous(h, 0) restarts timestep()'s chain: a handle reset after three steps takes the same next step
+    as a fresh handle holding its psi and q, on a closed basin and on the periodic domain (whose handle is the tile of
+    a 1 x 1 group)."""
+    from msom_b200 import capi as G
+    from common import synth_psi
+    N, nl = 64, 3
+    kw = base_kw(N, nl, sbc=sbc)
+    a = G.Model(G.make_params(**kw), gpu)
+    a.set(G.PSI, periodic_psi(N, nl) if sbc < 0 else synth_psi(N, nl))
+    a.set_const()
+    for _ in range(3):
+        a.step()
+    a.L.msqg_set_ts_previous(a.h, 0.)
+    b = G.Model(G.make_params(**kw), gpu)
+    b.set_const()
+    b.set(G.PSI, a.get(G.PSI)); b.set(G.Q, a.get(G.Q))
+    assert a.step() == b.step()
+    assert np.array_equal(a.get(G.PSI), b.get(G.PSI))
+    assert np.array_equal(a.get(G.Q), b.get(G.Q))
+    a.close(); b.close()
+
+
 def test_periodic_rejects_what_is_not_built(gpu):
     from msom_b200 import capi as G
     from msom_b200.dist import Group
